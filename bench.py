@@ -2,6 +2,7 @@
 """Benchmark of the B200 spherical-harmonic synthesis path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling strong|weak]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -23,6 +24,9 @@ Output: one JSON line (rank 0).
 
 `--impl reference` times the reference's own CPU implementation (baseline/_ref when present, else the
 numpy oracle port) on the same config, metric and unit; rank 0 only.
+
+`--dump-outputs DIR` writes a fixed sample of the grid values of the last timed step to DIR (see dump_outputs); the
+inputs are seeded, so runs with the same arguments on two builds can be compared output for output.
 """
 import os
 import sys
@@ -68,6 +72,49 @@ def algorithmic_flops(nmax, nlat, nlon, epochs):
 def synthetic_batch(nmax, epochs, first_epoch=0):
     from oracle import sh_oracle  # input generator only (shared with the tests)
     return np.stack([sh_oracle.synthetic_coefficients(nmax, first_epoch + e) for e in range(epochs)])
+
+
+DUMP_EPOCHS, DUMP_VALUES, DUMP_SEED = 8, 1 << 20, 20240
+
+
+def dump_outputs(directory, out, first_epoch, total_epochs, dist=None, rank=0):
+    """Write a fixed sample of the job's grid values to `directory` as .npy files, so that the outputs of two builds
+    can be compared value for value.  `out` [epochs, nlat, nlon] (float64) holds this rank's epochs first_epoch, ...
+    of the job's total_epochs.  The whole batch of config 2 is 498 MB; the sample is about 34 MB: the first, the last
+    and six seeded whole epochs, and 2^20 seeded single values of the job, each beside the indices it was taken at
+    (epoch numbers, and flat indices into the [total_epochs, nlat, nlon] values), stored as float64.  The sample is
+    drawn over the whole job and collected on rank 0, which writes it: the same files for any number of GPUs."""
+    import torch
+    epochs, nlat, nlon = out.shape
+    points = nlat * nlon
+    rng = np.random.default_rng(DUMP_SEED)
+    inner = np.arange(1, max(total_epochs - 1, 1))
+    pick = np.unique(np.concatenate(([0, total_epochs - 1], rng.choice(inner, min(DUMP_EPOCHS - 2, inner.size), replace=False))))
+    flat = np.sort(rng.choice(total_epochs * points, min(DUMP_VALUES, total_epochs * points), replace=False))
+
+    def share(index, per_epoch, source):
+        """The entries of the sample at `index` that this rank holds; the others stay zero."""
+        held = (index >= first_epoch * per_epoch) & (index < (first_epoch + epochs) * per_epoch)
+        dst = torch.zeros((index.size,) + source.shape[1:], dtype=torch.float64, device=out.device)
+        dst[torch.as_tensor(np.flatnonzero(held), device=out.device)] = \
+            source[torch.as_tensor(index[held] - first_epoch * per_epoch, device=out.device)]
+        return dst
+
+    whole, values = share(pick, 1, out), share(flat, points, out.reshape(-1))
+    if dist is not None:
+        for t in (whole, values):       # one rank holds each entry: the integer sum of the bit patterns is exact
+            dist.reduce(t.view(torch.int64), dst=0, op=dist.ReduceOp.SUM)
+    if rank != 0:
+        return
+    os.makedirs(directory, exist_ok=True)
+    arrays = {
+        "grid_values_epochs": whole.cpu().numpy(),
+        "grid_values_epochs_index": pick.astype(np.float64),
+        "grid_values_sample": values.cpu().numpy(),
+        "grid_values_sample_index": flat.astype(np.float64),
+    }
+    for name, array in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), array)
 
 
 class ClockSampler(threading.Thread):
@@ -149,9 +196,9 @@ def blas_threads():
 
 
 def load_reference():
-    """The unmodified reference package from baseline/_ref (git-ignored, shipped to the GPU box with the snapshot);
-    netCDF4 / h5py are absent and unused on this path (grates/__init__.py:48 -> io.py:18-19), so they are stubbed.
-    Returns the module or None."""
+    """The unmodified reference package from baseline/_ref (git-ignored; __graft_entry__.install_reference puts it
+    there when a reference checkout is present); netCDF4 / h5py are unused on this path (grates/__init__.py:48 ->
+    io.py:18-19), so they are stubbed.  Returns the module or None."""
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref_dir, "grates")):
         return None
@@ -257,7 +304,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=None, help="steps of the host-buffer loop (default min(steps, 30))")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs 1/3/4/5 block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the grid values of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -352,6 +405,9 @@ def main():
     max_time = reduce_max(my_time)
     total_units = reduce_sum(float(units_per_step))
     value = total_units * args.steps / max_time
+    if args.dump_outputs is not None:          # `out` holds the last timed step's result until the pass below
+        dump_outputs(args.dump_outputs, out, first, int(round(total_units / (nlat * nlon))),
+                     dist if distributed else None, rank)
 
     # ---- the same K steps with an event pair around every kernel (per-kernel times for the roofline; the extra
     #      stream operations between the kernels switch the launch chaining off, so this pass is not the headline) ----

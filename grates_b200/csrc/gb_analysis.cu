@@ -425,7 +425,7 @@ static int set_analysis(gb_plan* plan, int nmin, const double* lon_ops, const do
             }
         }
     }
-    if (getenv("GB_NO_SYMMETRY") && getenv("GB_NO_SYMMETRY")[0] && getenv("GB_NO_SYMMETRY")[0] != '0') sym = false;
+    if (gb_env_flag("GB_NO_SYMMETRY")) sym = false;
     std::vector<std::vector<int>> cols;   // spectral rows (2m+cs) per set
     if (sym) {
         cols.resize(4);
@@ -527,7 +527,7 @@ static int launch_analysis(gb_plan* p, const double* d_grid, int E, double* d_an
     const long long M = (long long)E * p->nlat;
     const long long mpad = p->ws_mpad;
     GB_CUDA(cudaMemsetAsync(d_anm, 0, (size_t)E * L * L * sizeof(double), st));
-    if (getenv("GB_SIMPLE_ANALYSIS") && getenv("GB_SIMPLE_ANALYSIS")[0] != '0') {
+    if (gb_env_flag("GB_SIMPLE_ANALYSIS")) {
         // plain FMA longitude stage (cross-check of the tensor-core path)
         dim3 grid((unsigned)((M + LT - 1) / LT), (p->kpad + LT - 1) / LT);
         gb_analysis_lon_kernel<<<grid, 256, 0, st>>>(d_grid, p->d_lon_ops, p->d_ab, M, p->nlon, p->kpad, mpad);

@@ -3,6 +3,7 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstdarg>
+#include <cstdlib>
 #include <cuda_runtime.h>
 #include "../../include/grates_b200.h"
 
@@ -34,6 +35,13 @@ void gb_count_launch(int n = 1);
         gb_count_launch();                                                                      \
         GB_CUDA(cudaGetLastError());                                                            \
     } while (0)
+
+// Environment switch `name`: set, non-empty and not starting with '0'.  Read on every call, so that a process (a test)
+// can change it between calls.
+inline bool gb_env_flag(const char* name) {
+    const char* v = getenv(name);
+    return v && v[0] && v[0] != '0';
+}
 
 // ---------------------------------------------------------------------------------------------
 // tiled HBM layouts shared by the synthesis kernels
@@ -177,8 +185,9 @@ int gb_launch_unpack(const double* d_x, double* d_anm, int L, int E, cudaStream_
 // d_roff [L + 1] = first row of every order (gb_plan::d_ptab_roff).  The buffer must have been cleared for this layout.
 int gb_launch_pack_tiled(const double* d_anm, double* d_x, int L, int E, const int* d_roff, int tn, int n_ct,
                          cudaStream_t st, const double* d_wn = nullptr);
-// symmetric Fourier stage of the synthesis on rows [0, M) of an AB-layout operand (gb_synthesis.cu); needs p->sym
-int gb_launch_stage2_sym(gb_plan* p, const double* d_ab, long long M, double* d_out, cudaStream_t st);
+// symmetric Fourier stage of the synthesis on rows [0, M) of an AB-layout operand (gb_synthesis.cu); needs p->sym.
+// pdl: launched with programmatic dependent launch (the kernel may start while its predecessor drains)
+int gb_launch_stage2_sym(gb_plan* p, const double* d_ab, long long M, double* d_out, cudaStream_t st, bool pdl);
 const int* gb_stage2_krow(const gb_plan* p);    // spectral row 2m + cs -> row of that stage's AB layout
 // order-wise block filter of a batch, written straight into a synthesis workspace X (gb_filter.cu): order-wise packed
 // (d_roff == nullptr) or the tiled layout of gb_launch_pack_tiled (the buffer must have been cleared for it)
@@ -218,14 +227,9 @@ struct gb_scratch {
     }
 };
 
-// Kernel launch with the programmatic-stream-serialization attribute (PDL); GB_NO_PDL=1 launches plainly.
+// Kernel launch with the programmatic-stream-serialization attribute (PDL).
 #ifdef __CUDACC__
-#include <cstdlib>
 #include <utility>
-inline bool gb_pdl_enabled() {
-    static const bool on = [] { const char* v = getenv("GB_NO_PDL"); return !(v && v[0] && v[0] != '0'); }();
-    return on;
-}
 template <typename... KArgs, typename... Args>
 inline cudaError_t gb_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                                  Args&&... args) {
@@ -238,7 +242,7 @@ inline cudaError_t gb_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = gb_pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(std::forward<Args>(args))...);
 }
 #endif

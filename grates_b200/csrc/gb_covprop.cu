@@ -37,7 +37,6 @@
 //                        written in the A-tile layout of stage 4
 //   4. GEMM + LonEpilogue    W_i[k, j] = sum_k' H_i[k][k'] T[k'][j];          varpart[i][slot][j] = sum T[k][j] W
 //   5. gb_cov_finish     var = sum of the slots in order, optional sqrt
-#include <cstdlib>
 #include <vector>
 #include <cmath>
 #include <algorithm>
@@ -51,30 +50,14 @@ using gb::legendre_column;
 // row of degree offset r (n = n0 + r) inside its group: class (r + po) & 1, po = (n0 - m) & 1; class 1 starts at ne4
 __host__ __device__ __forceinline__ int cov_cls_pos(int r, int po, int ne4) { return (((r + po) & 1) ? ne4 : 0) + (r >> 1); }
 
-// St[gb_ab_offset(a', b, Kp4)] = Sigma[perm8[a']][perm4[b]]  (0 where either index is padding); cross-check of the
-// kernel below (GB_COV_PERMUTE_GATHER=1)
-__global__ void __launch_bounds__(256)
-gb_cov_permute(const double* __restrict__ sigma, double* __restrict__ St, const int* __restrict__ perm8,
-               const int* __restrict__ perm4, int rows_a, int Kp4, long long K) {
-    const int a = blockIdx.x * blockDim.x + threadIdx.x;   // a' fastest: coalesced writes
-    const int b = blockIdx.y;
-    if (a >= rows_a) return;
-    const int pa = perm8[a], pb = perm4[b];
-    St[gb_ab_offset(a, b, Kp4)] = (pa < 0 || pb < 0) ? 0.0 : sigma[(size_t)pa * K + pb];
-}
-
-// The same permutation, one CTA per (32 rows a', 64 columns of degree n): the 2n+1 columns of a degree
-// are contiguous in the degree-wise order, so Sigma is read in row segments of up to 512 bytes and St written in
-// 256-byte runs (the element-wise gather above fetches a 32-byte sector per double); 16 KB of shared memory per CTA
-// keeps a dozen CTAs resident per SM.
+// St[gb_ab_offset(a', b, Kp4)] = Sigma[perm8[a']][perm4[b]] (0 where either index is padding), one CTA per (32 rows a',
+// 64 columns of degree n): the 2n+1 columns of a degree are contiguous in the degree-wise order, so Sigma is read in
+// row segments of up to 512 bytes and St written in 256-byte runs (an element-wise gather fetches a 32-byte sector per
+// double); 16 KB of shared memory per CTA keeps a dozen CTAs resident per SM.
 // Symmetric Sigma (first_group != nullptr): a row tile only meets column groups k' >= its own first group kmin,
 // i.e. the columns j >= jmin of every degree: the rest of the row block is neither read nor written (the quadratic-form
 // kernel never touches it).
-#ifndef GB_CP_ROWS
-#define GB_CP_ROWS 32
-#define GB_CP_COLS 64
-#endif
-constexpr int CP_ROWS = GB_CP_ROWS, CP_COLS = GB_CP_COLS, CP_PITCH = CP_COLS + 1;     // odd pitch: conflict-free column reads
+constexpr int CP_ROWS = 32, CP_COLS = 64, CP_PITCH = CP_COLS + 1;     // odd pitch: conflict-free column reads
 __global__ void __launch_bounds__(256)
 gb_cov_permute_degree(const double* __restrict__ sigma, double* __restrict__ St, const int* __restrict__ perm8,
                       const int* __restrict__ goff4, const int* __restrict__ ne4, int Kp4, long long K, int nmin,
@@ -571,7 +554,7 @@ struct CovLayout {
     int Kp8 = 0, Kp4 = 0, Kg = 8, n_atiles = 0, rows_a = 0, nti = 0, hmt = 0, n_padrows = 0, n_pieces = 0;
     int nrep = 0, nout = 0, ni = 5, n_segs = 0, folded = 0;
     int* d_all = nullptr;     // one allocation; the pointers below point into it
-    int *d_perm8 = nullptr, *d_perm4 = nullptr, *d_rowgroup = nullptr, *d_goff8 = nullptr, *d_gcnt = nullptr,
+    int *d_perm8 = nullptr, *d_rowgroup = nullptr, *d_goff8 = nullptr, *d_gcnt = nullptr,
         *d_goff4 = nullptr, *d_ne4 = nullptr, *d_no4 = nullptr, *d_padrows = nullptr, *d_piece_of = nullptr,
         *d_pstart = nullptr, *d_first_group = nullptr, *d_rep = nullptr, *d_out_n = nullptr, *d_out_s = nullptr,
         *d_segs = nullptr;
@@ -715,10 +698,10 @@ int build_layout(gb_plan* p, int nmin, int row0, int nrows, int key_flags, CovLa
     c->n_padrows = (int)padrows.size();
     c->n_pieces = n_pieces;
     c->nrep = nrep; c->nout = nout; c->ni = ni;
-    constexpr int NT = 16;
-    const std::vector<int>* parts[NT] = {&perm8, &perm4, &rowgroup, &goff8, &gcnt, &goff4, &ne4, &no4, &padrows, &piece_of,
+    constexpr int NT = 15;
+    const std::vector<int>* parts[NT] = {&perm8, &rowgroup, &goff8, &gcnt, &goff4, &ne4, &no4, &padrows, &piece_of,
                                          &pstart, &first_group, &rep, &out_n, &out_s, &segs};
-    int** slots[NT] = {&c->d_perm8, &c->d_perm4, &c->d_rowgroup, &c->d_goff8, &c->d_gcnt, &c->d_goff4, &c->d_ne4, &c->d_no4,
+    int** slots[NT] = {&c->d_perm8, &c->d_rowgroup, &c->d_goff8, &c->d_gcnt, &c->d_goff4, &c->d_ne4, &c->d_no4,
                        &c->d_padrows, &c->d_piece_of, &c->d_pstart, &c->d_first_group, &c->d_rep, &c->d_out_n, &c->d_out_s,
                        &c->d_segs};
     std::vector<int> all;
@@ -801,8 +784,7 @@ extern "C" int gb_covariance_propagation_filtered(gb_plan* plan, const double* d
     CovLayout* lay = nullptr;
     {
         // an order-wise filter mixes the parity classes of a group: no fold then (GB_COV_NO_FOLD=1: never)
-        const char* nf_env = getenv("GB_COV_NO_FOLD");
-        const bool nofold = d_blocks != nullptr || (nf_env && nf_env[0] && nf_env[0] != '0');
+        const bool nofold = d_blocks != nullptr || gb_env_flag("GB_COV_NO_FOLD");
         const int key = (mirrored ? COV_KEY_MIRRORED : 0) | (symmetric ? COV_KEY_SYMMETRIC : 0) | (nofold ? COV_KEY_NOFOLD : 0);
         int rc0 = build_layout(p, nmin, row0, nrows, key, &lay);
         if (rc0) return rc0;
@@ -813,7 +795,6 @@ extern "C" int gb_covariance_propagation_filtered(gb_plan* plan, const double* d
     GB_REQUIRE(Kp4 <= 65535, "gb_covariance_propagation: degree %d is too large for this path", p->nmax);
     GB_REQUIRE((long long)n_ct * Kg * ldb < (1LL << 31),
                "gb_covariance_propagation: %d parallels at degree %d exceed the 32-bit tile index; pass row blocks", nrows, p->nmax);
-    const bool by_degree = getenv("GB_COV_PERMUTE_GATHER") == nullptr;      // the element-wise gather is a cross-check only
     const int n_pieces = lay->n_pieces, nslots = 4 * hmt;
     double *d_st = nullptr, *d_ut = nullptr, *d_ht = nullptr, *d_hpart = nullptr, *d_vpart = nullptr;
     int rc = GB_OK;
@@ -846,21 +827,15 @@ extern "C" int gb_covariance_propagation_filtered(gb_plan* plan, const double* d
         GB_LAUNCH_CHECK();
         d_ut = d_ut2;
     }
-    if (by_degree) {
-        // the padding rows of the classes are the only part of St the permutation does not write
-        if (lay->n_padrows > 0) {
-            gb_cov_zero_rows<<<dim3(n_atiles, (lay->n_padrows + 15) / 16), 128, 0, st>>>(d_st, lay->d_padrows, lay->n_padrows, Kp4);
-            GB_LAUNCH_CHECK();
-        }
-        dim3 grid(rows_a / CP_ROWS, L - nmin, (2 * p->nmax + 1 + CP_COLS - 1) / CP_COLS);
-        gb_cov_permute_degree<<<grid, 256, 0, st>>>(d_sigma, d_st, lay->d_perm8, lay->d_goff4, lay->d_ne4, Kp4, K,
-                                                               nmin, symmetric ? lay->d_first_group : nullptr);
-        GB_LAUNCH_CHECK();
-    } else {
-        dim3 grid((rows_a + 255) / 256, Kp4);
-        gb_cov_permute<<<grid, 256, 0, st>>>(d_sigma, d_st, lay->d_perm8, lay->d_perm4, rows_a, Kp4, K);
+    // the padding rows of the classes are the only part of St the permutation does not write
+    if (lay->n_padrows > 0) {
+        gb_cov_zero_rows<<<dim3(n_atiles, (lay->n_padrows + 15) / 16), 128, 0, st>>>(d_st, lay->d_padrows, lay->n_padrows, Kp4);
         GB_LAUNCH_CHECK();
     }
+    const dim3 pgrid(rows_a / CP_ROWS, L - nmin, (2 * p->nmax + 1 + CP_COLS - 1) / CP_COLS);
+    gb_cov_permute_degree<<<pgrid, 256, 0, st>>>(d_sigma, d_st, lay->d_perm8, lay->d_goff4, lay->d_ne4, Kp4, K, nmin,
+                                                 symmetric ? lay->d_first_group : nullptr);
+    GB_LAUNCH_CHECK();
     {
         QuadArgs qa;
         qa.St = d_st; qa.Ut = d_ut; qa.Hpart = d_hpart;
@@ -876,8 +851,7 @@ extern "C" int gb_covariance_propagation_filtered(gb_plan* plan, const double* d
     // longitude quadratic form.  Four-fold symmetric meridians (every grid the reference builds): W = H T is exactly the
     // Fourier stage of the synthesis on the rows (parallel, k) -- one quarter of the multiply-adds of a plain GEMM, no padded
     // spectral rows -- followed by a streaming reduction over k.  Otherwise: the GEMM with the fused reduction below.
-    const char* lon_env = getenv("GB_COV_LON_GEMM");
-    if (p->sym && !(lon_env && lon_env[0] && lon_env[0] != '0')) {
+    if (p->sym) {
         const long long Mrows = (long long)nout * kpad;
         const size_t h2_elems = (size_t)((Mrows + GB_TM - 1) / GB_TM) * p->ab_rows * GB_LDA;
         const size_t w_elems = (size_t)Mrows * p->nlon;
@@ -889,7 +863,7 @@ extern "C" int gb_covariance_propagation_filtered(gb_plan* plan, const double* d
                                                           lay->d_out_s, kpad, n_pieces, hmt, symmetric, nmin, gb_stage2_krow(p),
                                                           p->ab_rows, L);
         GB_LAUNCH_CHECK();
-        if ((rc = gb_launch_stage2_sym(p, d_h2, Mrows, d_w, st))) return rc;
+        if ((rc = gb_launch_stage2_sym(p, d_h2, Mrows, d_w, st, false))) return rc;
         const long long n = (long long)nout * p->nlon;
         gb_cov_lon_reduce<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_w, p->d_trig, d_out, kpad, p->nlp, p->nlon, n,
                                                                       take_sqrt ? 1 : 0);

@@ -246,8 +246,7 @@ static int launch_rows(const double* src, double* dst, int L, int E, const doubl
 int gb_launch_pack_tiled(const double* d_anm, double* d_x, int L, int E, const int* d_roff, int tn, int n_ct,
                          cudaStream_t st, const double* d_wn) {
     const XTiling xt{d_roff, tn, n_ct};
-    static const bool scalar_loads = getenv("GB_PACK_SCALAR") && getenv("GB_PACK_SCALAR")[0] == '1';
-    if (L <= PK_C && !scalar_loads)          // rows fetched by the TMA unit
+    if (L <= PK_C)      // rows fetched by the TMA unit
         return E <= 64 ? launch_rows<8>(d_anm, d_x, L, E, d_wn, xt, st) : launch_rows<32>(d_anm, d_x, L, E, d_wn, xt, st);
     return E <= 64 ? launch_pke<true, 8, true>(d_anm, d_x, L, E, d_wn, xt, st)
                    : launch_pke<true, 32, true>(d_anm, d_x, L, E, d_wn, xt, st);

@@ -280,8 +280,6 @@ extern "C" int gb_plan_create(gb_plan** plan, int nmax, int nlat, int nlon, cons
                 }
             }
         }
-        const char* env = getenv("GB_NO_OCTANT");
-        if (env && env[0] && env[0] != '0') oct = false;
         p->oct = oct ? 1 : 0;
         if (oct) {
             p->no = no;

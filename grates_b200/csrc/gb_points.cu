@@ -428,7 +428,7 @@ extern "C" int gb_points_synthesis(gb_points* p, const double* d_anm, int n_epoc
     if (n_epochs == 0) return GB_OK;
     GB_REQUIRE(d_anm && d_out, "gb_points_synthesis: NULL device pointer");
     GB_CUDA(cudaSetDevice(p->device));
-    if (n_epochs >= 16 && !(getenv("GB_POINTS_SIMPLE") && getenv("GB_POINTS_SIMPLE")[0] == '1')) {
+    if (n_epochs >= 16 && !gb_env_flag("GB_POINTS_SIMPLE")) {
         gb_retain_pool_memory(p->device);
         return points_synthesis_gemm(p, d_anm, n_epochs, d_out, static_cast<cudaStream_t>(stream));
     }

@@ -122,6 +122,7 @@ constexpr int T1_TM = GB_T1_TM, T1_KC = GB_T1_KC, T1_STAGES = 4;
 constexpr int T1_LDA = T1_TM + 4;    // 68
 __host__ __device__ constexpr int t1_tn(int nwn) { return 40 * nwn; }
 __host__ __device__ constexpr int t1_threads(int nwn) { return 32 * (2 * nwn + 3); }   // + copy warp + 2 Legendre warps
+__host__ __device__ constexpr int t1_ctas_per_sm(int nwn) { return nwn <= 2 ? 2 : 1; }
 __host__ __device__ constexpr size_t t1_smem(int nwn) {
     return (size_t)T1_STAGES * T1_KC * (T1_LDA + t1_tn(nwn) + 4) * sizeof(double) + 2 * T1_STAGES * sizeof(uint64_t);
 }
@@ -142,7 +143,7 @@ struct T1Tables {
 // classes (even / odd n - m: every other shared-memory row), north = even + odd, south = even - odd.  Half the
 // recursion steps and half the DMMAs for the same output; one Legendre warp per item.
 template <bool PAIRS, int NWN, bool FOLD>   // PAIRS: nlat even, rows (e, i), (e, i+1) with i even are 16-byte aligned in AB
-__global__ void __launch_bounds__(t1_threads(NWN), NWN <= 2 ? 2 : 1)
+__global__ void __launch_bounds__(t1_threads(NWN), t1_ctas_per_sm(NWN))
 gb_legendre_stage1(const double* __restrict__ X, double* __restrict__ AB, T1Tables tb, int L, int nlat, int E,
                    int ab_rows, int n_lattiles, int n_coltiles, int n_items, int polar) {
     // polar: FOLD -- number of leading 32-parallel tiles left to the unfolded launch; !FOLD -- nonzero selects the
@@ -389,20 +390,21 @@ gb_legendre_stage1(const double* __restrict__ X, double* __restrict__ AB, T1Tabl
 // gb_legendre_stage1; the degrees of a folded chunk are grouped [even n-m | odd n-m] per 8 rows, so both parity
 // classes read consecutive shared-memory rows (pitch 36 = 4 mod 16: conflict-free fragments).
 // ---------------------------------------------------------------------------------------------
+constexpr int TB_KC = 16;          // degrees per ring stage
 __host__ __device__ constexpr int tb_lda(bool fold) { return fold ? 36 : 68; }
 __host__ __device__ constexpr int tb_ctas_per_sm(int nwn, bool fold) { return nwn <= 2 ? (fold ? 3 : 2) : nwn == 3 ? 2 : 1; }
-__host__ __device__ constexpr size_t tb_stage_bytes(int nwn, bool fold, int kc) {
-    return (size_t)kc * (tb_lda(fold) + t1_tn(nwn) + 4) * sizeof(double);
+__host__ __device__ constexpr size_t tb_stage_bytes(int nwn, bool fold) {
+    return (size_t)TB_KC * (tb_lda(fold) + t1_tn(nwn) + 4) * sizeof(double);
 }
 // as many ring stages (at most 6) as the CTA's share of the 227 KB of shared memory holds
-__host__ __device__ constexpr int tb_stages(int nwn, bool fold, int kc) {
+__host__ __device__ constexpr int tb_stages(int nwn, bool fold) {
     const size_t budget = (232448 - 1024 * tb_ctas_per_sm(nwn, fold)) / tb_ctas_per_sm(nwn, fold) - 128;
-    const int s = (int)(budget / tb_stage_bytes(nwn, fold, kc));
+    const int s = (int)(budget / tb_stage_bytes(nwn, fold));
     return s > 6 ? 6 : s;
 }
 __host__ __device__ constexpr int tb_threads(int nwn) { return 32 * (2 * nwn + 1); }
-__host__ __device__ constexpr size_t tb_smem(int nwn, bool fold, int kc) {
-    return (size_t)tb_stages(nwn, fold, kc) * tb_stage_bytes(nwn, fold, kc) + 2 * tb_stages(nwn, fold, kc) * sizeof(uint64_t);
+__host__ __device__ constexpr size_t tb_smem(int nwn, bool fold) {
+    return (size_t)tb_stages(nwn, fold) * tb_stage_bytes(nwn, fold) + 2 * tb_stages(nwn, fold) * sizeof(uint64_t);
 }
 // row of degree offset nn inside a folded table / chunk: even offsets first
 __host__ __device__ __forceinline__ int tb_fold_row(int nn) { return (nn & ~7) + ((nn & 1) << 2) + ((nn & 7) >> 1); }
@@ -420,14 +422,12 @@ struct TabArgs {
 
 // MI: 8-column fragments per consumer warp (5: 40 columns; 4: shards of at most 32 epochs, whose 64 columns then carry
 // no padding fragment)
-template <bool PAIRS, int NWN, bool FOLD, int KC, int MI = 5>
+template <bool PAIRS, int NWN, bool FOLD, int MI = 5>
 __global__ void __launch_bounds__(tb_threads(NWN), tb_ctas_per_sm(NWN, FOLD))
 gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb, int L, int nlat, int E, int ab_rows,
               int n_lattiles, int n_coltiles, int n_items, int polar) {
-    constexpr int STAGES = tb_stages(NWN, FOLD, KC);
+    constexpr int KC = TB_KC, STAGES = tb_stages(NWN, FOLD);
     static_assert(STAGES >= 2, "the ring needs at least two stages");
-    const bool diag_nostore = (polar & 0x10000) != 0;   // DIAG (GB_DIAG_NOSTORE): the epilogue without its stores
-    polar &= 0xffff;
     constexpr int TN = 8 * MI * NWN, LDA = tb_lda(FOLD), LDB = TN + 4, CONSUMER_WARPS = 2 * NWN;
     constexpr int STAGE_DOUBLES = KC * (LDA + LDB);
     extern __shared__ __align__(128) unsigned char s_raw[];
@@ -585,10 +585,6 @@ gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb,
                             if (ib >= nh) continue;
                             const long long rn = (long long)e * nlat + ib;
                             const long long rs = (long long)e * nlat + (nlat - 4 - ib);
-                            if (diag_nostore) {
-                                if (ev[mi][0][0] + od[mi][0][0] + ev[mi][1][1] - od[mi][1][1] == 1.2345e300) AB[0] = 0.0;
-                                continue;
-                            }
                             gb::st_v4(AB + gb_ab_offset(rn, k, ab_rows), ev[mi][0][0] + od[mi][0][0], ev[mi][0][1] + od[mi][0][1],
                                       ev[mi][1][0] + od[mi][1][0], ev[mi][1][1] + od[mi][1][1]);
                             gb::st_v4(AB + gb_ab_offset(rs, k, ab_rows), ev[mi][1][1] - od[mi][1][1], ev[mi][1][0] - od[mi][1][0],
@@ -758,13 +754,12 @@ constexpr int Q_STAGES = 4;
 constexpr int Q_LDA = Q_TM + 4;               // 132
 constexpr int Q_LDB = Q_TN + 4;               // 36
 constexpr int Q_CONSUMER_WARPS = Q_WM * Q_WN;
-constexpr int Q_THREADS = 32 * (Q_CONSUMER_WARPS + 1);
 constexpr int Q_STAGE_DOUBLES = Q_KC * (Q_LDA + Q_LDB);
 constexpr size_t Q_SMEM = (size_t)Q_STAGES * Q_STAGE_DOUBLES * sizeof(double) + (2 * Q_STAGES + 4) * sizeof(uint64_t) + 16;
 
 struct QGroups { int off[5]; };
 
-// EW ("epilogue warps", the default): 16 warps.  The eight consumer warps never store to global memory: a finished
+// 16 warps.  The eight consumer warps never store to global memory: a finished
 // accumulator tile is parked in tensor memory (thread-private columns, gb::tmem_st16; double buffered: 2 x 2 x 128 of
 // the 512 columns per sub-partition) and the warp goes straight back to the next tile's K loop.  Four epilogue warps,
 // one per sub-partition (a warp reaches the tensor-memory lanes 32 (warp % 4) .. only), read the tile back, apply the
@@ -772,7 +767,6 @@ struct QGroups { int off[5]; };
 // LSU to drain its predecessors: 13 % of the consumers' time in the direct kernel) lands on warps that have a whole
 // tile period to absorb it.  Registers are rebalanced with setmaxnreg: the kernel starts with 128 per thread
 // (512 threads), consumers grow to 168, epilogue warps shrink to 104, the producer's warpgroup to 40.
-// !EW: the direct kernel (nine warps, epilogue in the consumers), kept for comparison (GB_S2_DIRECT_EPILOGUE=1).
 // Work list of a CTA: whole tiles t = b, b + grid, ... of the full rounds; when the last, partial round holds at most
 // grid / 2 tiles they are cut into halves of 64 rows, one per CTA, so that the tail costs half a tile period.
 struct QWork {
@@ -803,8 +797,7 @@ struct QWork {
 };
 
 constexpr int QE_THREADS = 512;
-template <bool EW>
-__global__ void __launch_bounds__(EW ? QE_THREADS : Q_THREADS, 1)
+__global__ void __launch_bounds__(QE_THREADS, 1)
 gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* __restrict__ trig_q_t, int kpad_s,
                       QGroups grp, double* __restrict__ out, long long M, int nlon, int nq, int n_mtiles,
                       int n_ntiles, int wide) {
@@ -817,7 +810,7 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(tempty + 2);
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    constexpr int PRODUCER_WARP = EW ? 12 : Q_CONSUMER_WARPS;
+    constexpr int PRODUCER_WARP = 12;
     if (threadIdx.x == 0) {
         for (int s = 0; s < Q_STAGES; ++s) {
             gb::mbar_init(&full[s], 1);
@@ -829,10 +822,10 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
         }
         gb::fence_mbar_init();
     }
-    if (EW && warp == 0) gb::tmem_alloc(s_tmem, 512);
-    if (EW) gb::tmem_fence_before_sync();
+    if (warp == 0) gb::tmem_alloc(s_tmem, 512);
+    gb::tmem_fence_before_sync();
     __syncthreads();
-    if (EW) gb::tmem_fence_after_sync();
+    gb::tmem_fence_after_sync();
     gb::griddep_wait();                 // AB comes from stage 1; `out` may still be read by whatever ran before
     gb::griddep_launch_dependents();
 
@@ -875,7 +868,7 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
     auto warp_row0 = [](int wm, int half) { return half < 0 ? wm * 32 : half * 64 + wm * 16; };
 
     if (warp >= PRODUCER_WARP) {
-        if (EW) asm volatile("setmaxnreg.dec.sync.aligned.u32 40;\n");
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 40;\n");
         if (warp == PRODUCER_WARP && lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
@@ -902,7 +895,7 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
                 }
             }
         }
-    } else if (EW && warp >= Q_CONSUMER_WARPS) {
+    } else if (warp >= Q_CONSUMER_WARPS) {
         // ===== epilogue warp of sub-partition sp: the tiles of consumer warps sp and sp + 4 =====
         asm volatile("setmaxnreg.dec.sync.aligned.u32 104;\n");
         const int sp = warp & 3;
@@ -933,14 +926,14 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
             if (++tb == 2) { tb = 0; tphase ^= 1u; }
         }
     } else {
-        if (EW) asm volatile("setmaxnreg.inc.sync.aligned.u32 168;\n");
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 168;\n");
         const int wm = warp / Q_WN;
         const int wn = warp % Q_WN;
         const int g = lane >> 2, q = lane & 3;
         int stage = 0, tb = 0;
         uint32_t phase = 0, tphase = 0;
         // one tile: MI 8-row slabs per warp (4: whole tile, 2: half tile)
-        auto run_tile = [&](auto mi_tag, long long mt, int nt, int half) {
+        auto run_tile = [&](auto mi_tag, int half) {
             constexpr int MI = decltype(mi_tag)::value;
             const int r0 = warp_row0(wm, half);
             double acc[4][MI][2][2];   // [set][mi][ni][2]
@@ -985,51 +978,35 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
                     k0 += kc;
                 }
             }
-            if (EW) {
-                // park the tile: this warp's 128 columns of buffer tb (lanes 32 (warp % 4) .., columns 256 tb + 128 (warp / 4) ..)
-                gb::mbar_wait(&tempty[tb], tphase ^ 1u);
-                gb::tmem_fence_after_sync();
-                const uint32_t taddr = *s_tmem + ((uint32_t)(32 * (warp & 3)) << 16) + (uint32_t)(tb * 256 + (warp >> 2) * 128);
+            // park the tile: this warp's 128 columns of buffer tb (lanes 32 (warp % 4) .., columns 256 tb + 128 (warp / 4) ..)
+            gb::mbar_wait(&tempty[tb], tphase ^ 1u);
+            gb::tmem_fence_after_sync();
+            const uint32_t taddr = *s_tmem + ((uint32_t)(32 * (warp & 3)) << 16) + (uint32_t)(tb * 256 + (warp >> 2) * 128);
 #pragma unroll
-                for (int mi = 0; mi < MI; ++mi) {
-                    double v[16];
+            for (int mi = 0; mi < MI; ++mi) {
+                double v[16];
 #pragma unroll
-                    for (int s = 0; s < 4; ++s)
+                for (int s = 0; s < 4; ++s)
 #pragma unroll
-                        for (int c = 0; c < 4; ++c) v[4 * s + c] = acc[s][mi][c >> 1][c & 1];
-                    gb::tmem_st16(taddr + 32u * mi, v);
-                }
-                gb::tmem_wait_st();
-                gb::tmem_fence_before_sync();
-                __syncwarp();
-                if (lane == 0) gb::mbar_arrive(&tfull[tb]);
-                if (++tb == 2) { tb = 0; tphase ^= 1u; }
-            } else {
-                const long long row0 = mt * Q_TM + r0 + g;
-                const int jq = nt * Q_TN + wn * 16 + 4 * q;
-#pragma unroll
-                for (int mi = 0; mi < MI; ++mi) {
-                    double v[16];
-#pragma unroll
-                    for (int s = 0; s < 4; ++s)
-#pragma unroll
-                        for (int c = 0; c < 4; ++c) v[4 * s + c] = acc[s][mi][c >> 1][c & 1];
-                    emit_row(row0 + mi * 8, jq, v);
-                }
+                    for (int c = 0; c < 4; ++c) v[4 * s + c] = acc[s][mi][c >> 1][c & 1];
+                gb::tmem_st16(taddr + 32u * mi, v);
             }
+            gb::tmem_wait_st();
+            gb::tmem_fence_before_sync();
+            __syncwarp();
+            if (lane == 0) gb::mbar_arrive(&tfull[tb]);
+            if (++tb == 2) { tb = 0; tphase ^= 1u; }
         };
         long long mt;
         int nt, half;
         for (long long i = 0; work.get(blockIdx.x, i, mt, nt, half); ++i) {
-            if (half < 0) run_tile(std::integral_constant<int, 4>{}, mt, nt, half);
-            else run_tile(std::integral_constant<int, 2>{}, mt, nt, half);
+            if (half < 0) run_tile(std::integral_constant<int, 4>{}, half);
+            else run_tile(std::integral_constant<int, 2>{}, half);
         }
     }
-    if (EW) {
-        gb::tmem_fence_before_sync();
-        __syncthreads();
-        if (warp == 0) gb::tmem_dealloc(*s_tmem, 512);
-    }
+    gb::tmem_fence_before_sync();
+    __syncthreads();
+    if (warp == 0) gb::tmem_dealloc(*s_tmem, 512);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1043,7 +1020,7 @@ gb_fourier_stage2_sym(const double* __restrict__ AB, int ab_rows, const double* 
 // CO = AS, SO = BC), hence eight meridians: the even orders cost half the multiply-adds of the quadrant kernel, the odd
 // ones the same -- 3/4 in total -- and an odd k-step feeds two accumulator sets from ONE coefficient fragment (8 LDS per
 // 16 DMMA instead of 6 per 8).
-// Same structure as gb_fourier_stage2_sym<EW>: persistent, 8 consumer warps (4 x 2, 32 rows x 16 octant columns), 4
+// Same structure as gb_fourier_stage2_sym: persistent, 8 consumer warps (4 x 2, 32 rows x 16 octant columns), 4
 // epilogue warps, 1 producer lane, 4-stage ring (coefficient chunk + one or two table chunks).  CTA tile 128 rows x 32 octant
 // columns = 128 x 256 outputs.  A tile is parked in tensor memory in two halves (the four even sets after the even groups,
 // the four odd sets at the end: 2 x 128 columns per consumer warp, single buffered -- the epilogue warp of the lane quarter
@@ -1411,24 +1388,19 @@ gb_legendre_table_kernel(double* __restrict__ out, const double* __restrict__ ct
     });
 }
 
-bool env_flag(const char* name) {
-    const char* v = getenv(name);
-    return v && v[0] && v[0] != '0';
-}
-
 }  // namespace
 
+constexpr size_t PTAB_MAX_BYTES = (size_t)2048 << 20;     // memory budget of one Legendre table
+
 // Build (once) the Legendre table of `kind` (gb_common.cuh: 0 folded tiles, 1 polar-cap tiles, 2 plain tiles).
-// Returns 1 if the table exists, 0 if it is over the memory budget (GB_PTAB_MAX_MB, default 2048: the caller then runs
-// the on-the-fly recursion kernel), < 0 on error (-code).
+// Returns 1 if the table exists, 0 if it is over PTAB_MAX_BYTES or cannot be allocated (the caller then runs the
+// on-the-fly recursion kernel), < 0 on error (-code).
 static int ensure_ptab(gb_plan* p, int kind, int n_tiles, int tile0, cudaStream_t st) {
     if (p->ptab_state[kind] != 0) return p->ptab_state[kind] > 0 ? 1 : 0;
     const int L = p->L;
     const int lda = kind == 0 ? 36 : 68, per_tile = kind == 0 ? 32 : 64;
     const size_t elems = (size_t)n_tiles * p->ptab_rtot * lda;
-    const char* lim = getenv("GB_PTAB_MAX_MB");
-    const double max_mb = lim ? atof(lim) : 2048.0;
-    if (elems * sizeof(double) > max_mb * 1048576.0) {
+    if (elems * sizeof(double) > PTAB_MAX_BYTES) {
         p->ptab_state[kind] = -1;
         return 0;
     }
@@ -1458,6 +1430,119 @@ struct SynthesisFilter {
     int nf;
 };
 
+// Column tiling of the stage-1 items: NWN column warps of MI 8-column fragments, tn = 8 MI NWN columns (e, cos|sin).
+struct S1Tiling {
+    int nwn, mi;
+    int tn() const { return 8 * mi * nwn; }
+};
+
+// Narrow batches (at most 80 epochs) run 80-column items, several CTAs per SM; wider batches 240-column items.  The
+// table-fed kernel on folded grids without polar caps (tab_fold) has two more tilings.
+static S1Tiling stage1_tiling(int E, bool tab_fold) {
+    const int cols = 2 * E;
+    if (tab_fold && cols <= 64) return {2, 4};      // shards of at most 32 epochs: 64-column items (no padding fragment)
+    // 41 .. 60 epochs: ONE 120-column tile per order pair and latitude tile, two CTAs per SM (80-column tiles would leave
+    // a second, mostly empty round of items)
+    if (tab_fold && cols > 80 && cols <= 120) return {3, 5};
+    return cols <= 160 ? S1Tiling{2, 5} : S1Tiling{6, 5};
+}
+
+// what the stage-1 launches of one synthesis share
+struct S1Launch {
+    gb_plan* p;
+    const int* krow;
+    int E, n_coltiles;
+    cudaStream_t st;
+};
+
+// Table-fed stage 1 over `lattiles` latitude tiles of the plan's table of `kind`.  Threads and shared memory follow from
+// the template arguments.
+template <bool PAIRS, int NWN, bool FOLD, int MI = 5>
+static int launch_tab(const S1Launch& a, int kind, int lattiles, int items, int polar) {
+    const gb_plan* p = a.p;
+    auto kernel = gb_stage1_tab<PAIRS, NWN, FOLD, MI>;
+    const int max_ctas = tb_ctas_per_sm(NWN, FOLD) * p->sm_count;
+    const int grid = items < max_ctas ? items : max_ctas;
+    size_t smem = tb_smem(NWN, FOLD);
+    // Fewer items than CTA slots (a narrow shard): the CTAs are launched while the pack kernel still holds part of every
+    // SM (programmatic dependent launch) and the block scheduler fills whatever is free first -- three CTAs on some SMs,
+    // one on others, and the crowded SMs finish last.  Asking for more shared memory than a CTA needs caps the CTAs per
+    // SM at the even share.
+    const int per_sm = (grid + p->sm_count - 1) / p->sm_count;
+    if (per_sm < tb_ctas_per_sm(NWN, FOLD)) {
+        const size_t forbid = 233472 / (size_t)(per_sm + 1) - 1024 + 256;      // per_sm + 1 CTAs no longer fit
+        const size_t allow = 233472 / (size_t)per_sm - 1024;                    // per_sm CTAs still do
+        if (forbid > smem && forbid <= allow && forbid <= 232448) smem = forbid;
+    }
+    const TabArgs ta{p->d_ptab[kind], p->d_ptab_roff, p->ptab_rtot * tb_lda(FOLD), a.krow};
+    GB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GB_CUDA(gb_launch_pdl(kernel, dim3(grid), dim3(tb_threads(NWN)), smem, a.st, p->d_x, p->d_ab, ta, p->L, p->nlat, a.E,
+                          p->ab_rows, lattiles, a.n_coltiles, items, polar));
+    GB_LAUNCH_CHECK();
+    return GB_OK;
+}
+
+// Stage 1 with the Legendre recursion on the fly (no table), same items as launch_tab with MI = 5.
+template <bool PAIRS, int NWN, bool FOLD>
+static int launch_otf(const S1Launch& a, int lattiles, int items, int polar) {
+    const gb_plan* p = a.p;
+    const int max_ctas = t1_ctas_per_sm(NWN) * p->sm_count;
+    const int grid = items < max_ctas ? items : max_ctas;
+    const T1Tables tb{p->d_ct_pad, p->d_kn_t, p->d_pmm_t, p->d_rec_a, p->d_rec_b, p->d_zero, a.krow, p->nlat_pad, p->lpad};
+    GB_CUDA(cudaFuncSetAttribute(gb_legendre_stage1<PAIRS, NWN, FOLD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)t1_smem(NWN)));
+    gb_legendre_stage1<PAIRS, NWN, FOLD><<<grid, t1_threads(NWN), t1_smem(NWN), a.st>>>(
+        p->d_x, p->d_ab, tb, p->L, p->nlat, a.E, p->ab_rows, lattiles, a.n_coltiles, items, polar);
+    GB_LAUNCH_CHECK();
+    return GB_OK;
+}
+
+// the eight-fold symmetric stage 2: plan gate + override
+static bool stage2_octant(const gb_plan* p) { return p->sym && p->oct && !gb_env_flag("GB_S2_QUADRANT"); }
+
+// spectral row k = 2m + cs -> row of the AB layout the symmetric Fourier stage of this plan reads (octant or quadrant order)
+const int* gb_stage2_krow(const gb_plan* p) { return stage2_octant(p) ? p->d_krow_oct : p->d_krow_sym; }
+
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_maybe_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                    Args... args) {
+    if (pdl) return gb_launch_pdl(kernel, grid, block, smem, st, args...);
+    kernel<<<grid, block, smem, st>>>(args...);
+    return cudaSuccess;      // launch errors: GB_LAUNCH_CHECK
+}
+
+// The symmetric Fourier stage on any row set in the AB layout: d_out[row][j] = sum_k d_ab[row][k] trig[k][j], rows
+// [0, M).  The synthesis launches it behind its stage 1 with programmatic dependent launch (pdl); the covariance
+// propagation, whose longitude quadratic form starts with the same contraction, launches it plainly.
+int gb_launch_stage2_sym(gb_plan* p, const double* d_ab, long long M, double* d_out, cudaStream_t st, bool pdl) {
+    GB_REQUIRE(p->sym, "gb_launch_stage2_sym: the plan's meridians are not four-fold symmetric");
+    const bool oct = stage2_octant(p);
+    const int n_mtiles = (int)((M + Q_TM - 1) / Q_TM);
+    const int n_ntiles = oct ? p->n_otiles : p->n_qtiles;
+    const long long n_tiles = (long long)n_mtiles * n_ntiles;
+    if (n_tiles == 0) return GB_OK;
+    const int grid = (int)((n_tiles < p->sm_count) ? n_tiles : p->sm_count);
+    // 32-byte stores need 32-byte aligned rows: the base pointer, and a meridian count that keeps every row aligned
+    const bool out32 = reinterpret_cast<uintptr_t>(d_out) % 32 == 0;
+    if (oct) {
+        OGroups grp;
+        for (int g = 0; g < 7; ++g) grp.off[g] = p->ogrp_off[g];
+        const int wide = out32 && p->nlon % 16 == 0;
+        GB_CUDA(cudaFuncSetAttribute(gb_fourier_stage2_oct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O_SMEM));
+        GB_CUDA(launch_maybe_pdl(pdl, gb_fourier_stage2_oct, dim3(grid), dim3(QE_THREADS), O_SMEM, st, d_ab, p->ab_rows,
+                                 p->d_trig_o_t, p->kpad_o, grp, d_out, M, p->nlon, p->no, n_mtiles, n_ntiles, wide));
+    } else {
+        QGroups grp;
+        for (int g = 0; g < 5; ++g) grp.off[g] = p->grp_off[g];
+        const int wide = out32 && p->nlon % 8 == 0;
+        GB_CUDA(cudaFuncSetAttribute(gb_fourier_stage2_sym, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
+        GB_CUDA(launch_maybe_pdl(pdl, gb_fourier_stage2_sym, dim3(grid), dim3(QE_THREADS), Q_SMEM, st, d_ab, p->ab_rows,
+                                 p->d_trig_q_t, p->kpad_s, grp, d_out, M, p->nlon, p->nq, n_mtiles, n_ntiles, wide));
+    }
+    GB_LAUNCH_CHECK();
+    return GB_OK;
+}
+
 static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_out, cudaStream_t st,
                             const double* d_wn = nullptr, const SynthesisFilter* flt = nullptr) {
     const int L = p->L;
@@ -1467,35 +1552,22 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
         if (rca) return rca;
     }
     cudaEvent_t* prof = (p->prof_ev && p->prof_count < p->prof_capacity) ? p->prof_ev + (size_t)p->prof_count * 4 : nullptr;
-    const bool naive2 = env_flag("GB_NAIVE_STAGE2");
-    const bool use_sym = p->sym && !naive2 && !env_flag("GB_NO_SYMMETRY");
-    const bool use_oct = use_sym && p->oct && !env_flag("GB_S2_QUADRANT");      // eight-fold symmetry (plan gate + override)
-    // (gb_launch_stage2_sym / gb_stage2_krow below apply the same rule for the covariance propagation)
-    const int* d_krow = use_oct ? p->d_krow_oct : use_sym ? p->d_krow_sym : p->d_krow_id;
-    // stage-1 tiling: narrow batches (at most 80 epochs) run 80-column items, several CTAs per SM
-    const bool simple1 = env_flag("GB_SIMPLE_STAGE1");
-    const char* s1_nwn = getenv("GB_S1_NWN");                       // experiment: column warps of the wide items (2, 3, 6)
-    const int nwn_wide = s1_nwn ? atoi(s1_nwn) : 6;
-    const bool fold = p->fold_ns && !env_flag("GB_NO_FOLD");        // equatorial symmetry: 32 northern parallels per item
-    const bool tab_fold = fold && p->fold_cap == 0 && !simple1 && !env_flag("GB_S1_ONTHEFLY");
-    // 41 .. 60 epochs on folded grids without polar caps: ONE 120-column tile per order pair and latitude tile, two CTAs
-    // per SM (80-column tiles would leave a second, mostly empty round of items)
-    const bool mid = tab_fold && !env_flag("GB_S1_WIDE") &&
-                     (nwn_wide == 3 || (!s1_nwn && 2 * E > t1_tn(2) && 2 * E <= t1_tn(3)));
-    const bool narrow = ((2 * E <= 2 * t1_tn(2) && !env_flag("GB_S1_WIDE")) || nwn_wide == 2) && !mid;
-    // shards of at most 32 epochs on folded grids without polar caps: 64-column items (no padding fragment)
-    const bool narrow32 = narrow && tab_fold && 2 * E <= 64 && !env_flag("GB_S1_MI5");
-    const int tn = narrow32 ? 64 : narrow ? t1_tn(2) : mid ? t1_tn(3) : t1_tn(6);
-    const int n_coltiles = (2 * E + tn - 1) / tn;
+    const bool naive2 = gb_env_flag("GB_NAIVE_STAGE2");
+    const bool use_sym = p->sym && !naive2 && !gb_env_flag("GB_NO_SYMMETRY");
+    const int* d_krow = use_sym ? gb_stage2_krow(p) : p->d_krow_id;
+    const bool simple1 = gb_env_flag("GB_SIMPLE_STAGE1");
+    const bool fold = p->fold_ns && !gb_env_flag("GB_NO_FOLD");     // equatorial symmetry: 32 northern parallels per item
     const int cap_tiles = fold ? p->fold_cap / 32 : 0;              // polar tiles that stay unfolded
     const int n_lattiles = fold ? (p->nlat / 2 + 31) / 32 - cap_tiles : (p->nlat + T1_TM - 1) / T1_TM;
-    const int n_items = (L + 1) / 2 * n_lattiles * n_coltiles;     // order pairs (p, nmax - p) x tiles
-    const int cap_items = (L + 1) / 2 * cap_tiles * n_coltiles;
-    const bool pairs = p->nlat % 2 == 0;
-    // the Legendre table(s) of this tiling; 0 = over budget -> on-the-fly recursion
-    int have_tab = (simple1 || env_flag("GB_S1_ONTHEFLY")) ? 0 : ensure_ptab(p, fold ? 0 : 2, n_lattiles, cap_tiles, st);
+    // the Legendre table(s) of these latitude tiles; 0 = over budget -> on-the-fly recursion
+    int have_tab = (simple1 || gb_env_flag("GB_S1_ONTHEFLY")) ? 0 : ensure_ptab(p, fold ? 0 : 2, n_lattiles, cap_tiles, st);
     if (have_tab > 0 && cap_tiles > 0) have_tab = ensure_ptab(p, 1, cap_tiles, 0, st);
     if (have_tab < 0) return -have_tab;
+    const S1Tiling tiling = stage1_tiling(E, have_tab && fold && p->fold_cap == 0);
+    const int tn = tiling.tn();
+    const int n_coltiles = (2 * E + tn - 1) / tn;
+    const int n_items = (L + 1) / 2 * n_lattiles * n_coltiles;     // order pairs (p, nmax - p) x tiles
+    const int cap_items = (L + 1) / 2 * cap_tiles * n_coltiles;
     if (have_tab) {
         // tiled X: pad rows, pad columns and the (non-existent) sine plane of order 0 are never written by the pack
         const long long key = ((long long)E << 16) | tn;
@@ -1527,82 +1599,39 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
                                                            p->d_rb, p->d_rc, d_krow, L, p->nlat, E, p->ab_rows);
         GB_LAUNCH_CHECK();
     } else {
-        if (have_tab) {
-            auto launch_tab = [&](auto kernel, int nwn, bool kfold, int kc, int kind, int lattiles, int items, int polar) -> int {
-                const int max_ctas = tb_ctas_per_sm(nwn, kfold) * p->sm_count;
-                const int grid = items < max_ctas ? items : max_ctas;
-                size_t smem = tb_smem(nwn, kfold, kc);
-                // Fewer items than CTA slots (a narrow shard): the CTAs are launched while the pack kernel still holds part
-                // of every SM (programmatic dependent launch) and the block scheduler fills whatever is free first -- three
-                // CTAs on some SMs, one on others, and the crowded SMs finish last.  Asking for more shared memory than a
-                // CTA needs caps the CTAs per SM at the even share.
-                const int per_sm = (grid + p->sm_count - 1) / p->sm_count;
-                if (per_sm < tb_ctas_per_sm(nwn, kfold) && !env_flag("GB_S1_NO_SPREAD")) {
-                    const size_t forbid = 233472 / (size_t)(per_sm + 1) - 1024 + 256;      // per_sm + 1 CTAs no longer fit
-                    const size_t allow = 233472 / (size_t)per_sm - 1024;                    // per_sm CTAs still do
-                    if (forbid > smem && forbid <= allow && forbid <= 232448) smem = forbid;
-                }
-                TabArgs ta{p->d_ptab[kind], p->d_ptab_roff, p->ptab_rtot * tb_lda(kfold), d_krow};
-                GB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                GB_CUDA(gb_launch_pdl(kernel, dim3(grid), dim3(tb_threads(nwn)), smem, st, p->d_x, p->d_ab, ta, L, p->nlat, E,
-                                      p->ab_rows, lattiles, n_coltiles, items, polar));
-                GB_LAUNCH_CHECK();
-                return GB_OK;
-            };
-            const bool kc32 = env_flag("GB_S1_KC32");
-            int rc = GB_OK;
-            if (fold) {
-                rc = narrow32 ? launch_tab(gb_stage1_tab<true, 2, true, 16, 4>, 2, true, 16, 0, n_lattiles, n_items, cap_tiles)
-                     : narrow ? launch_tab(gb_stage1_tab<true, 2, true, 16>, 2, true, 16, 0, n_lattiles, n_items, cap_tiles)
-                     : mid ? launch_tab(gb_stage1_tab<true, 3, true, 16>, 3, true, 16, 0, n_lattiles, n_items, cap_tiles)
-                     : kc32 ? launch_tab(gb_stage1_tab<true, 6, true, 32>, 6, true, 32, 0, n_lattiles, n_items, cap_tiles)
-                            : launch_tab(gb_stage1_tab<true, 6, true, 16>, 6, true, 16, 0, n_lattiles, n_items, cap_tiles | (env_flag("GB_DIAG_NOSTORE") ? 0x10000 : 0));
-                if (!rc && cap_tiles > 0)
-                    rc = narrow ? launch_tab(gb_stage1_tab<true, 2, false, 16>, 2, false, 16, 1, cap_tiles, cap_items, 1)
-                                : launch_tab(gb_stage1_tab<true, 6, false, 16>, 6, false, 16, 1, cap_tiles, cap_items, 1);
-            } else if (narrow) {
-                rc = pairs ? launch_tab(gb_stage1_tab<true, 2, false, 16>, 2, false, 16, 2, n_lattiles, n_items, 0)
-                           : launch_tab(gb_stage1_tab<false, 2, false, 16>, 2, false, 16, 2, n_lattiles, n_items, 0);
-            } else {
-                rc = pairs ? launch_tab(gb_stage1_tab<true, 6, false, 16>, 6, false, 16, 2, n_lattiles, n_items, 0)
-                           : launch_tab(gb_stage1_tab<false, 6, false, 16>, 6, false, 16, 2, n_lattiles, n_items, 0);
-            }
-            if (rc) return rc;
+        // the polar caps (parallels whose mirror image is not close enough in the reference's tables) run the unfolded
+        // kernel on tiles of 32 northern parallels + their 32 mirror images (polar = 1); tiling.nwn is 2 or 6 outside
+        // the first branch
+        const S1Launch a{p, d_krow, E, n_coltiles, st};
+        const bool pairs = p->nlat % 2 == 0;
+        const bool nw2 = tiling.nwn == 2;
+        int rc;
+        if (have_tab && fold) {
+            rc = tiling.mi == 4 ? launch_tab<true, 2, true, 4>(a, 0, n_lattiles, n_items, cap_tiles)
+                 : nw2 ? launch_tab<true, 2, true>(a, 0, n_lattiles, n_items, cap_tiles)
+                 : tiling.nwn == 3 ? launch_tab<true, 3, true>(a, 0, n_lattiles, n_items, cap_tiles)
+                                   : launch_tab<true, 6, true>(a, 0, n_lattiles, n_items, cap_tiles);
+            if (!rc && cap_tiles > 0)
+                rc = nw2 ? launch_tab<true, 2, false>(a, 1, cap_tiles, cap_items, 1)
+                         : launch_tab<true, 6, false>(a, 1, cap_tiles, cap_items, 1);
+        } else if (have_tab) {
+            rc = nw2 ? (pairs ? launch_tab<true, 2, false>(a, 2, n_lattiles, n_items, 0)
+                              : launch_tab<false, 2, false>(a, 2, n_lattiles, n_items, 0))
+                     : (pairs ? launch_tab<true, 6, false>(a, 2, n_lattiles, n_items, 0)
+                              : launch_tab<false, 6, false>(a, 2, n_lattiles, n_items, 0));
+        } else if (fold) {              // implies an even number of parallels
+            rc = nw2 ? launch_otf<true, 2, true>(a, n_lattiles, n_items, cap_tiles)
+                     : launch_otf<true, 6, true>(a, n_lattiles, n_items, cap_tiles);
+            if (!rc && cap_tiles > 0)
+                rc = nw2 ? launch_otf<true, 2, false>(a, cap_tiles, cap_items, 1)
+                         : launch_otf<true, 6, false>(a, cap_tiles, cap_items, 1);
         } else {
-        const int max_ctas = narrow ? 2 * p->sm_count : p->sm_count;
-        const int grid = n_items < max_ctas ? n_items : max_ctas;
-        T1Tables tb{p->d_ct_pad, p->d_kn_t, p->d_pmm_t, p->d_rec_a, p->d_rec_b, p->d_zero, d_krow, p->nlat_pad, p->lpad};
-#define GB_S1_LAUNCH(PAIRS, NWN, FOLD)                                                                               \
-    do {                                                                                                             \
-        GB_CUDA(cudaFuncSetAttribute(gb_legendre_stage1<PAIRS, NWN, FOLD>,                                           \
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t1_smem(NWN)));               \
-        gb_legendre_stage1<PAIRS, NWN, FOLD><<<grid, t1_threads(NWN), t1_smem(NWN), st>>>(                            \
-            p->d_x, p->d_ab, tb, L, p->nlat, E, p->ab_rows, n_lattiles, n_coltiles, n_items, cap_tiles);             \
-    } while (0)
-        if (fold) {                     // implies an even number of parallels
-            if (narrow) GB_S1_LAUNCH(true, 2, true); else GB_S1_LAUNCH(true, 6, true);
-            if (cap_tiles > 0) {
-                // the polar caps (parallels whose mirror image is not close enough in the reference's tables): the
-                // unfolded kernel on tiles of 32 northern parallels + their 32 mirror images
-                const int cap_grid = cap_items < max_ctas ? cap_items : max_ctas;
-#define GB_S1_CAP(NWN)                                                                                               \
-    do {                                                                                                             \
-        GB_CUDA(cudaFuncSetAttribute(gb_legendre_stage1<true, NWN, false>,                                           \
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t1_smem(NWN)));               \
-        gb_legendre_stage1<true, NWN, false><<<cap_grid, t1_threads(NWN), t1_smem(NWN), st>>>(                        \
-            p->d_x, p->d_ab, tb, L, p->nlat, E, p->ab_rows, cap_tiles, n_coltiles, cap_items, 1);                    \
-    } while (0)
-                if (narrow) GB_S1_CAP(2); else GB_S1_CAP(6);
-#undef GB_S1_CAP
-            }
-        } else if (narrow) {
-            if (pairs) GB_S1_LAUNCH(true, 2, false); else GB_S1_LAUNCH(false, 2, false);
-        } else {
-            if (pairs) GB_S1_LAUNCH(true, 6, false); else GB_S1_LAUNCH(false, 6, false);
+            rc = nw2 ? (pairs ? launch_otf<true, 2, false>(a, n_lattiles, n_items, 0)
+                              : launch_otf<false, 2, false>(a, n_lattiles, n_items, 0))
+                     : (pairs ? launch_otf<true, 6, false>(a, n_lattiles, n_items, 0)
+                              : launch_otf<false, 6, false>(a, n_lattiles, n_items, 0));
         }
-#undef GB_S1_LAUNCH
-        GB_LAUNCH_CHECK();
-        }
+        if (rc) return rc;
     }
     if (prof) GB_CUDA(cudaEventRecord(prof[2], st));
     if (naive2) {
@@ -1610,33 +1639,9 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
         gb_fourier_stage2_naive<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(p->d_ab, p->ab_rows, p->d_trig, p->nlp,
                                                                                 p->kpad, d_out, M, p->nlon);
         GB_LAUNCH_CHECK();
-    } else if (use_oct) {
-        const int n_mtiles = (int)((M + Q_TM - 1) / Q_TM);
-        const int n_ntiles = p->n_otiles;
-        const long long n_tiles = (long long)n_mtiles * n_ntiles;
-        const int grid = (int)((n_tiles < p->sm_count) ? n_tiles : p->sm_count);
-        OGroups grp;
-        for (int g = 0; g < 7; ++g) grp.off[g] = p->ogrp_off[g];
-        GB_CUDA(cudaFuncSetAttribute(gb_fourier_stage2_oct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O_SMEM));
-        const int wide = (reinterpret_cast<uintptr_t>(d_out) % 32 == 0 && p->nlon % 16 == 0 && !env_flag("GB_S2_NARROW_STORES")) ? 1 : 0;
-        GB_CUDA(gb_launch_pdl(gb_fourier_stage2_oct, dim3(grid), dim3(QE_THREADS), O_SMEM, st, p->d_ab, p->ab_rows, p->d_trig_o_t,
-                              p->kpad_o, grp, d_out, M, p->nlon, p->no, n_mtiles, n_ntiles, wide));
-        GB_LAUNCH_CHECK();
     } else if (use_sym) {
-        const int n_mtiles = (int)((M + Q_TM - 1) / Q_TM);
-        const int n_ntiles = p->n_qtiles;
-        const long long n_tiles = (long long)n_mtiles * n_ntiles;
-        const int grid = (int)((n_tiles < p->sm_count) ? n_tiles : p->sm_count);
-        QGroups grp;
-        for (int g = 0; g < 5; ++g) grp.off[g] = p->grp_off[g];
-        const bool defer = !env_flag("GB_S2_DIRECT_EPILOGUE");
-        auto s2_kernel = defer ? gb_fourier_stage2_sym<true> : gb_fourier_stage2_sym<false>;
-        GB_CUDA(cudaFuncSetAttribute(s2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-        // 32-byte stores need 32-byte aligned rows: nlon is a multiple of 8 here, so only the base pointer matters
-        const int wide = (reinterpret_cast<uintptr_t>(d_out) % 32 == 0 && p->nlon % 8 == 0 && !env_flag("GB_S2_NARROW_STORES")) ? 1 : 0;
-        GB_CUDA(gb_launch_pdl(s2_kernel, dim3(grid), dim3(defer ? QE_THREADS : Q_THREADS), Q_SMEM, st, p->d_ab, p->ab_rows,
-                              p->d_trig_q_t, p->kpad_s, grp, d_out, M, p->nlon, p->nq, n_mtiles, n_ntiles, wide));
-        GB_LAUNCH_CHECK();
+        int rc = gb_launch_stage2_sym(p, p->d_ab, M, d_out, st, true);
+        if (rc) return rc;
     } else {
         gbgemm::Shape sh;
         sh.A_t = p->d_ab;
@@ -1658,50 +1663,12 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
     return GB_OK;
 }
 
-// The symmetric Fourier stage on any row set in the AB layout (used by the covariance propagation, whose longitude
-// quadratic form starts with the same contraction): d_out[row][j] = sum_k d_ab[row][k] trig[k][j], rows [0, M).
-static bool stage2_octant(const gb_plan* p) { return p->sym && p->oct && !env_flag("GB_S2_QUADRANT"); }
-
-// spectral row k = 2m + cs -> row of the AB layout the symmetric Fourier stage of this plan reads (octant or quadrant order)
-const int* gb_stage2_krow(const gb_plan* p) { return stage2_octant(p) ? p->d_krow_oct : p->d_krow_sym; }
-
-int gb_launch_stage2_sym(gb_plan* p, const double* d_ab, long long M, double* d_out, cudaStream_t st) {
-    GB_REQUIRE(p->sym, "gb_launch_stage2_sym: the plan's meridians are not four-fold symmetric");
-    if (stage2_octant(p)) {
-        const int n_mtiles = (int)((M + Q_TM - 1) / Q_TM);
-        const int n_ntiles = p->n_otiles;
-        const long long n_tiles = (long long)n_mtiles * n_ntiles;
-        if (n_tiles == 0) return GB_OK;
-        const int grid = (int)((n_tiles < p->sm_count) ? n_tiles : p->sm_count);
-        OGroups grp;
-        for (int g = 0; g < 7; ++g) grp.off[g] = p->ogrp_off[g];
-        GB_CUDA(cudaFuncSetAttribute(gb_fourier_stage2_oct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O_SMEM));
-        const int wide = (reinterpret_cast<uintptr_t>(d_out) % 32 == 0 && p->nlon % 16 == 0) ? 1 : 0;
-        gb_fourier_stage2_oct<<<grid, QE_THREADS, O_SMEM, st>>>(d_ab, p->ab_rows, p->d_trig_o_t, p->kpad_o, grp, d_out, M,
-                                                                 p->nlon, p->no, n_mtiles, n_ntiles, wide);
-        GB_LAUNCH_CHECK();
-        return GB_OK;
-    }
-    const int n_mtiles = (int)((M + Q_TM - 1) / Q_TM);
-    const int n_ntiles = p->n_qtiles;
-    const long long n_tiles = (long long)n_mtiles * n_ntiles;
-    if (n_tiles == 0) return GB_OK;
-    const int grid = (int)((n_tiles < p->sm_count) ? n_tiles : p->sm_count);
-    QGroups grp;
-    for (int g = 0; g < 5; ++g) grp.off[g] = p->grp_off[g];
-    GB_CUDA(cudaFuncSetAttribute(gb_fourier_stage2_sym<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-    const int wide = (reinterpret_cast<uintptr_t>(d_out) % 32 == 0 && p->nlon % 8 == 0) ? 1 : 0;
-    gb_fourier_stage2_sym<true><<<grid, QE_THREADS, Q_SMEM, st>>>(d_ab, p->ab_rows, p->d_trig_q_t, p->kpad_s, grp, d_out, M,
-                                                                 p->nlon, p->nq, n_mtiles, n_ntiles, wide);
-    GB_LAUNCH_CHECK();
-    return GB_OK;
-}
-
 extern "C" int gb_synthesis(gb_plan* plan, const double* d_anm, int n_epochs, double* d_out, void* stream) {
     GB_REQUIRE(plan != nullptr, "gb_synthesis: plan is NULL");
     GB_REQUIRE(n_epochs >= 0, "gb_synthesis: n_epochs=%d is negative", n_epochs);
     if (n_epochs == 0) return GB_OK;
     GB_REQUIRE(d_anm && d_out, "gb_synthesis: NULL device pointer");
+    GB_REQUIRE(reinterpret_cast<uintptr_t>(d_out) % 16 == 0, "gb_synthesis: d_out is not 16-byte aligned");
     GB_CUDA(cudaSetDevice(plan->device));
     int rc = gb_plan_ensure_workspace(plan, n_epochs);
     if (rc) return rc;
@@ -1714,6 +1681,7 @@ extern "C" int gb_synthesis_weighted(gb_plan* plan, const double* d_anm, const d
     GB_REQUIRE(n_epochs >= 0, "gb_synthesis_weighted: n_epochs=%d is negative", n_epochs);
     if (n_epochs == 0) return GB_OK;
     GB_REQUIRE(d_anm && d_out && d_wn, "gb_synthesis_weighted: NULL device pointer");
+    GB_REQUIRE(reinterpret_cast<uintptr_t>(d_out) % 16 == 0, "gb_synthesis_weighted: d_out is not 16-byte aligned");
     GB_CUDA(cudaSetDevice(plan->device));
     int rc = gb_plan_ensure_workspace(plan, n_epochs);
     if (rc) return rc;
@@ -1728,6 +1696,7 @@ extern "C" int gb_synthesis_orderwise_filtered(gb_plan* plan, const double* d_bl
                plan->nmax);
     if (n_epochs == 0) return GB_OK;
     GB_REQUIRE(d_anm && d_out && d_blocks && block_offsets, "gb_synthesis_orderwise_filtered: NULL pointer");
+    GB_REQUIRE(reinterpret_cast<uintptr_t>(d_out) % 16 == 0, "gb_synthesis_orderwise_filtered: d_out is not 16-byte aligned");
     GB_CUDA(cudaSetDevice(plan->device));
     int rc = gb_plan_ensure_workspace(plan, n_epochs);
     if (rc) return rc;

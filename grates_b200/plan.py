@@ -31,6 +31,11 @@ def _stream_handle(device):
     return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def _env_flag(name):
+    """A switch of the CUDA library, read the way it reads it (gb_env_flag): set, non-empty, not starting with '0'."""
+    return os.environ.get(name, "")[:1] not in ("", "0")
+
+
 def _check_out(out, shape, device, name="out"):
     """A caller-supplied result buffer goes to the kernels as a raw pointer: it must be exactly what they write."""
     if not isinstance(out, torch.Tensor):
@@ -138,23 +143,18 @@ class SHPlan:
     @property
     def symmetric(self):
         """True if synthesis uses the four-fold longitude symmetry (see gb_plan_is_symmetric)."""
-        import os
-        forced_off = os.environ.get("GB_NO_SYMMETRY", "") not in ("", "0")
-        return bool(self._lib.gb_plan_is_symmetric(self._handle)) and not forced_off
+        return bool(self._lib.gb_plan_is_symmetric(self._handle)) and not _env_flag("GB_NO_SYMMETRY")
 
     @property
     def octant(self):
         """True if synthesis uses the eight-fold longitude symmetry (gb_plan_is_symmetric returns 2)."""
-        import os
-        forced_off = any(os.environ.get(v, "") not in ("", "0") for v in ("GB_NO_SYMMETRY", "GB_S2_QUADRANT"))
-        return self._lib.gb_plan_is_symmetric(self._handle) == 2 and not forced_off
+        return (self._lib.gb_plan_is_symmetric(self._handle) == 2 and not _env_flag("GB_NO_SYMMETRY")
+                and not _env_flag("GB_S2_QUADRANT"))
 
     @property
     def folded(self):
         """True if the Legendre stage uses the equatorial symmetry of the parallels (see gb_plan_is_folded)."""
-        import os
-        forced_off = os.environ.get("GB_NO_FOLD", "") not in ("", "0")
-        return bool(self._lib.gb_plan_is_folded(self._handle)) and not forced_off
+        return bool(self._lib.gb_plan_is_folded(self._handle)) and not _env_flag("GB_NO_FOLD")
 
     def _check_anm(self, anm):
         if anm.dim() != 3 or anm.shape[1] != self.L or anm.shape[2] != self.L:
@@ -168,7 +168,8 @@ class SHPlan:
         degree_weights: optional [L] weights w_n of an isotropic filter (Gaussian, Butterworth),
         multiplied into the coefficients while they are packed (gb_synthesis_weighted).
         orderwise_filter: an OrderWiseFilter applied to the batch first (gb_synthesis_orderwise_filtered: its result goes
-        straight into the layout the Legendre stage reads; bit-identical to filter_batch followed by synthesis)."""
+        straight into the layout the Legendre stage reads; bit-identical to filter_batch followed by synthesis).
+        out: 16-byte aligned (as every torch allocation is): the kernels store pairs of doubles."""
         self._check_anm(anm)
         anm = anm.contiguous()
         E = anm.shape[0]
@@ -176,6 +177,8 @@ class SHPlan:
             out = torch.empty((E, self.nlat, self.nlon), dtype=torch.float64, device=anm.device)
         else:
             _check_out(out, (E, self.nlat, self.nlon), self.device)
+            if out.data_ptr() % 16:
+                raise ValueError("out must be 16-byte aligned: the kernels store pairs of doubles")
         if orderwise_filter is not None:
             if degree_weights is not None:
                 raise ValueError("pass either degree_weights or orderwise_filter")
@@ -250,7 +253,7 @@ class SHPlan:
             raise ValueError("analysis up to degree {0} needs more than {1} meridians (got {2})"
                              .format(self.max_degree, 2 * self.max_degree, self.nlon))
         w_lat, u_lon = separable_weights(areas)
-        if os.environ.get("GB_ANALYSIS_HOST_OPERATORS", "0") not in ("", "0"):
+        if _env_flag("GB_ANALYSIS_HOST_OPERATORS"):
             # cross-check: the per-order solves with numpy on the host (0.5-0.8 s at degree 180)
             lon_ops, lat_ops, offsets = analysis_operators(self, int(min_degree), w_lat, u_lon)
             with self._lock:

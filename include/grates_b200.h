@@ -100,8 +100,8 @@ int gb_plan_info(const gb_plan* plan, int* nmax, int* nlat, int* nlon, int* devi
  * Returns 2 if in addition the first-quadrant meridians mirror about pi/4 (meridian count divisible by 16, e.g. the
  * 0.5 and 0.25 degree GeographicGrid): gb_synthesis then evaluates the first OCTANT only -- the orders 0, 2 (mod 4) change
  * the sign of their cosine / sine rows under mu -> pi/2 - mu, the odd orders swap them -- for three quarters of the
- * four-fold kernel's multiply-adds.  Both gates are measured on the plan's own tables.  GB_NO_OCTANT=1 at plan creation
- * or GB_S2_QUADRANT=1 at call time keep the four-fold kernel.
+ * four-fold kernel's multiply-adds.  Both gates are measured on the plan's own tables.  GB_S2_QUADRANT=1 at call time
+ * keeps the four-fold kernel.
  */
 int gb_plan_is_symmetric(const gb_plan* plan);
 
@@ -122,6 +122,7 @@ int gb_plan_is_folded(const gb_plan* plan);
  * Replaces the body of PotentialCoefficients.to_grid, gravityfield.py:358-368, for a batch:
  *   out[e][i][j] = sum_n kn[i][n] sum_m P_nm(theta_i) (C_nm^e cos m lon_j + S_nm^e sin m lon_j)
  *   d_anm [n_epochs][L][L] packed, d_out [n_epochs][nlat][nlon].
+ * d_out must be 16-byte aligned (the kernels store pairs of doubles); GB_ERR_ARGUMENT otherwise, before any launch.
  */
 int gb_synthesis(gb_plan* plan, const double* d_anm, int n_epochs, double* d_out, void* stream);
 
@@ -211,6 +212,7 @@ int gb_covariance_propagation_filtered(gb_plan* plan, const double* d_sigma, int
  *   gb_synthesis_weighted   gb_synthesis of the scaled coefficients without materialising them: the
  *                           weights are multiplied in while the coefficients are packed order-wise
  *   d_wn [nmax+1] device array (the reference leaves degrees 0, 1 unscaled for the Gaussian: w = 1)
+ *   d_out of gb_synthesis_weighted: 16-byte aligned, as for gb_synthesis
  */
 int gb_scale_by_degree(const double* d_anm_in, const double* d_wn, int n_epochs, int nmax,
                        double* d_anm_out, int device, void* stream);
@@ -221,7 +223,7 @@ int gb_synthesis_weighted(gb_plan* plan, const double* d_anm, const double* d_wn
  * Order-wise block filter (gb_orderwise_filter) followed by gb_synthesis of the filtered batch, without materialising
  * it: the filter writes its result in the layout the Legendre stage of the synthesis reads.  Replaces
  * OrderWiseFilter.filter (filter.py:180-189) + PotentialCoefficients.to_grid (gravityfield.py:331-368) per epoch;
- * bit-identical to the two calls in sequence.  nf >= the plan's nmax.
+ * bit-identical to the two calls in sequence.  nf >= the plan's nmax.  d_out: 16-byte aligned, as for gb_synthesis.
  */
 int gb_synthesis_orderwise_filtered(gb_plan* plan, const double* d_blocks, const int64_t* block_offsets, int nf,
                                     const double* d_anm, int n_epochs, double* d_out, void* stream);

@@ -134,9 +134,12 @@ def test_synthesis_symmetric_vs_general_path(gb, orc, monkeypatch, nmax, dlon, E
     if nmax >= 1:
         anm[:, 1, 0], anm[:, 1, 1], anm[:, 0, 1] = 2e-6, -3e-6, 4e-6
     sym = gb.to_grid_batch(anm, grid, "ewh")
-    monkeypatch.setenv("GB_S2_NARROW_STORES", "1")       # 16-byte store path (output rows not 32-byte aligned)
-    np.testing.assert_array_equal(gb.to_grid_batch(anm, grid, "ewh"), sym)
-    monkeypatch.delenv("GB_S2_NARROW_STORES")
+    # 16-byte store path: an output 16- but not 32-byte aligned (two doubles past the start of its allocation)
+    plan, x = gb.get_plan(grid, nmax, "ewh"), torch.as_tensor(anm).cuda()
+    aligned = plan.synthesis(x)
+    narrow = torch.empty(aligned.numel() + 2, dtype=torch.float64, device="cuda")[2:].view(aligned.shape)
+    assert narrow.data_ptr() % 32 == 16
+    assert plan.synthesis(x, out=narrow) is narrow and torch.equal(narrow, aligned)
     monkeypatch.setenv("GB_NO_SYMMETRY", "1")
     gen = gb.to_grid_batch(anm, grid, "ewh")
     monkeypatch.delenv("GB_NO_SYMMETRY")
@@ -1007,8 +1010,8 @@ def test_api_errors(gb):
 
 
 def test_out_buffers_are_checked(gb):
-    """A caller-supplied result buffer reaches the kernels as a raw pointer: wrong device, dtype, shape or strides
-    must raise before anything is launched."""
+    """A caller-supplied result buffer reaches the kernels as a raw pointer: wrong device, dtype, shape, strides or an
+    address that is not 16-byte aligned must raise before anything is launched."""
     grid = gb.GeographicGrid(30.0, 30.0)
     plan = gb.get_plan(grid, 3, "ewh")
     x = torch.zeros((2, 4, 4), dtype=torch.float64, device="cuda")
@@ -1017,9 +1020,15 @@ def test_out_buffers_are_checked(gb):
     for bad in (torch.empty((2, 6, 12), dtype=torch.float64),                      # host tensor
                 torch.empty((2, 6, 12), dtype=torch.float32, device="cuda"),
                 torch.empty((2, 6, 13), dtype=torch.float64, device="cuda"),
-                torch.empty((2, 12, 6), dtype=torch.float64, device="cuda").transpose(1, 2)):
+                torch.empty((2, 12, 6), dtype=torch.float64, device="cuda").transpose(1, 2),
+                torch.empty(2 * 6 * 12 + 1, dtype=torch.float64, device="cuda")[1:].view(2, 6, 12)):   # 8-byte aligned
         with pytest.raises(ValueError):
             plan.synthesis(x, out=bad)
+    # the library itself refuses the misaligned buffer too
+    import ctypes
+    odd = torch.empty(2 * 6 * 12 + 1, dtype=torch.float64, device="cuda")[1:]
+    rc = gb._lib.load().gb_synthesis(plan._handle, ctypes.c_void_p(x.data_ptr()), 2, ctypes.c_void_p(odd.data_ptr()), None)
+    assert rc == gb._lib.GB_ERR_ARGUMENT
     plan.set_analysis(0, grid.area.reshape(plan.nlat, plan.nlon))
     with pytest.raises(ValueError):
         plan.analysis(good, out=torch.empty((2, 4, 5), dtype=torch.float64, device="cuda"))

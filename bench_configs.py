@@ -300,7 +300,7 @@ def config4(pk, ctx=None, with_cpu=True, extras=True):
         res["direct_point_kernel"] = {"points": sl.point_count, "ms": ms_direct, "flops": direct_flops,
                                       "frac_fp64_peak": direct_flops / ms_direct / 1e9 / pk,
                                       "ms_upper_triangle_of_symmetric_sigma": ms_direct_sym,
-                                      "note": "gb_points_quadform: blocked diag(F Sigma F') on DMMA, no grid structure assumed"}
+                                      "note": "gbgemm::kernel<PointQuadForm>: blocked diag(F Sigma F') on DMMA, no grid structure assumed"}
     return res
 
 

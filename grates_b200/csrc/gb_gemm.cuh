@@ -1,5 +1,6 @@
-// Persistent FP64 tensor-core GEMM building block (sm_100a), shared by synthesis stage 2 (direct
-// path) and the analysis longitude stage.
+// Persistent FP64 tensor-core GEMM building block (sm_100a).  Users: synthesis stage 2 (direct path), both analysis
+// stages (longitude and latitude), the dense filter, the covariance longitude form of grids without four-fold symmetric
+// meridians, and at arbitrary points the synthesis, the adjoint and the covariance diag(F Sigma F').
 //
 //   C[row, col] = sum_k A[k, row] * B[k, col]
 //
@@ -51,11 +52,8 @@ struct Shape {
     int b_rows;             // k rows per B tile
     int klen;               // contraction length (multiple of 4), k = 0..klen-1 of B, a_koff.. of A
     int n_mtiles, n_ntiles;
-    const int* nt_koff = nullptr;   // optional per-column-tile A k offset and contraction length
-    const int* nt_klen = nullptr;   // (overrides a_koff_mul / klen; used by the covariance quadratic form)
-    const int* mt_first_nt = nullptr;   // optional: row tile mt only computes column tiles nt >= mt_first_nt[mt]
     int mt_kstart_mod = 0, mt_kstart_mul = 0;   // optional: row tile mt starts its contraction at k = (mt % mod) * mul
-                                        // (operand rows below are known zeros: upper-triangular A blocks)
+                                        // (operand rows below are known zeros: triangular A blocks)
     const int* mt_bgroup = nullptr;     // optional: row tile mt multiplies B tile mt_bgroup[mt] * n_ntiles + nt
                                         // (block-diagonal batches: the analysis latitude stage, one group per order)
 };
@@ -94,12 +92,10 @@ __global__ void __launch_bounds__(THREADS, 1) kernel(Shape sh, Epilogue epi) {
         if (lane == 0) {
             for (; mt < sh.n_mtiles; mt += step_m, nt += step_n) {
                 if (nt >= sh.n_ntiles) { nt -= sh.n_ntiles; ++mt; if (mt >= sh.n_mtiles) break; }
-                if (sh.mt_first_nt && nt < sh.mt_first_nt[mt]) continue;
-                const int a_koff = sh.nt_koff ? sh.nt_koff[nt] : (nt / sh.tiles_per_group) * sh.a_koff_mul;
-                const int klen = sh.nt_klen ? sh.nt_klen[nt] : sh.klen;
+                const int a_koff = (nt / sh.tiles_per_group) * sh.a_koff_mul;
                 const int kstart = sh.mt_kstart_mod ? (mt % sh.mt_kstart_mod) * sh.mt_kstart_mul : 0;
-                for (int k0 = kstart; k0 < klen; k0 += KC) {
-                    const int kc = min(KC, klen - k0);
+                for (int k0 = kstart; k0 < sh.klen; k0 += KC) {
+                    const int kc = min(KC, sh.klen - k0);
                     gb::mbar_wait(&empty[stage], phase ^ 1u);
                     double* sA = s_tiles + (size_t)stage * STAGE_DOUBLES;
                     double* sB = sA + KC * LDA;
@@ -120,13 +116,11 @@ __global__ void __launch_bounds__(THREADS, 1) kernel(Shape sh, Epilogue epi) {
         const int q = lane & 3;
         for (; mt < sh.n_mtiles; mt += step_m, nt += step_n) {
             if (nt >= sh.n_ntiles) { nt -= sh.n_ntiles; ++mt; if (mt >= sh.n_mtiles) break; }
-            if (sh.mt_first_nt && nt < sh.mt_first_nt[mt]) continue;
             double acc[4][NI][2];
 #pragma unroll
             for (int mi = 0; mi < 4; ++mi)
 #pragma unroll
                 for (int ni = 0; ni < NI; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
-            const int klen = sh.nt_klen ? sh.nt_klen[nt] : sh.klen;
             const long long row_base = (long long)mt * TM + wm * 32 + g;
             const int col_base = nt * TN + wn * (8 * NI) + 2 * q;
             auto pre = [&] {
@@ -134,8 +128,8 @@ __global__ void __launch_bounds__(THREADS, 1) kernel(Shape sh, Epilogue epi) {
                 else return 0;
             }();
             const int kstart = sh.mt_kstart_mod ? (mt % sh.mt_kstart_mod) * sh.mt_kstart_mul : 0;
-            for (int k0 = kstart; k0 < klen; k0 += KC) {
-                const int kc = min(KC, klen - k0);
+            for (int k0 = kstart; k0 < sh.klen; k0 += KC) {
+                const int kc = min(KC, sh.klen - k0);
                 gb::mbar_wait(&full[stage], phase);
                 const double* sA = s_tiles + (size_t)stage * STAGE_DOUBLES + wm * 32 + g;
                 const double* sB = s_tiles + (size_t)stage * STAGE_DOUBLES + KC * LDA + wn * (8 * NI) + g;

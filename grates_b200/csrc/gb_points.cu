@@ -7,9 +7,9 @@
 //   gb_points_covariance   replaces IrregularGrid.covariance_propagation (reference grid.py:1096-1120):
 //                          var[p] = sum_ab F[p,a] Sigma[a,b] F[p,b] -- the direct, blocked
 //                          diag(F Sigma F') of the north star: F tiles generated on the fly
-//                          (gb_points_design), T = F Sigma on the FP64 tensor cores with Sigma rows
-//                          staged by the TMA unit (cp.async.bulk + mbarrier pipeline), and the
-//                          row-wise product with F folded into the epilogue with warp shuffles.
+//                          (gb_points_design), (F Sigma)' = Sigma' F' on the shared FP64 tensor-core
+//                          GEMM (gb_gemm.cuh) with Sigma as the A operand and F' as the B operand, and
+//                          the product with F folded into the epilogue with warp shuffles.
 //                          2 P K^2 flops, nothing assumed about the point geometry.
 #include <vector>
 #include <cmath>
@@ -87,25 +87,27 @@ gb_points_synthesis_kernel(const double* __restrict__ anm, double* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
-// design matrix F^T in the tiled layout [point tile][a][GB_LDA], a = degree-wise index - nmin^2
+// design matrix F^T as GEMM tiles [point tile of tn][a][ld], a = degree-wise index - nmin^2: the A operand
+// (tn = GB_TM, ld = GB_LDA) of the point synthesis, the B operand (GB_S2_TN, GB_S2_LDB) of the point covariance
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128)
 gb_points_design(double* __restrict__ FT, const double* __restrict__ ct, const double* __restrict__ kn,
                  const double* __restrict__ pmm, const double* __restrict__ cml, const double* __restrict__ sml,
                  const double* __restrict__ ra, const double* __restrict__ rb, const double* __restrict__ rc, int L,
-                 int nmin, int npts, int rows, int p0) {
+                 int nmin, int npts, int rows, int p0, int tn, int ld) {
     const int p = p0 + blockIdx.x * blockDim.x + threadIdx.x;      // tiles are numbered from point p0
     const int m = blockIdx.y;
     if (p >= npts) return;
     const double* kn_p = kn + (size_t)p * L;
     const double cm = cml[(size_t)p * L + m], sm = sml[(size_t)p * L + m];
     const int off = nmin * nmin;
+    double* col = FT + (size_t)((p - p0) / tn) * rows * ld + (p - p0) % tn;
     legendre_column(m, L, ct[p], pmm[(size_t)p * L + m], ra, rb, rc, [&](int n, double pn) {
         if (n < nmin) return;
         const double pk = __dmul_rn(pn, kn_p[n]);
         const int a = n * n + (m == 0 ? 0 : 2 * m - 1) - off;
-        FT[gb_ab_offset(p - p0, a, rows)] = __dmul_rn(pk, cm);
-        if (m > 0) FT[gb_ab_offset(p - p0, a + 1, rows)] = __dmul_rn(pk, sm);
+        col[(size_t)a * ld] = __dmul_rn(pk, cm);
+        if (m > 0) col[(size_t)(a + 1) * ld] = __dmul_rn(pk, sm);
     });
 }
 
@@ -175,121 +177,6 @@ gb_points_value_tiles(const double* __restrict__ values, double* __restrict__ Bt
     Bt[((size_t)(e / tn) * rows + pp) * ldb + e % tn] = values[(size_t)e * npts + p0 + pp];
 }
 
-// ---------------------------------------------------------------------------------------------
-// blocked diag(F Sigma F'): tile = 128 points x 120 columns b; K loop over a in chunks of 28
-// ---------------------------------------------------------------------------------------------
-constexpr int C_WM = 4, C_WN = 3, C_TM = 128, C_TN = 120, C_KC = 28, C_STAGES = 3;
-constexpr int C_LDA = GB_LDA, C_LDB = C_TN + 4;
-constexpr int C_CONSUMER_WARPS = C_WM * C_WN;
-constexpr int C_THREADS = 32 * (C_CONSUMER_WARPS + 1);
-constexpr int C_STAGE_DOUBLES = C_KC * (C_LDA + C_LDB);
-constexpr size_t C_SMEM = (size_t)C_STAGES * C_STAGE_DOUBLES * sizeof(double) + 2 * C_STAGES * sizeof(uint64_t);
-
-__global__ void __launch_bounds__(C_THREADS, 1)
-gb_points_quadform(const double* __restrict__ FT, int rows, const double* __restrict__ sig, long long lds, int Kp,
-                   long long Kc, double* __restrict__ var, int npts, int n_mtiles, int n_ntiles, int upper) {
-    extern __shared__ __align__(128) unsigned char s_raw[];
-    double* s_tiles = reinterpret_cast<double*>(s_raw);
-    uint64_t* full = reinterpret_cast<uint64_t*>(s_raw + (size_t)C_STAGES * C_STAGE_DOUBLES * sizeof(double));
-    uint64_t* empty = full + C_STAGES;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < C_STAGES; ++s) {
-            gb::mbar_init(&full[s], 1);
-            gb::mbar_init(&empty[s], C_CONSUMER_WARPS);
-        }
-        gb::fence_mbar_init();
-    }
-    __syncthreads();
-    const long long n_tiles = (long long)n_mtiles * n_ntiles;
-    int stage = 0;
-    uint32_t phase = 0;
-    if (warp == C_CONSUMER_WARPS) {
-        // producer: one bulk copy for the F^T chunk, one per covariance row
-        for (long long t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-            // upper-triangular operand: the work of a tile grows with its column tile, so the heaviest column tiles
-            // go first (and the CTAs of one wave share the same covariance columns in L2)
-            const long long mt = upper ? t % n_mtiles : t / n_ntiles;
-            const int n0 = (int)(upper ? n_ntiles - 1 - t / n_mtiles : t % n_ntiles) * C_TN;
-            long long w = Kc - n0;
-            if (w > C_TN) w = C_TN;
-            const int width = (int)((w + 1) & ~1LL);     // even number of doubles (16-byte granules)
-            // upper-triangular operand (symmetric Sigma, off-diagonal entries doubled): rows a beyond the tile's last
-            // column are zero
-            const int kend = upper ? min(Kp, (n0 + C_TN + 3) & ~3) : Kp;
-            for (int k0 = 0; k0 < kend; k0 += C_KC) {
-                const int kc = min(C_KC, kend - k0);
-                gb::mbar_wait(&empty[stage], phase ^ 1u);
-                double* sA = s_tiles + (size_t)stage * C_STAGE_DOUBLES;
-                double* sB = sA + C_KC * C_LDA;
-                if (lane == 0) {
-                    const uint32_t bytes_a = (uint32_t)(kc * C_LDA * sizeof(double));
-                    gb::mbar_arrive_expect_tx(&full[stage], bytes_a + (uint32_t)(kc * width * sizeof(double)));
-                    gb::bulk_g2s(sA, FT + ((size_t)mt * rows + k0) * C_LDA, bytes_a, &full[stage]);
-                }
-                __syncwarp();
-                if (lane < kc)
-                    gb::bulk_g2s(sB + lane * C_LDB, sig + (size_t)(k0 + lane) * lds + n0,
-                                 (uint32_t)(width * sizeof(double)), &full[stage]);
-                if (++stage == C_STAGES) { stage = 0; phase ^= 1u; }
-            }
-        }
-    } else {
-        const int wm = warp / C_WN, wn = warp % C_WN;
-        const int g = lane >> 2, q = lane & 3;
-        for (long long t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-            const long long mt = upper ? t % n_mtiles : t / n_ntiles;
-            const int n0 = (int)(upper ? n_ntiles - 1 - t / n_mtiles : t % n_ntiles) * C_TN;
-            double acc[4][5][2];
-#pragma unroll
-            for (int mi = 0; mi < 4; ++mi)
-#pragma unroll
-                for (int ni = 0; ni < 5; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
-            const int kend = upper ? min(Kp, (n0 + C_TN + 3) & ~3) : Kp;
-            for (int k0 = 0; k0 < kend; k0 += C_KC) {
-                const int kc = min(C_KC, kend - k0);
-                gb::mbar_wait(&full[stage], phase);
-                const double* sA = s_tiles + (size_t)stage * C_STAGE_DOUBLES + wm * 32 + g;
-                const double* sB = s_tiles + (size_t)stage * C_STAGE_DOUBLES + C_KC * C_LDA + wn * 40 + g;
-#pragma unroll
-                for (int kk = 0; kk < C_KC; kk += 4) {
-                    if (kk >= kc) break;
-                    double a[4], b[5];
-#pragma unroll
-                    for (int mi = 0; mi < 4; ++mi) a[mi] = sA[(kk + q) * C_LDA + mi * 8];
-#pragma unroll
-                    for (int ni = 0; ni < 5; ++ni) b[ni] = sB[(kk + q) * C_LDB + ni * 8];
-#pragma unroll
-                    for (int mi = 0; mi < 4; ++mi)
-#pragma unroll
-                        for (int ni = 0; ni < 5; ++ni) gb::dmma_884(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
-                }
-                __syncwarp();
-                if (lane == 0) gb::mbar_arrive(&empty[stage]);
-                if (++stage == C_STAGES) { stage = 0; phase ^= 1u; }
-            }
-            // epilogue: var[p] += sum_b T[p,b] F[p,b] over this tile's columns
-            const double* ft = FT + (size_t)mt * rows * C_LDA;
-#pragma unroll
-            for (int mi = 0; mi < 4; ++mi) {
-                const int r = wm * 32 + mi * 8 + g;
-                double part = 0.0;
-#pragma unroll
-                for (int ni = 0; ni < 5; ++ni) {
-                    const long long b = (long long)n0 + wn * 40 + ni * 8 + 2 * q;
-                    if (b < Kc) part = fma(acc[mi][ni][0], ft[(size_t)b * C_LDA + r], part);
-                    if (b + 1 < Kc) part = fma(acc[mi][ni][1], ft[(size_t)(b + 1) * C_LDA + r], part);
-                }
-                part += __shfl_xor_sync(0xffffffffu, part, 1);
-                part += __shfl_xor_sync(0xffffffffu, part, 2);
-                const long long p = mt * C_TM + r;
-                // one writer per (point, column tile, warp column): gb_points_finish adds the slots in order
-                if (q == 0 && p < npts) var[(size_t)p * (n_ntiles * C_WN) + (n0 / C_TN) * C_WN + wn] = part;
-            }
-        }
-    }
-}
-
 // out[p] = (sqrt of) the sum of the point's partial sums, in slot order: bit-identical from run to run
 __global__ void gb_points_finish(const double* __restrict__ part, double* __restrict__ out, int nslots, int n, int take_sqrt) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -324,14 +211,6 @@ extern "C" int gb_points_create(gb_points** out, int nmax, int npts, const doubl
     if (prop.major < 10)
         return gb_set_error(GB_ERR_UNSUPPORTED, "gb_points_create: device %d is sm_%d%d; built for sm_100a", device,
                             prop.major, prop.minor);
-    {   // keep stream-ordered workspace allocations in the pool between calls (default threshold 0
-        // returns them to the driver at every synchronisation: milliseconds per GB on the next call)
-        cudaMemPool_t pool;
-        if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
-            unsigned long long keep = ~0ULL;
-            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
-        }
-    }
     gb_points* p = new gb_points();
     p->device = device;
     p->nmax = nmax;
@@ -377,6 +256,51 @@ struct PointStore {
     }
 };
 
+// epilogue of the point covariance: the GEMM rows are the columns b of Sigma, its columns the points of a block, so that
+// C[b][p] = (F Sigma)[p][b].  part[p][slot] = sum_b C[b][p] F[p][b] over the warp's 32 rows b, with F[p][b] read back from
+// the design tiles (the B operand); slot = (row tile, warp row), one writer per slot.  gb_points_finish adds the slots in
+// order.
+struct PointQuadForm {
+    static constexpr bool whole_tile = true;
+    const double* ft;    // design tiles [point tile][rows][GB_S2_LDB]
+    double* part;        // [count][nslots]
+    long long K;         // coefficients (rows b >= K are padding)
+    int rows, count, nslots;
+    __device__ __forceinline__ const double* prepare(long long, int nt, int col_base) const {
+        return ft + (size_t)nt * rows * GB_S2_LDB + (col_base - nt * GB_S2_TN);
+    }
+    __device__ __forceinline__ void tile(const double* f, long long row_base, int col_base, double (&acc)[4][5][2]) const {
+        // the thread's four rows first, then over g; the sums go to acc[0] (a second set of 10 sums spills at 128 registers)
+#pragma unroll
+        for (int mi = 0; mi < 4; ++mi) {
+            const long long b = row_base + mi * 8;
+#pragma unroll
+            for (int ni = 0; ni < 5; ++ni) {
+                const double2 fb = b < K ? __ldg(reinterpret_cast<const double2*>(f + (size_t)b * GB_S2_LDB + ni * 8))
+                                         : make_double2(0.0, 0.0);
+                acc[0][ni][0] = mi ? fma(acc[mi][ni][0], fb.x, acc[0][ni][0]) : acc[0][ni][0] * fb.x;
+                acc[0][ni][1] = mi ? fma(acc[mi][ni][1], fb.y, acc[0][ni][1]) : acc[0][ni][1] * fb.y;
+            }
+        }
+#pragma unroll
+        for (int ni = 0; ni < 5; ++ni)
+#pragma unroll
+            for (int r = 0; r < 2; ++r)
+#pragma unroll
+                for (int o = 4; o < 32; o <<= 1) acc[0][ni][r] += __shfl_xor_sync(0xffffffffu, acc[0][ni][r], o);
+        if ((threadIdx.x & 31) < 4) {      // g = 0
+            const int slot = (int)(row_base >> 5);
+#pragma unroll
+            for (int ni = 0; ni < 5; ++ni)
+#pragma unroll
+                for (int r = 0; r < 2; ++r) {
+                    const int pp = col_base + ni * 8 + r;
+                    if (pp < count) part[(size_t)pp * nslots + slot] = acc[0][ni][r];
+                }
+        }
+    }
+};
+
 // Epoch batches at arbitrary points as a GEMM: the design tiles F^T of a block of points are generated once (on-the-fly
 // recursion, gb_points_design) and multiplied with ALL epochs on the DMMA GEMM, instead of re-running the recursion for
 // every eight epochs.  2 P K E flops; the design matrix only ever exists for one block of points.
@@ -405,7 +329,7 @@ static int points_synthesis_gemm(gb_points* p, const double* d_anm, int E, doubl
         GB_CUDA(cudaMemsetAsync(d_ft, 0, (size_t)nt * Kp * GB_LDA * sizeof(double), st));   // padding rows / points
         dim3 grid((count + 127) / 128, L);
         gb_points_design<<<grid, 128, 0, st>>>(d_ft, p->d_ct, p->d_kn, p->d_pmm, p->d_cml, p->d_sml, p->d_ra, p->d_rb,
-                                              p->d_rc, L, 0, p0 + count, Kp, p0);
+                                              p->d_rc, L, 0, p0 + count, Kp, p0, GB_TM, GB_LDA);
         GB_LAUNCH_CHECK();
         gbgemm::Shape sh;
         sh.A_t = d_ft;
@@ -524,22 +448,26 @@ extern "C" int gb_points_synthesis_matrix(gb_points* p, int nmin, double* d_out,
     return GB_OK;
 }
 
-// Sigma re-pitched to an even leading dimension; for a symmetric Sigma only its upper triangle is kept, the
-// off-diagonal entries doubled:  x' S x = sum_a S_aa x_a^2 + 2 sum_{a<b} S_ab x_a x_b
-__global__ void __launch_bounds__(256)
-gb_points_sigma_operand(const double* __restrict__ sigma, double* __restrict__ sig, long long Kc, long long lds, int upper) {
-    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long a = blockIdx.y;
-    if (b >= Kc) return;
-    double v = sigma[(size_t)a * Kc + b];
-    if (upper) v = (a < b) ? v + v : (a == b ? v : 0.0);
-    sig[(size_t)a * lds + b] = v;
+// Sigma as the GEMM A operand, tiles [b tile][a][GB_LDA] with A[k = a][row = b] = Sigma[a][b] (a row tile holds runs of 128
+// consecutive entries of the rows of Sigma), zero beyond K' in a and b.  For a symmetric Sigma only its lower triangle is
+// kept, the off-diagonal entries doubled:  x' S x = sum_b S_bb x_b^2 + 2 sum_{a>b} S_ab x_a x_b, so that row tile j only
+// needs k = a >= 128 j.
+__global__ void __launch_bounds__(GB_TM)
+gb_points_sigma_tiles(const double* __restrict__ sigma, double* __restrict__ St, long long Kc, int Kp, int lower) {
+    const long long a = blockIdx.x;
+    const long long b = (long long)blockIdx.y * GB_TM + threadIdx.x;
+    double v = 0.0;
+    if (a < Kc && b < Kc) {
+        v = sigma[(size_t)a * Kc + b];
+        if (lower) v = (a > b) ? v + v : (a == b ? v : 0.0);
+    }
+    St[gb_ab_offset(b, (int)a, Kp)] = v;
 }
 
 extern "C" int gb_points_covariance(gb_points* p, const double* d_sigma, int nmin, double* d_out, int flags,
                                     void* stream) {
     const int take_sqrt = flags & GB_COV_SQRT;
-    const int upper = (flags & GB_COV_SYMMETRIC) ? 1 : 0;
+    const int lower = (flags & GB_COV_SYMMETRIC) ? 1 : 0;
     GB_REQUIRE(p != nullptr, "gb_points_covariance: point set is NULL");
     GB_REQUIRE(nmin >= 0 && nmin <= p->nmax, "gb_points_covariance: min_degree=%d outside [0, %d]", nmin, p->nmax);
     GB_REQUIRE(d_sigma && d_out, "gb_points_covariance: NULL device pointer");
@@ -548,43 +476,47 @@ extern "C" int gb_points_covariance(gb_points* p, const double* d_sigma, int nmi
     const int L = p->L;
     const long long Kc = (long long)L * L - (long long)nmin * nmin;   // coefficients
     const int Kp = (int)((Kc + 3) / 4 * 4);                            // padded to whole k4 steps
-    const long long lds = (Kc + 1) / 2 * 2 + 2;                        // even leading dimension, room for the tail
-    const int n_mtiles_all = (p->npts + C_TM - 1) / C_TM;
-    const int n_ntiles = (int)((Kc + C_TN - 1) / C_TN);
-    // the design matrix only ever exists for one block of points (about four waves of GEMM tiles): 75 KB per point at
+    const int n_btiles = (int)((Kc + GB_TM - 1) / GB_TM);              // GEMM row tiles: columns b of Sigma
+    const int n_ptiles_all = (p->npts + GB_S2_TN - 1) / GB_S2_TN;       // GEMM column tiles: points
+    // the design matrix only ever exists for one block of points (several waves of GEMM tiles): 75 KB per point at
     // degree 96 would otherwise be 12 GB for a 0.5-degree Reuter grid
-    int tiles_per_block = 4 * p->sm_count / (n_ntiles > 0 ? n_ntiles : 1);
+    int tiles_per_block = 4 * p->sm_count / n_btiles;
     if (tiles_per_block < 16) tiles_per_block = 16;
-    if (tiles_per_block > n_mtiles_all) tiles_per_block = n_mtiles_all;
-    double *d_ft = nullptr, *d_sig = nullptr, *d_part = nullptr;
-    const size_t ft_elems = (size_t)tiles_per_block * Kp * C_LDA;
-    const int nslots = n_ntiles * C_WN;
+    if (tiles_per_block > n_ptiles_all) tiles_per_block = n_ptiles_all;
+    const int nslots = n_btiles * gbgemm::WM;
+    double *d_st = nullptr, *d_ft = nullptr, *d_part = nullptr;
     gb_retain_pool_memory(p->device);
     gb_scratch scratch(st);
-    GB_CUDA(scratch.alloc(&d_ft, ft_elems));
-    GB_CUDA(scratch.alloc(&d_sig, (size_t)Kp * lds));
-    GB_CUDA(scratch.alloc(&d_part, (size_t)tiles_per_block * C_TM * nslots));
-    GB_CUDA(cudaMemsetAsync(d_sig, 0, (size_t)Kp * lds * sizeof(double), st));
-    {   // covariance rows re-pitched to an even leading dimension (16-byte aligned rows for the bulk copies)
-        dim3 grid((unsigned)((Kc + 255) / 256), (unsigned)Kc);
-        gb_points_sigma_operand<<<grid, 256, 0, st>>>(d_sigma, d_sig, Kc, lds, upper);
-        GB_LAUNCH_CHECK();
+    GB_CUDA(scratch.alloc(&d_st, (size_t)n_btiles * Kp * GB_LDA));
+    GB_CUDA(scratch.alloc(&d_ft, (size_t)tiles_per_block * Kp * GB_S2_LDB));
+    GB_CUDA(scratch.alloc(&d_part, (size_t)tiles_per_block * GB_S2_TN * nslots));
+    gb_points_sigma_tiles<<<dim3((unsigned)Kp, (unsigned)n_btiles), GB_TM, 0, st>>>(d_sigma, d_st, Kc, Kp, lower);
+    GB_LAUNCH_CHECK();
+    gbgemm::Shape sh;
+    sh.A_t = d_st;
+    sh.a_rows = Kp;
+    sh.a_koff_mul = 0;
+    sh.tiles_per_group = 1;
+    sh.B_t = d_ft;
+    sh.b_rows = Kp;
+    sh.klen = Kp;
+    sh.n_mtiles = n_btiles;
+    if (lower) {                // row tile j starts its contraction at k = 128 j (the rows above are zeros)
+        sh.mt_kstart_mod = n_btiles;
+        sh.mt_kstart_mul = GB_TM;
     }
-    GB_CUDA(cudaFuncSetAttribute(gb_points_quadform, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C_SMEM));
-    for (int t0 = 0; t0 < n_mtiles_all; t0 += tiles_per_block) {
-        const int n_mtiles = (n_mtiles_all - t0 < tiles_per_block) ? (n_mtiles_all - t0) : tiles_per_block;
-        const int p0 = t0 * C_TM;
-        const int count = (p->npts - p0 < n_mtiles * C_TM) ? (p->npts - p0) : n_mtiles * C_TM;
-        GB_CUDA(cudaMemsetAsync(d_ft, 0, (size_t)n_mtiles * Kp * C_LDA * sizeof(double), st));
+    for (int t0 = 0; t0 < n_ptiles_all; t0 += tiles_per_block) {
+        const int n_ptiles = (n_ptiles_all - t0 < tiles_per_block) ? (n_ptiles_all - t0) : tiles_per_block;
+        const int p0 = t0 * GB_S2_TN;
+        const int count = (p->npts - p0 < n_ptiles * GB_S2_TN) ? (p->npts - p0) : n_ptiles * GB_S2_TN;
+        GB_CUDA(cudaMemsetAsync(d_ft, 0, (size_t)n_ptiles * Kp * GB_S2_LDB * sizeof(double), st));   // padding rows / points
         dim3 grid((count + 127) / 128, L);
         gb_points_design<<<grid, 128, 0, st>>>(d_ft, p->d_ct, p->d_kn, p->d_pmm, p->d_cml, p->d_sml, p->d_ra, p->d_rb,
-                                              p->d_rc, L, nmin, p0 + count, Kp, p0);
+                                              p->d_rc, L, nmin, p0 + count, Kp, p0, GB_S2_TN, GB_S2_LDB);
         GB_LAUNCH_CHECK();
-        const long long n_tiles = (long long)n_mtiles * n_ntiles;
-        const int gridq = (int)(n_tiles < p->sm_count ? n_tiles : p->sm_count);
-        gb_points_quadform<<<gridq, C_THREADS, C_SMEM, st>>>(d_ft, Kp, d_sig, lds, Kp, Kc, d_part, count, n_mtiles,
-                                                             n_ntiles, upper);
-        GB_LAUNCH_CHECK();
+        sh.n_ntiles = n_ptiles;
+        int rc = gbgemm::launch(sh, PointQuadForm{d_ft, d_part, Kc, Kp, count, nslots}, p->sm_count, st);
+        if (rc) return rc;
         gb_points_finish<<<(count + 255) / 256, 256, 0, st>>>(d_part, d_out + p0, nslots, count, take_sqrt ? 1 : 0);
         GB_LAUNCH_CHECK();
     }

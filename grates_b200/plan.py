@@ -605,7 +605,7 @@ class PointsPlan:
 
     def covariance_propagation(self, sigma, min_degree, take_sqrt=True, symmetric=None):
         """sigma: CUDA tensor [K', K'] in degree-wise order -> [npts] standard deviations / variances.
-        symmetric: contract only the upper triangle of sigma (half the flops); None decides on sampled entries."""
+        symmetric: contract only the lower triangle of sigma (half the flops); None decides on sampled entries."""
         kp = self.L ** 2 - min_degree ** 2
         if sigma.dim() != 2 or tuple(sigma.shape) != (kp, kp):
             raise ValueError("covariance matrix must have shape [{0}, {0}] (got {1})".format(kp, tuple(sigma.shape)))

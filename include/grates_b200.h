@@ -260,7 +260,7 @@ int gb_orderwise_filter(const double* d_blocks, const int64_t* block_offsets, in
  * gb_points_synthesis replaces gravityfield.py:376-388: d_anm [n_epochs][L][L] -> d_out [n_epochs][npts].
  * gb_points_covariance replaces grid.py:1103-1116: direct blocked diag(F Sigma F') with Sigma
  *   [K'][K'] (degree-wise order, offset nmin^2) -> d_out [npts] variances; flags as for gb_covariance_propagation
- *   (GB_COV_SQRT: std-devs; GB_COV_SYMMETRIC: only the upper triangle of Sigma is contracted, half the flops).
+ *   (GB_COV_SQRT: std-devs; GB_COV_SYMMETRIC: only the lower triangle of Sigma is contracted, half the flops).
  * gb_points_adjoint replaces the sum over nodal points of RadialBasisFunctions.to_potential_coefficients,
  *   gravityfield.py:707-724 (the transposed design matrix): d_values [n_epochs][npts] -> d_anm [n_epochs][L][L],
  *   anm[n, m] = sum_p kn[p][n] Y_nm(p) v[p]; the shape factors K[n, m] are applied by the caller.

@@ -621,7 +621,7 @@ def test_irregular_covariance_golden(gb, golden, orc):
     std = gb.IrregularGrid(lon, lat).covariance_propagation(sigma, nmin, N, "potential")
     ref = orc.covariance_propagation_points(sigma, lon, lat, nmin, N, "potential")
     assert maxnorm_err(std, ref) < TOL
-    # upper-triangle path (symmetric Sigma) and full path agree; an antisymmetric perturbation needs the full path
+    # triangle path (symmetric Sigma) and full path agree; an antisymmetric perturbation needs the full path
     pp = gb.get_points_plan(gb.IrregularGrid(lon, lat), N, "potential")
     sd = torch.as_tensor(sigma).cuda()
     half = pp.covariance_propagation(sd, nmin, symmetric=True).cpu().numpy()

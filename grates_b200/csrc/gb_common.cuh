@@ -79,9 +79,8 @@ struct gb_plan {
     double* d_rb = nullptr;     // [L][L]      recursion coefficient b_nm (utilities.py:54)
     double* d_rc = nullptr;     // [L]         sqrt(2n+1), first off-diagonal (utilities.py:46)
     double* d_trig = nullptr;   // [kpad][nlp] row 2m: cos(m lon_j), row 2m+1: sin(m lon_j)
-    double* d_zero = nullptr;   // 4 KB of zeros (source of padding rows for bulk copies)
-    // stage-1 tables, transposed and zero padded so that the Legendre warps read them coalesced and
-    // unguarded: parallels padded to GB_T1_TM, degrees of one order padded to whole GB_T1_KC chunks
+    // recursion tables of stage 1 (Source Recursion), transposed and zero padded so that the Legendre warps read them
+    // coalesced and unguarded: parallels padded to GB_T1_TM, degrees of one order padded to whole GB_T1_KC chunks
     int nlat_pad = 0, lpad = 0;
     double* d_ct_pad = nullptr; // [nlat_pad]
     double* d_kn_t = nullptr;   // [L + GB_T1_KC][nlat_pad]   kn_t[n][i]
@@ -115,7 +114,8 @@ struct gb_plan {
     // synthesis workspace, grown on demand (epochs)
     int ws_epochs = 0;
     long long ws_mpad = 0;
-    double* d_x = nullptr;      // order-wise packed coefficients, see gb_synthesis.cu
+    double* d_x = nullptr;      // packed coefficients: tiled for stage 1 (gb_launch_pack_tiled), order-wise for the FMA
+                                // cross-check (gb_launch_pack), see gb_synthesis.cu
     double* d_ab = nullptr;     // [mpad/128][ab_rows][GB_LDA] spectral intermediate (see above)
     // host-buffer pipeline
     cudaStream_t s_compute = nullptr, s_copy = nullptr;
@@ -155,9 +155,9 @@ struct gb_plan {
     double* d_ptab[3] = {nullptr, nullptr, nullptr};
     int* d_ptab_roff = nullptr;      // [L + 1] first table row of every order (orders padded to 8 rows)
     long long ptab_rtot = 0;         // rows per lat tile
-    int ptab_state[3] = {0, 0, 0};
+    int ptab_state[3] = {0, 0, 0};   // 0: not built yet, 1: built, -1: over the budget or no memory (recursion instead)
     long long x_layout_key = 0;      // (epochs, tile width) d_x was last cleared for; 0: order-wise layout / unknown
-    size_t x_elems = 0;              // doubles allocated in d_x   // 0: not built yet, 1: built, -1: over the memory budget (on-the-fly recursion instead)
+    size_t x_elems = 0;              // doubles allocated in d_x
     // stream ordering of the shared workspace (d_x, d_ab, analysis / covariance scratch, cached index tables): a call
     // on another stream than the previous call's first waits for everything that stream holds (gb_plan_acquire)
     cudaEvent_t ws_free = nullptr;

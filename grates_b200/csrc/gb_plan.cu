@@ -394,7 +394,7 @@ extern "C" int gb_plan_create(gb_plan** plan, int nmax, int nlat, int nlon, cons
         (rc_ = upload(&p->d_trig_t, trig_t)) || (p->sym && (rc_ = upload(&p->d_trig_q_t, trig_q_t))) ||
         (rc_ = upload(&p->d_ct, ct)) || (rc_ = upload(&p->d_kn, knv)) || (rc_ = upload(&p->d_pmm, pmm)) ||
         (rc_ = upload(&p->d_ra, ra)) || (rc_ = upload(&p->d_rb, rb)) || (rc_ = upload(&p->d_rc, rc)) ||
-        (rc_ = upload(&p->d_trig, trig)) || (rc_ = upload(&p->d_zero, std::vector<double>(512, 0.0))) ||
+        (rc_ = upload(&p->d_trig, trig)) ||
         (rc_ = upload(&p->d_krow_id, krow_id)) || (rc_ = upload(&p->d_krow_sym, krow_sym)) ||
         (p->oct && ((rc_ = upload(&p->d_krow_oct, krow_oct)) || (rc_ = upload(&p->d_trig_o_t, trig_o_t)))) ||
         (p->sym && (rc_ = upload(&p->d_trig_q, trig_q)))) {
@@ -422,7 +422,7 @@ extern "C" int gb_plan_destroy(gb_plan* p) {
     if (!p) return GB_OK;
     cudaSetDevice(p->device);
     cudaFree(p->d_ct); cudaFree(p->d_kn); cudaFree(p->d_pmm); cudaFree(p->d_ra); cudaFree(p->d_rb);
-    cudaFree(p->d_rc); cudaFree(p->d_trig); cudaFree(p->d_zero);
+    cudaFree(p->d_rc); cudaFree(p->d_trig);
     cudaFree(p->d_ct_pad); cudaFree(p->d_kn_t); cudaFree(p->d_pmm_t); cudaFree(p->d_rec_a); cudaFree(p->d_rec_b);
     cudaFree(p->d_krow_id); cudaFree(p->d_krow_sym); cudaFree(p->d_trig_q);
     cudaFree(p->d_krow_oct); cudaFree(p->d_trig_o_t);

@@ -7,20 +7,23 @@
 //
 // HBM layout
 //   anm   [E][L][L]          packed coefficients as the reference stores them
-//   X     order-wise packed  X_m[n-m][cs*E+e], block of order m at offset 2E*(m*L - m(m-1)/2) (gb_pack.cu)
+//   X     [order][column tile][degree row][tn+4]  X_m[n-m][cs*E+e], degree rows in the Legendre table's order
+//                            (tb_fold_row, gb_pack.cu); order-wise X_m[n-m][cs*E+e] for the FMA cross-check
 //   AB    [row tile][k][132]  spectral intermediate, tiled by 128 grid rows (e*nlat + i), see gb_common.cuh;
 //                            row order k = 2m+cs, or [CE|CO|SE|SO] groups for the symmetric stage 2
 //   trig  [col tile][k][124]  row 2m = cos(m lon_j), row 2m+1 = sin(m lon_j) (first quadrant only when symmetric)
 //   V     [E][nlat][nlon]    output
 //
 // Kernels
-//   gb_pack_kernel       transposes anm into X (gb_pack.cu; HBM-bound)
-//   gb_legendre_stage1   per (latitude tile, order m): runs the Legendre recursion on the fly
-//                        (unfused IEEE ops -> bit-identical to utilities.py:37-54), multiplies
-//                        kn[i,n] in, contracts against all epochs, writes AB
-//   gbgemm::kernel       persistent FP64 tensor-core GEMM  V = AB^T * trig  (DMMA.8x8x4, gb_gemm.cuh),
-//                        operands staged by the TMA unit (cp.async.bulk) through a 3-stage
-//                        mbarrier pipeline fed by a dedicated producer warp
+//   gb_pack_rows_kernel / gb_pack_kernel   transpose anm into X (gb_pack.cu; HBM-bound)
+//   gb_stage1            per (order pair, latitude tile, column tile): contracts kn[i,n] P_nm(theta_i) against all
+//                        epochs on the FP64 tensor cores (DMMA.8x8x4) and writes AB; the Legendre values (unfused IEEE
+//                        ops -> bit-identical to utilities.py:37-54) come from the plan's table (gb_ptab_kernel) or
+//                        from the recursion run inside the kernel
+//   gb_fourier_stage2_oct / gb_fourier_stage2_sym   stage 2 on meridians with eight- / four-fold symmetry
+//   gbgemm::kernel       stage 2 on other meridians: persistent FP64 tensor-core GEMM  V = AB^T * trig (gb_gemm.cuh)
+// All stage-1 and stage-2 kernels stage their operands with the TMA unit (cp.async.bulk) through mbarrier rings fed
+// by a producer lane.
 #include <type_traits>
 #include <vector>
 #include "gb_common.cuh"
@@ -104,331 +107,99 @@ gb_legendre_stage1_simple(const double* __restrict__ X, double* __restrict__ AB,
 
 
 // ---------------------------------------------------------------------------------------------
-// stage 1 on the FP64 tensor cores, persistent.  Work item = (order pair (p, nmax-p), 64 parallels,
-// 240 columns (e, cos|sin)); every item carries L+1 degrees, so items cost the same:
-//   D[i, col] = sum_n Pk[i, n] X_m[n, col],  Pk = kn * P_nm produced ON THE FLY:
-//   two Legendre warps (lane = parallel) advance the recursion 16 degrees at a time and write the
-//   chunk k-major into shared memory; a copy warp streams the matching rows of X_m with bulk
-//   copies; twelve consumer warps (2 x 6, 32 x 40 register tiles) issue DMMA.8x8x4.
-// One CTA per SM walks the items with a 4-stage ring that never drains: the Legendre and copy warps
-// run ahead into the next order / item while the consumers store their tile, and all tables they
-// read are global (transposed, zero padded: gb_plan::d_rec_a/b, d_kn_t, d_pmm_t, d_ct_pad), so no
-// per-item prologue exists.  The last chunk of an order is processed in whole 4-degree steps only.
+// stage 1 on the FP64 tensor cores, persistent.  Work item = (order pair (p, nmax-p), 32 or 64 parallels, TN = 8 MI NWN
+// columns (e, cos|sin)); every item carries L+1 degrees, so items cost the same:
+//   D[i, col] = sum_n Pk[i, n] X_m[n, col],  Pk[i, n] = kn[i,n] * P_nm(theta_i)
+// A ring stage holds 16 degrees of both operands: Pk [16][lda] and X_m [16][TN + 4].  A copy lane fills the X half with
+// one bulk copy from the tiled X; where the Pk half comes from is the Source:
+//   Table      the plan's Legendre table (the default).  Pk does not depend on the epoch, so the plan holds it -- written
+//              once by gb_ptab_kernel with the same bit-exact recursion -- in exactly the tile layout a stage needs, and
+//              the copy lane fetches it with one more bulk copy.  No FP64 instruction competes with the DMMA stream for
+//              the pipe (a recursion warp shares its scheduler with three DMMA-issuing warps: 300 cycles per degree,
+//              DMMA pipe 45 % active at config 2).
+//   Recursion  Legendre warps (lane = column of the tile, recursion state in registers) run the recursion on the fly and
+//              write the stage: the fallback when the table is over its memory budget or cannot be allocated.
+// Both sources lay a stage out alike: column li holds parallel s1_parallel(li), degree offset nn sits in row
+// tb_fold_row(nn) ([even n-m | odd n-m] per 8 rows, so both parity classes of a folded chunk read consecutive
+// shared-memory rows; pitch 36 = 4 mod 16: conflict-free fragments).  The consumers and epilogues are therefore the same,
+// and so are the results, bit for bit.
 // ---------------------------------------------------------------------------------------------
-// NWN = warps along the columns: 6 (240-column items, one CTA per SM) for epoch batches, 2 (80-column items, two
-// CTAs per SM) for narrow batches, where an item is paced by the Legendre warps' dependent recursion and twice as many
-// resident items double the recursion throughput.
-constexpr int T1_TM = GB_T1_TM, T1_KC = GB_T1_KC, T1_STAGES = 4;
-constexpr int T1_LDA = T1_TM + 4;    // 68
-__host__ __device__ constexpr int t1_tn(int nwn) { return 40 * nwn; }
-__host__ __device__ constexpr int t1_threads(int nwn) { return 32 * (2 * nwn + 3); }   // + copy warp + 2 Legendre warps
-__host__ __device__ constexpr int t1_ctas_per_sm(int nwn) { return nwn <= 2 ? 2 : 1; }
-__host__ __device__ constexpr size_t t1_smem(int nwn) {
-    return (size_t)T1_STAGES * T1_KC * (T1_LDA + t1_tn(nwn) + 4) * sizeof(double) + 2 * T1_STAGES * sizeof(uint64_t);
+enum class S1Source { Table, Recursion };
+__host__ __device__ constexpr int s1_lda(bool fold) { return fold ? 36 : 68; }
+// one Legendre warp per 32 parallels of an item
+__host__ __device__ constexpr int s1_legendre_warps(bool fold, S1Source src) {
+    return src == S1Source::Recursion ? (fold ? 1 : 2) : 0;
 }
-
-struct T1Tables {
-    const double* ct_pad;   // [nlat_pad]
-    const double* kn_t;     // [L + 16][nlat_pad]
-    const double* pmm_t;    // [L][nlat_pad]
-    const double* rec_a;    // [L][lpad]   rec_a[m][n - m]
-    const double* rec_b;    // [L][lpad]
-    const double* zeros;
-    const int* krow;
-    int nlat_pad, lpad;
-};
-
-// FOLD (declared shortcut, grids that are symmetric about the equator): P_nm(pi - theta) = (-1)^(n-m) P_nm(theta), so an
-// item covers 32 northern parallels AND their mirror images: the degrees of a chunk are contracted in two parity
-// classes (even / odd n - m: every other shared-memory row), north = even + odd, south = even - odd.  Half the
-// recursion steps and half the DMMAs for the same output; one Legendre warp per item.
-template <bool PAIRS, int NWN, bool FOLD>   // PAIRS: nlat even, rows (e, i), (e, i+1) with i even are 16-byte aligned in AB
-__global__ void __launch_bounds__(t1_threads(NWN), t1_ctas_per_sm(NWN))
-gb_legendre_stage1(const double* __restrict__ X, double* __restrict__ AB, T1Tables tb, int L, int nlat, int E,
-                   int ab_rows, int n_lattiles, int n_coltiles, int n_items, int polar) {
-    // polar: FOLD -- number of leading 32-parallel tiles left to the unfolded launch; !FOLD -- nonzero selects the
-    // "polar cap" tiling (tile t = northern parallels [32t, 32t+32) and their mirror images), see launch_synthesis
-    constexpr int T1_TN = t1_tn(NWN), T1_LDB = T1_TN + 4, T1_CONSUMER_WARPS = 2 * NWN;
-    constexpr int T1_STAGE_DOUBLES = T1_KC * (T1_LDA + T1_LDB);
-    extern __shared__ __align__(128) unsigned char s_raw[];
-    double* s_tiles = reinterpret_cast<double*>(s_raw);
-    uint64_t* full = reinterpret_cast<uint64_t*>(s_raw + (size_t)T1_STAGES * T1_STAGE_DOUBLES * sizeof(double));
-    uint64_t* empty = full + T1_STAGES;
-    const int cols = 2 * E;
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < T1_STAGES; ++s) {
-            gb::mbar_init(&full[s], FOLD ? 2 : 3);           // copy warp (+tx bytes) and the Legendre warp(s)
-            gb::mbar_init(&empty[s], T1_CONSUMER_WARPS);
-        }
-        gb::fence_mbar_init();
-    }
-    __syncthreads();
-
-    int stage = 0;
-    uint32_t phase = 0;
-    const int tiles_per_pair = n_lattiles * n_coltiles;
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-        const int m_first = item / tiles_per_pair;
-        const int rem = item - m_first * tiles_per_pair;
-        const int i0 = FOLD ? (polar + rem / n_coltiles) * 32 : (rem / n_coltiles) * (polar ? 32 : T1_TM);
-        const int i_south = nlat - 64 - i0;            // cap tiling: rows 32..63 of the tile are parallels nlat-32-i0 ..
-        const int c0 = (rem % n_coltiles) * T1_TN;
-        const int m_second = L - 1 - m_first;
-        const int npass = (m_second == m_first) ? 1 : 2;
-        const int width = min(T1_TN, cols - c0);       // even
-
-        if (warp == T1_CONSUMER_WARPS) {
-            // ===== copy warp: the rows of X_m a chunk needs (whole 4-degree steps) =====
-            for (int pass = 0; pass < npass; ++pass) {
-                const int m = pass ? m_second : m_first;
-                const int Kn = L - m;
-                const int n_chunks = (Kn + T1_KC - 1) / T1_KC;
-                const long long xo = (long long)cols * ((long long)m * L - (long long)m * (m - 1) / 2);
-                const double* Xm = X + xo + c0;
-                for (int c = 0; c < n_chunks; ++c) {
-                    const int rows = min(T1_KC, FOLD ? ((Kn - c * T1_KC + 7) & ~7) : ((Kn - c * T1_KC + 3) & ~3));
-                    gb::mbar_wait(&empty[stage], phase ^ 1u);
-                    double* sB = s_tiles + (size_t)stage * T1_STAGE_DOUBLES + T1_KC * T1_LDA;
-                    if (lane == 0) gb::mbar_arrive_expect_tx(&full[stage], (uint32_t)(rows * width * sizeof(double)));
-                    __syncwarp();
-                    if (lane < rows) {
-                        const int nn = c * T1_KC + lane;
-                        const double* src = (nn < Kn) ? Xm + (size_t)nn * cols : tb.zeros;
-                        gb::bulk_g2s(sB + lane * T1_LDB, src, (uint32_t)(width * sizeof(double)), &full[stage]);
-                    }
-                    if (++stage == T1_STAGES) { stage = 0; phase ^= 1u; }
-                }
-            }
-        } else if (warp > T1_CONSUMER_WARPS) {
-            // ===== Legendre warps: lane = parallel, recursion state lives in registers =====
-            if (FOLD && warp != T1_CONSUMER_WARPS + 1) continue;      // folded items hold 32 parallels: one warp
-            const int li = (warp - T1_CONSUMER_WARPS - 1) * 32 + lane;
-            const int i = (!FOLD && polar && li >= 32) ? i_south + li : i0 + li;   // < nlat_pad; padded parallels read zeros
-            const double cti = tb.ct_pad[i];
-            for (int pass = 0; pass < npass; ++pass) {
-                const int m = pass ? m_second : m_first;
-                const int n_chunks = (L - m + T1_KC - 1) / T1_KC;
-                const double* kn_i = tb.kn_t + (size_t)m * tb.nlat_pad + i;
-                const double* c_ra = tb.rec_a + (size_t)m * tb.lpad;
-                const double* c_rb = tb.rec_b + (size_t)m * tb.lpad;
-                const double seed = tb.pmm_t[(size_t)m * tb.nlat_pad + i];
-                double p1 = 0.0, p2 = 0.0;
-                for (int c = 0; c < n_chunks; ++c) {
-                    // factors and recursion coefficients of the chunk first (independent loads in flight
-                    // together), then the serial chain: per degree one dependent multiply + subtract
-                    double knv[T1_KC], act[T1_KC], rbv[T1_KC];
-#pragma unroll
-                    for (int kk = 0; kk < T1_KC; ++kk) {
-                        const int nn = c * T1_KC + kk;
-                        knv[kk] = __ldg(kn_i + (size_t)nn * tb.nlat_pad);     // 0 beyond nmax / nlat
-                        act[kk] = __dmul_rn(__ldg(c_ra + nn), cti);
-                        rbv[kk] = __ldg(c_rb + nn);
-                    }
-                    gb::mbar_wait(&empty[stage], phase ^ 1u);
-                    double* sA = s_tiles + (size_t)stage * T1_STAGE_DOUBLES + li;
-#pragma unroll
-                    for (int kk = 0; kk < T1_KC; ++kk) {
-                        double pn;
-                        if (c == 0 && kk == 0) pn = seed;
-                        else pn = __dsub_rn(__dmul_rn(act[kk], p1), __dmul_rn(rbv[kk], p2));
-                        p2 = p1;
-                        p1 = pn;
-                        sA[kk * T1_LDA] = __dmul_rn(pn, knv[kk]);
-                    }
-                    __syncwarp();
-                    if (lane == 0) gb::mbar_arrive(&full[stage]);
-                    if (++stage == T1_STAGES) { stage = 0; phase ^= 1u; }
-                }
-            }
-        } else {
-            // ===== consumer warps: D[col][i] = sum_n X_m[n][col] Pk[n][i] =====
-            // The columns (e, cos|sin) are the M side of the DMMA tiles and the parallels the N side, so a
-            // thread ends up with two neighbouring parallels of one column: one 16-byte store into AB.
-            const int wm = warp / NWN;
-            const int wn = warp % NWN;
-            const int g = lane >> 2, q = lane & 3;
-            const bool has_columns = wn * 40 < width;      // narrow batches (few epochs): the other warps only keep the ring moving
-            if constexpr (FOLD) {
-                const int nh = nlat >> 1;
-                for (int pass = 0; pass < npass; ++pass) {
-                    const int m = pass ? m_second : m_first;
-                    const int Kn = L - m;
-                    const int n_chunks = (Kn + T1_KC - 1) / T1_KC;
-                    double ev[5][2][2], od[5][2][2];         // even / odd n - m, 40 columns x 16 northern parallels
-#pragma unroll
-                    for (int mi = 0; mi < 5; ++mi)
-#pragma unroll
-                        for (int ni = 0; ni < 2; ++ni) ev[mi][ni][0] = ev[mi][ni][1] = od[mi][ni][0] = od[mi][ni][1] = 0.0;
-                    for (int c = 0; c < n_chunks; ++c) {
-                        const int rows = Kn - c * T1_KC;
-                        gb::mbar_wait(&full[stage], phase);
-                        const double* sP = s_tiles + (size_t)stage * T1_STAGE_DOUBLES + wm * 16 + g;
-                        const double* sX = s_tiles + (size_t)stage * T1_STAGE_DOUBLES + T1_KC * T1_LDA + wn * 40 + g;
-#pragma unroll
-                        for (int kk = 0; kk < T1_KC; kk += 8) {
-                            if (kk >= rows || !has_columns) break;
-                            double a[5], b[2];
-#pragma unroll
-                            for (int mi = 0; mi < 5; ++mi) a[mi] = sX[(kk + 2 * q) * T1_LDB + mi * 8];
-#pragma unroll
-                            for (int ni = 0; ni < 2; ++ni) b[ni] = sP[(kk + 2 * q) * T1_LDA + ni * 8];
-#pragma unroll
-                            for (int mi = 0; mi < 5; ++mi)
-#pragma unroll
-                                for (int ni = 0; ni < 2; ++ni) gb::dmma_884(ev[mi][ni][0], ev[mi][ni][1], a[mi], b[ni]);
-#pragma unroll
-                            for (int mi = 0; mi < 5; ++mi) a[mi] = sX[(kk + 2 * q + 1) * T1_LDB + mi * 8];
-#pragma unroll
-                            for (int ni = 0; ni < 2; ++ni) b[ni] = sP[(kk + 2 * q + 1) * T1_LDA + ni * 8];
-#pragma unroll
-                            for (int mi = 0; mi < 5; ++mi)
-#pragma unroll
-                                for (int ni = 0; ni < 2; ++ni) gb::dmma_884(od[mi][ni][0], od[mi][ni][1], a[mi], b[ni]);
-                        }
-                        __syncwarp();
-                        if (lane == 0) gb::mbar_arrive(&empty[stage]);
-                        if (++stage == T1_STAGES) { stage = 0; phase ^= 1u; }
-                    }
-                    // epilogue: northern parallels i, i + 1 get even + odd, their mirror images nlat-1-i, nlat-2-i even - odd
-                    const int kc_row = tb.krow[2 * m], ks_row = tb.krow[2 * m + 1];
-                    const int ib = i0 + wm * 16 + 2 * q;
-#pragma unroll
-                    for (int mi = 0; mi < 5; ++mi) {
-                        const int col = c0 + wn * 40 + mi * 8 + g;
-                        if (col >= cols) continue;
-                        const int cs = col >= E;
-                        const int e = col - cs * E;
-                        const int k = cs ? ks_row : kc_row;
-#pragma unroll
-                        for (int ni = 0; ni < 2; ++ni) {
-                            const int i = ib + ni * 8;
-                            if (i >= nh) continue;               // nlat even: i even, so i + 1 < nh as well
-                            const long long rn = (long long)e * nlat + i;
-                            const long long rs = (long long)e * nlat + (nlat - 2 - i);
-                            gb::st_v2(AB + gb_ab_offset(rn, k, ab_rows), ev[mi][ni][0] + od[mi][ni][0],
-                                      ev[mi][ni][1] + od[mi][ni][1]);
-                            gb::st_v2(AB + gb_ab_offset(rs, k, ab_rows), ev[mi][ni][1] - od[mi][ni][1],
-                                      ev[mi][ni][0] - od[mi][ni][0]);
-                        }
-                    }
-                }
-                continue;
-            }
-            for (int pass = 0; pass < npass; ++pass) {
-                const int m = pass ? m_second : m_first;
-                const int Kn = L - m;
-                const int n_chunks = (Kn + T1_KC - 1) / T1_KC;
-                double acc[5][4][2];
-#pragma unroll
-                for (int mi = 0; mi < 5; ++mi)
-#pragma unroll
-                    for (int ni = 0; ni < 4; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
-                for (int c = 0; c < n_chunks; ++c) {
-                    const int rows = Kn - c * T1_KC;             // degrees left (whole steps are processed)
-                    gb::mbar_wait(&full[stage], phase);
-                    const double* sP = s_tiles + (size_t)stage * T1_STAGE_DOUBLES + wm * 32 + g;
-                    const double* sX = s_tiles + (size_t)stage * T1_STAGE_DOUBLES + T1_KC * T1_LDA + wn * 40 + g;
-#pragma unroll
-                    for (int kk = 0; kk < T1_KC; kk += 4) {
-                        if (kk >= rows || !has_columns) break;
-                        double a[5], b[4];
-#pragma unroll
-                        for (int mi = 0; mi < 5; ++mi) a[mi] = sX[(kk + q) * T1_LDB + mi * 8];
-#pragma unroll
-                        for (int ni = 0; ni < 4; ++ni) b[ni] = sP[(kk + q) * T1_LDA + ni * 8];
-#pragma unroll
-                        for (int mi = 0; mi < 5; ++mi)
-#pragma unroll
-                            for (int ni = 0; ni < 4; ++ni) gb::dmma_884(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
-                    }
-                    __syncwarp();
-                    if (lane == 0) gb::mbar_arrive(&empty[stage]);
-                    if (++stage == T1_STAGES) { stage = 0; phase ^= 1u; }
-                }
-                // epilogue: columns [0, E) are the cosine coefficients of epoch col, [E, 2E) the sines.
-                // The 32 parallels of a warp sit in at most two neighbouring 128-row tiles of AB.
-                const int kc_row = tb.krow[2 * m], ks_row = tb.krow[2 * m + 1];
-                const int ib = ((polar && wm) ? i_south : i0) + wm * 32 + 2 * q;
-                const int tile_step = ab_rows * GB_LDA - GB_TM;      // to the same k row of the next row tile
-#pragma unroll
-                for (int mi = 0; mi < 5; ++mi) {
-                    const int col = c0 + wn * 40 + mi * 8 + g;
-                    if (col >= cols) continue;
-                    const int cs = col >= E;
-                    const int e = col - cs * E;
-                    const long long row = (long long)e * nlat + ib;
-                    const int o0 = (int)(row & (GB_TM - 1));
-                    double* base = AB + ((size_t)(row >> 7) * ab_rows + (cs ? ks_row : kc_row)) * GB_LDA + o0;
-#pragma unroll
-                    for (int ni = 0; ni < 4; ++ni) {
-                        const int i = ib + ni * 8;
-                        if (PAIRS) {
-                            if (i < nlat)
-                                gb::st_v2(base + ni * 8 + ((o0 + ni * 8 >= GB_TM) ? tile_step : 0), acc[mi][ni][0],
-                                          acc[mi][ni][1]);
-                        } else {
-                            if (i < nlat) base[ni * 8 + ((o0 + ni * 8 >= GB_TM) ? tile_step : 0)] = acc[mi][ni][0];
-                            if (i + 1 < nlat)
-                                base[ni * 8 + 1 + ((o0 + ni * 8 + 1 >= GB_TM) ? tile_step : 0)] = acc[mi][ni][1];
-                        }
-                    }
-                }
-            }
-        }
-    }
+// Narrow column tiles run several CTAs per SM.  The recursion keeps at most two (an item there is paced by the Legendre
+// warps' dependent recursion, so resident items add throughput, but a third CTA would leave its warps too few registers).
+__host__ __device__ constexpr int s1_ctas_per_sm(int nwn, bool fold, S1Source src) {
+    return src == S1Source::Recursion ? (nwn <= 3 ? 2 : 1) : nwn <= 2 ? (fold ? 3 : 2) : nwn == 3 ? 2 : 1;
 }
-
-// ---------------------------------------------------------------------------------------------
-// stage 1 fed from the plan's Legendre table (the default).  kn[i,n] * P_nm(theta_i) does not depend on the epoch, so
-// the plan holds it -- written once by gb_ptab_kernel with the same bit-exact recursion -- in exactly the tile layout a
-// pipeline chunk needs: ONE bulk copy per chunk, no recursion warp, no FP64 instructions that compete with the DMMA
-// stream for the pipe (the on-the-fly recursion warp above was starved by the three DMMA-issuing warps of its
-// sub-partition: 300 cycles per degree, DMMA pipe 45 % active).  Same items, tiles, epilogues and AB layout as
-// gb_legendre_stage1; the degrees of a folded chunk are grouped [even n-m | odd n-m] per 8 rows, so both parity
-// classes read consecutive shared-memory rows (pitch 36 = 4 mod 16: conflict-free fragments).
-// ---------------------------------------------------------------------------------------------
-constexpr int TB_KC = 16;          // degrees per ring stage
-__host__ __device__ constexpr int tb_lda(bool fold) { return fold ? 36 : 68; }
-__host__ __device__ constexpr int tb_ctas_per_sm(int nwn, bool fold) { return nwn <= 2 ? (fold ? 3 : 2) : nwn == 3 ? 2 : 1; }
-__host__ __device__ constexpr size_t tb_stage_bytes(int nwn, bool fold) {
-    return (size_t)TB_KC * (tb_lda(fold) + t1_tn(nwn) + 4) * sizeof(double);
+__host__ __device__ constexpr int s1_threads(int nwn, bool fold, S1Source src) {
+    return 32 * (2 * nwn + 1 + s1_legendre_warps(fold, src));    // consumers + copy warp + Legendre warps
+}
+__host__ __device__ constexpr size_t s1_stage_bytes(int nwn, bool fold) {
+    return (size_t)GB_T1_KC * (s1_lda(fold) + 40 * nwn + 4) * sizeof(double);
 }
 // as many ring stages (at most 6) as the CTA's share of the 227 KB of shared memory holds
-__host__ __device__ constexpr int tb_stages(int nwn, bool fold) {
-    const size_t budget = (232448 - 1024 * tb_ctas_per_sm(nwn, fold)) / tb_ctas_per_sm(nwn, fold) - 128;
-    const int s = (int)(budget / tb_stage_bytes(nwn, fold));
+__host__ __device__ constexpr int s1_stages(int nwn, bool fold, S1Source src) {
+    const size_t budget = (232448 - 1024 * s1_ctas_per_sm(nwn, fold, src)) / s1_ctas_per_sm(nwn, fold, src) - 128;
+    const int s = (int)(budget / s1_stage_bytes(nwn, fold));
     return s > 6 ? 6 : s;
 }
-__host__ __device__ constexpr int tb_threads(int nwn) { return 32 * (2 * nwn + 1); }
-__host__ __device__ constexpr size_t tb_smem(int nwn, bool fold) {
-    return (size_t)tb_stages(nwn, fold) * tb_stage_bytes(nwn, fold) + 2 * tb_stages(nwn, fold) * sizeof(uint64_t);
+__host__ __device__ constexpr size_t s1_smem(int nwn, bool fold, S1Source src) {
+    return (size_t)s1_stages(nwn, fold, src) * s1_stage_bytes(nwn, fold) + 2 * s1_stages(nwn, fold, src) * sizeof(uint64_t);
 }
-// row of degree offset nn inside a folded table / chunk: even offsets first
+// row of degree offset nn inside a Legendre table / ring stage / tiled X: even offsets first
 __host__ __device__ __forceinline__ int tb_fold_row(int nn) { return (nn & ~7) + ((nn & 1) << 2) + ((nn & 7) >> 1); }
 __host__ __device__ __forceinline__ int tb_fold_degree(int row) {
     const int r = row & 7;
     return (row & ~7) + (r < 4 ? 2 * r : 2 * (r - 4) + 1);
 }
+// Parallel of column li of a stage-1 tile whose first (northern) parallel is i0, by tile kind (gb_common.cuh):
+// 0 folded -- inside every 16-column slab of a warp the columns are interleaved so that a lane's two DMMA fragments (tile
+//   columns 2q, 2q+1 and 8+2q, 9+2q) are FOUR CONSECUTIVE parallels 4q .. 4q+3: one 32-byte store per lane (parallels
+//   beyond the equator keep their own values: a lane's parallels may straddle it);
+// 1 polar cap -- 32 northern parallels, then their 32 mirror images (i_south = nlat - 64 - i0 onwards);
+// 2 plain -- 64 consecutive parallels.
+__host__ __device__ __forceinline__ int s1_parallel(int kind, int i0, int li, int nlat) {
+    if (kind == 0) {
+        const int cc = li & 15;
+        return i0 + (li & 16) + 4 * ((cc & 7) >> 1) + 2 * (cc >> 3) + (cc & 1);
+    }
+    return (kind == 1 && li >= 32) ? nlat - 64 - i0 + li : i0 + li;
+}
 
-struct TabArgs {
-    const double* tab;      // [lat tile][rtot][lda]
-    const int* roff;        // [L + 1]
-    long long tile_stride;  // rtot * lda
+struct S1Args {
+    const int* roff;        // [L + 1] first row of every order in the table and in the tiled X
     const int* krow;
+    const double* tab;      // Table: [lat tile][rtot][lda]
+    long long tile_stride;  // Table: rtot * lda
+    // Recursion: the plan's transposed, zero-padded recursion tables (gb_common.cuh)
+    const double* ct_pad;   // [nlat_pad]
+    const double* kn_t;     // [L + 16][nlat_pad]
+    const double* pmm_t;    // [L][nlat_pad]
+    const double* rec_a;    // [L][lpad]   rec_a[m][n - m]
+    const double* rec_b;    // [L][lpad]
+    int nlat_pad, lpad;
 };
 
+// PAIRS: nlat even, rows (e, i), (e, i+1) with i even are 16-byte aligned in AB.
+// FOLD (declared shortcut, grids that are symmetric about the equator): P_nm(pi - theta) = (-1)^(n-m) P_nm(theta), so an
+// item covers 32 northern parallels AND their mirror images: the degrees of a chunk are contracted in two parity
+// classes, north = even + odd, south = even - odd.  Half the recursion steps and half the DMMAs for the same output.
 // MI: 8-column fragments per consumer warp (5: 40 columns; 4: shards of at most 32 epochs, whose 64 columns then carry
 // no padding fragment)
-template <bool PAIRS, int NWN, bool FOLD, int MI = 5>
-__global__ void __launch_bounds__(tb_threads(NWN), tb_ctas_per_sm(NWN, FOLD))
-gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb, int L, int nlat, int E, int ab_rows,
-              int n_lattiles, int n_coltiles, int n_items, int polar) {
-    constexpr int KC = TB_KC, STAGES = tb_stages(NWN, FOLD);
+template <S1Source SRC, bool PAIRS, int NWN, bool FOLD, int MI>
+__global__ void __launch_bounds__(s1_threads(NWN, FOLD, SRC), s1_ctas_per_sm(NWN, FOLD, SRC))
+gb_stage1(const double* __restrict__ X, double* __restrict__ AB, S1Args tb, int L, int nlat, int E, int ab_rows,
+          int n_lattiles, int n_coltiles, int n_items, int polar) {
+    // polar: FOLD -- number of leading 32-parallel tiles left to the unfolded launch; !FOLD -- nonzero selects the
+    // "polar cap" tiling (tile t = northern parallels [32t, 32t+32) and their mirror images), see launch_synthesis
+    constexpr bool REC = SRC == S1Source::Recursion;
+    constexpr int KC = GB_T1_KC, STAGES = s1_stages(NWN, FOLD, SRC);
     static_assert(STAGES >= 2, "the ring needs at least two stages");
-    constexpr int TN = 8 * MI * NWN, LDA = tb_lda(FOLD), LDB = TN + 4, CONSUMER_WARPS = 2 * NWN;
+    constexpr int TN = 8 * MI * NWN, LDA = s1_lda(FOLD), LDB = TN + 4, CONSUMER_WARPS = 2 * NWN;
     constexpr int STAGE_DOUBLES = KC * (LDA + LDB);
     extern __shared__ __align__(128) unsigned char s_raw[];
     double* s_tiles = reinterpret_cast<double*>(s_raw);
@@ -441,7 +212,7 @@ gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb,
     if (threadIdx.x == 0) {
         GB_TRACE_MARK(0, 0);
         for (int s = 0; s < STAGES; ++s) {
-            gb::mbar_init(&full[s], 1);
+            gb::mbar_init(&full[s], 1 + s1_legendre_warps(FOLD, SRC));    // copy lane (+tx bytes), Legendre warps
             gb::mbar_init(&empty[s], CONSUMER_WARPS);
         }
         gb::fence_mbar_init();
@@ -449,13 +220,14 @@ gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb,
     __syncthreads();
     gb::griddep_launch_dependents();
     // griddepcontrol.wait (X comes from the pack kernel, AB is still being read by the previous call) is executed by the
-    // copy lane alone: the Legendre table is a plan constant, so the table halves of the first ring stages are already in
-    // flight (a cold DRAM round trip after an L2 flush) when the wait returns; the consumers touch global memory only
-    // after they have seen chunks of X, which the copy lane requests after the wait.
+    // copy lane alone: the Legendre table and the recursion tables are plan constants, so the table halves of the first
+    // ring stages are already in flight (a cold DRAM round trip after an L2 flush) when the wait returns, and the
+    // Legendre warps start their recursion at once; the consumers touch global memory only after they have seen chunks
+    // of X, which the copy lane requests after the wait.
     const int tiles_per_pair = n_lattiles * n_coltiles;
     int n_pre = 0;                      // chunks whose table half (and byte count) went out before the wait
     if (warp == CONSUMER_WARPS && lane == 0) {
-        for (int item = blockIdx.x; item < n_items && n_pre < STAGES; item += gridDim.x) {
+        for (int item = blockIdx.x; !REC && item < n_items && n_pre < STAGES; item += gridDim.x) {
             const int m_first = item / tiles_per_pair;
             const int lt = (item - m_first * tiles_per_pair) / n_coltiles;
             const int m_second = L - 1 - m_first;
@@ -483,7 +255,7 @@ gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb,
         const int m_first = item / tiles_per_pair;
         const int rem = item - m_first * tiles_per_pair;
         const int lt = rem / n_coltiles;
-        const int i0 = FOLD ? (polar + lt) * 32 : lt * (polar ? 32 : T1_TM);
+        const int i0 = FOLD ? (polar + lt) * 32 : lt * (polar ? 32 : GB_T1_TM);
         const int i_south = nlat - 64 - i0;
         const int c0 = (rem % n_coltiles) * TN;
         const int m_second = L - 1 - m_first;
@@ -491,7 +263,7 @@ gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb,
         const int width = min(TN, cols - c0);
 
         if (warp == CONSUMER_WARPS) {
-            // ===== copy warp (one elected lane): one bulk copy for the table chunk, one for the chunk of X_m =====
+            // ===== copy warp (one elected lane): one bulk copy for the chunk of X_m (and one for the table chunk) =====
             if (lane == 0) {
                 const double* tab_t = tb.tab + (size_t)lt * tb.tile_stride;
                 const int ct = rem % n_coltiles;
@@ -503,21 +275,64 @@ gb_stage1_tab(const double* __restrict__ X, double* __restrict__ AB, TabArgs tb,
                     for (int r = 0; r < kn_pad; r += KC) {
                         const int rows = min(KC, kn_pad - r);
                         double* sA = s_tiles + (size_t)stage * STAGE_DOUBLES;
-                        if (chunk_idx++ >= n_pre) {
+                        if (REC || chunk_idx++ >= n_pre) {
                             gb::mbar_wait(&empty[stage], phase ^ 1u);
-                            gb::mbar_arrive_expect_tx(&full[stage], (uint32_t)(rows * (LDB + LDA) * sizeof(double)));
-                            gb::bulk_g2s(sA, tab_m + (size_t)r * LDA, (uint32_t)(rows * LDA * sizeof(double)), &full[stage]);
+                            gb::mbar_arrive_expect_tx(&full[stage], (uint32_t)(rows * (REC ? LDB : LDB + LDA) * sizeof(double)));
+                            if (!REC)
+                                gb::bulk_g2s(sA, tab_m + (size_t)r * LDA, (uint32_t)(rows * LDA * sizeof(double)), &full[stage]);
                         }
                         gb::bulk_g2s(sA + KC * LDA, x_m + (size_t)r * LDB, (uint32_t)(rows * LDB * sizeof(double)), &full[stage]);
                         if (++stage == STAGES) { stage = 0; phase ^= 1u; }
                     }
                 }
             }
+        } else if (REC && warp > CONSUMER_WARPS) {
+            // ===== Legendre warps: lane = column li of the tile, recursion state lives in registers =====
+            const int li = (warp - CONSUMER_WARPS - 1) * 32 + lane;
+            const int i = s1_parallel(FOLD ? 0 : polar ? 1 : 2, i0, li, nlat);   // < nlat_pad; padded parallels read zeros
+            const double cti = tb.ct_pad[i];
+            for (int pass = 0; pass < npass; ++pass) {
+                const int m = pass ? m_second : m_first;
+                const int n_chunks = (L - m + KC - 1) / KC;
+                const double* kn_i = tb.kn_t + (size_t)m * tb.nlat_pad + i;
+                const double* c_ra = tb.rec_a + (size_t)m * tb.lpad;
+                const double* c_rb = tb.rec_b + (size_t)m * tb.lpad;
+                const double seed = tb.pmm_t[(size_t)m * tb.nlat_pad + i];
+                double p1 = 0.0, p2 = 0.0;
+                for (int c = 0; c < n_chunks; ++c) {
+                    // factors and recursion coefficients of the chunk first (independent loads in flight
+                    // together), then the serial chain: per degree one dependent multiply + subtract
+                    double knv[KC], act[KC], rbv[KC];
+#pragma unroll
+                    for (int kk = 0; kk < KC; ++kk) {
+                        const int nn = c * KC + kk;
+                        knv[kk] = __ldg(kn_i + (size_t)nn * tb.nlat_pad);     // 0 beyond nmax / nlat
+                        act[kk] = __dmul_rn(__ldg(c_ra + nn), cti);
+                        rbv[kk] = __ldg(c_rb + nn);
+                    }
+                    gb::mbar_wait(&empty[stage], phase ^ 1u);
+                    double* sA = s_tiles + (size_t)stage * STAGE_DOUBLES + li;
+#pragma unroll
+                    for (int kk = 0; kk < KC; ++kk) {
+                        double pn;
+                        if (c == 0 && kk == 0) pn = seed;
+                        else pn = __dsub_rn(__dmul_rn(act[kk], p1), __dmul_rn(rbv[kk], p2));
+                        p2 = p1;
+                        p1 = pn;
+                        sA[tb_fold_row(kk) * LDA] = __dmul_rn(pn, knv[kk]);
+                    }
+                    __syncwarp();
+                    if (lane == 0) gb::mbar_arrive(&full[stage]);
+                    if (++stage == STAGES) { stage = 0; phase ^= 1u; }
+                }
+            }
         } else {
+            // ===== consumer warps: D[col][i] = sum_n X_m[n][col] Pk[n][i], the columns (e, cos|sin) on the M side of the
+            // DMMA tiles and the parallels on the N side =====
             const int wm = warp / NWN;
             const int wn = warp % NWN;
             const int g = lane >> 2, q = lane & 3;
-            const bool has_columns = wn * (8 * MI) < width;
+            const bool has_columns = wn * (8 * MI) < width;    // narrow batches: the other warps only keep the ring moving
             if constexpr (FOLD) {
                 const int nh = nlat >> 1;
                 for (int pass = 0; pass < npass; ++pass) {
@@ -693,18 +508,7 @@ gb_ptab_kernel(double* __restrict__ tab, const int* __restrict__ roff, long long
     const int li = (int)(idx % per_tile);
     const int m = (int)((idx / per_tile) % L);
     const int t = (int)(idx / ((long long)per_tile * L));
-    int i;
-    if (kind == 0) {
-        // inside every 16-column slab of a warp the columns are interleaved so that a lane's two DMMA fragments (tile
-        // columns 2q, 2q+1 and 8+2q, 9+2q) are FOUR CONSECUTIVE parallels 4q .. 4q+3: one 32-byte store per lane
-        const int cc = li & 15;
-        i = (tile0 + t) * 32 + (li & 16) + 4 * ((cc & 7) >> 1) + 2 * (cc >> 3) + (cc & 1);
-        // (parallels beyond the equator keep their own values: a lane's parallels may straddle it)
-    } else if (kind == 1) {
-        i = li < 32 ? t * 32 + li : nlat - 64 - 32 * t + li;
-    } else {
-        i = t * 64 + li;
-    }
+    const int i = s1_parallel(kind, kind == 2 ? t * 64 : (kind == 0 ? tile0 + t : t) * 32, li, nlat);   // i0 as in gb_stage1
     if (i < 0 || i >= nlat) return;
     double* out = tab + ((size_t)t * rtot + roff[m]) * lda + li;
     const double* kn_i = kn + (size_t)i * L;
@@ -1393,8 +1197,8 @@ gb_legendre_table_kernel(double* __restrict__ out, const double* __restrict__ ct
 constexpr size_t PTAB_MAX_BYTES = (size_t)2048 << 20;     // memory budget of one Legendre table
 
 // Build (once) the Legendre table of `kind` (gb_common.cuh: 0 folded tiles, 1 polar-cap tiles, 2 plain tiles).
-// Returns 1 if the table exists, 0 if it is over PTAB_MAX_BYTES or cannot be allocated (the caller then runs the
-// on-the-fly recursion kernel), < 0 on error (-code).
+// Returns 1 if the table exists, 0 if it is over PTAB_MAX_BYTES or cannot be allocated (the caller then runs stage 1
+// in its Recursion mode), < 0 on error (-code).
 static int ensure_ptab(gb_plan* p, int kind, int n_tiles, int tile0, cudaStream_t st) {
     if (p->ptab_state[kind] != 0) return p->ptab_state[kind] > 0 ? 1 : 0;
     const int L = p->L;
@@ -1406,7 +1210,7 @@ static int ensure_ptab(gb_plan* p, int kind, int n_tiles, int tile0, cudaStream_
     }
     if (cudaMalloc(reinterpret_cast<void**>(&p->d_ptab[kind]), elems * sizeof(double)) != cudaSuccess) {
         cudaGetLastError();
-        p->ptab_state[kind] = -1;          // no room: the recursion kernel needs none
+        p->ptab_state[kind] = -1;          // no room: the Recursion mode needs none
         return 0;
     }
     cudaError_t e = cudaMemsetAsync(p->d_ptab[kind], 0, elems * sizeof(double), st);
@@ -1436,14 +1240,14 @@ struct S1Tiling {
     int tn() const { return 8 * mi * nwn; }
 };
 
-// Narrow batches (at most 80 epochs) run 80-column items, several CTAs per SM; wider batches 240-column items.  The
-// table-fed kernel on folded grids without polar caps (tab_fold) has two more tilings.
-static S1Tiling stage1_tiling(int E, bool tab_fold) {
+// Narrow batches (at most 80 epochs) run 80-column items, several CTAs per SM; wider batches 240-column items.  Folded
+// grids without polar caps (fold_only: nothing runs the unfolded instances there) have two more tilings.
+static S1Tiling stage1_tiling(int E, bool fold_only) {
     const int cols = 2 * E;
-    if (tab_fold && cols <= 64) return {2, 4};      // shards of at most 32 epochs: 64-column items (no padding fragment)
+    if (fold_only && cols <= 64) return {2, 4};      // shards of at most 32 epochs: 64-column items (no padding fragment)
     // 41 .. 60 epochs: ONE 120-column tile per order pair and latitude tile, two CTAs per SM (80-column tiles would leave
     // a second, mostly empty round of items)
-    if (tab_fold && cols > 80 && cols <= 120) return {3, 5};
+    if (fold_only && cols > 80 && cols <= 120) return {3, 5};
     return cols <= 160 ? S1Tiling{2, 5} : S1Tiling{6, 5};
 }
 
@@ -1451,50 +1255,55 @@ static S1Tiling stage1_tiling(int E, bool tab_fold) {
 struct S1Launch {
     gb_plan* p;
     const int* krow;
+    S1Tiling tiling;
     int E, n_coltiles;
     cudaStream_t st;
 };
 
-// Table-fed stage 1 over `lattiles` latitude tiles of the plan's table of `kind`.  Threads and shared memory follow from
-// the template arguments.
-template <bool PAIRS, int NWN, bool FOLD, int MI = 5>
-static int launch_tab(const S1Launch& a, int kind, int lattiles, int items, int polar) {
+// Stage 1 over `lattiles` latitude tiles of `kind` (gb_common.cuh).  Threads and shared memory follow from the template
+// arguments.
+template <S1Source SRC, bool PAIRS, int NWN, bool FOLD, int MI>
+static int launch_stage1(const S1Launch& a, int kind, int lattiles, int items, int polar) {
     const gb_plan* p = a.p;
-    auto kernel = gb_stage1_tab<PAIRS, NWN, FOLD, MI>;
-    const int max_ctas = tb_ctas_per_sm(NWN, FOLD) * p->sm_count;
+    auto kernel = gb_stage1<SRC, PAIRS, NWN, FOLD, MI>;
+    constexpr int ctas_per_sm = s1_ctas_per_sm(NWN, FOLD, SRC);
+    const int max_ctas = ctas_per_sm * p->sm_count;
     const int grid = items < max_ctas ? items : max_ctas;
-    size_t smem = tb_smem(NWN, FOLD);
+    size_t smem = s1_smem(NWN, FOLD, SRC);
     // Fewer items than CTA slots (a narrow shard): the CTAs are launched while the pack kernel still holds part of every
     // SM (programmatic dependent launch) and the block scheduler fills whatever is free first -- three CTAs on some SMs,
     // one on others, and the crowded SMs finish last.  Asking for more shared memory than a CTA needs caps the CTAs per
     // SM at the even share.
     const int per_sm = (grid + p->sm_count - 1) / p->sm_count;
-    if (per_sm < tb_ctas_per_sm(NWN, FOLD)) {
+    if (per_sm < ctas_per_sm) {
         const size_t forbid = 233472 / (size_t)(per_sm + 1) - 1024 + 256;      // per_sm + 1 CTAs no longer fit
         const size_t allow = 233472 / (size_t)per_sm - 1024;                    // per_sm CTAs still do
         if (forbid > smem && forbid <= allow && forbid <= 232448) smem = forbid;
     }
-    const TabArgs ta{p->d_ptab[kind], p->d_ptab_roff, p->ptab_rtot * tb_lda(FOLD), a.krow};
+    const S1Args args{p->d_ptab_roff, a.krow,     p->d_ptab[kind], p->ptab_rtot * s1_lda(FOLD), p->d_ct_pad, p->d_kn_t,
+                      p->d_pmm_t,     p->d_rec_a, p->d_rec_b,      p->nlat_pad,                 p->lpad};
     GB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    GB_CUDA(gb_launch_pdl(kernel, dim3(grid), dim3(tb_threads(NWN)), smem, a.st, p->d_x, p->d_ab, ta, p->L, p->nlat, a.E,
-                          p->ab_rows, lattiles, a.n_coltiles, items, polar));
+    GB_CUDA(gb_launch_pdl(kernel, dim3(grid), dim3(s1_threads(NWN, FOLD, SRC)), smem, a.st, p->d_x, p->d_ab, args, p->L,
+                          p->nlat, a.E, p->ab_rows, lattiles, a.n_coltiles, items, polar));
     GB_LAUNCH_CHECK();
     return GB_OK;
 }
 
-// Stage 1 with the Legendre recursion on the fly (no table), same items as launch_tab with MI = 5.
-template <bool PAIRS, int NWN, bool FOLD>
-static int launch_otf(const S1Launch& a, int lattiles, int items, int polar) {
-    const gb_plan* p = a.p;
-    const int max_ctas = t1_ctas_per_sm(NWN) * p->sm_count;
-    const int grid = items < max_ctas ? items : max_ctas;
-    const T1Tables tb{p->d_ct_pad, p->d_kn_t, p->d_pmm_t, p->d_rec_a, p->d_rec_b, p->d_zero, a.krow, p->nlat_pad, p->lpad};
-    GB_CUDA(cudaFuncSetAttribute(gb_legendre_stage1<PAIRS, NWN, FOLD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)t1_smem(NWN)));
-    gb_legendre_stage1<PAIRS, NWN, FOLD><<<grid, t1_threads(NWN), t1_smem(NWN), a.st>>>(
-        p->d_x, p->d_ab, tb, p->L, p->nlat, a.E, p->ab_rows, lattiles, a.n_coltiles, items, polar);
-    GB_LAUNCH_CHECK();
-    return GB_OK;
+// The stage-1 instance for the tiling, the fold and the parity of the parallel count (folded grids have an even one).
+template <S1Source SRC>
+static int dispatch_stage1(const S1Launch& a, bool fold, bool pairs, int kind, int lattiles, int items, int polar) {
+    const S1Tiling t = a.tiling;
+    if (fold) {
+        if (t.mi == 4) return launch_stage1<SRC, true, 2, true, 4>(a, kind, lattiles, items, polar);
+        if (t.nwn == 2) return launch_stage1<SRC, true, 2, true, 5>(a, kind, lattiles, items, polar);
+        if (t.nwn == 3) return launch_stage1<SRC, true, 3, true, 5>(a, kind, lattiles, items, polar);
+        return launch_stage1<SRC, true, 6, true, 5>(a, kind, lattiles, items, polar);
+    }
+    if (t.nwn == 2)
+        return pairs ? launch_stage1<SRC, true, 2, false, 5>(a, kind, lattiles, items, polar)
+                     : launch_stage1<SRC, false, 2, false, 5>(a, kind, lattiles, items, polar);
+    return pairs ? launch_stage1<SRC, true, 6, false, 5>(a, kind, lattiles, items, polar)
+                 : launch_stage1<SRC, false, 6, false, 5>(a, kind, lattiles, items, polar);
 }
 
 // the eight-fold symmetric stage 2: plan gate + override
@@ -1555,20 +1364,20 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
     const bool naive2 = gb_env_flag("GB_NAIVE_STAGE2");
     const bool use_sym = p->sym && !naive2 && !gb_env_flag("GB_NO_SYMMETRY");
     const int* d_krow = use_sym ? gb_stage2_krow(p) : p->d_krow_id;
-    const bool simple1 = gb_env_flag("GB_SIMPLE_STAGE1");
+    const bool simple1 = gb_env_flag("GB_SIMPLE_STAGE1");           // FMA cross-check on the order-wise X
     const bool fold = p->fold_ns && !gb_env_flag("GB_NO_FOLD");     // equatorial symmetry: 32 northern parallels per item
     const int cap_tiles = fold ? p->fold_cap / 32 : 0;              // polar tiles that stay unfolded
-    const int n_lattiles = fold ? (p->nlat / 2 + 31) / 32 - cap_tiles : (p->nlat + T1_TM - 1) / T1_TM;
-    // the Legendre table(s) of these latitude tiles; 0 = over budget -> on-the-fly recursion
+    const int n_lattiles = fold ? (p->nlat / 2 + 31) / 32 - cap_tiles : (p->nlat + GB_T1_TM - 1) / GB_T1_TM;
+    // the Legendre table(s) of these latitude tiles; 0 = over budget -> recursion on the fly
     int have_tab = (simple1 || gb_env_flag("GB_S1_ONTHEFLY")) ? 0 : ensure_ptab(p, fold ? 0 : 2, n_lattiles, cap_tiles, st);
     if (have_tab > 0 && cap_tiles > 0) have_tab = ensure_ptab(p, 1, cap_tiles, 0, st);
     if (have_tab < 0) return -have_tab;
-    const S1Tiling tiling = stage1_tiling(E, have_tab && fold && p->fold_cap == 0);
+    const S1Tiling tiling = stage1_tiling(E, fold && cap_tiles == 0);
     const int tn = tiling.tn();
     const int n_coltiles = (2 * E + tn - 1) / tn;
     const int n_items = (L + 1) / 2 * n_lattiles * n_coltiles;     // order pairs (p, nmax - p) x tiles
     const int cap_items = (L + 1) / 2 * cap_tiles * n_coltiles;
-    if (have_tab) {
+    if (!simple1) {
         // tiled X: pad rows, pad columns and the (non-existent) sine plane of order 0 are never written by the pack
         const long long key = ((long long)E << 16) | tn;
         if (p->x_layout_key != key) {
@@ -1582,11 +1391,11 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
     if (flt) {
         // pack -> filter, whose epilogue writes X in the layout the Legendre stage reads (no unpack / second pack)
         int rc = gb_filter_into_x(flt->d_blocks, flt->block_offsets, flt->nf, d_anm, E, p->nmax, p->d_x,
-                                  have_tab ? p->d_ptab_roff : nullptr, tn, n_coltiles, st);
+                                  simple1 ? nullptr : p->d_ptab_roff, tn, n_coltiles, st);
         if (rc) return rc;
     } else {
-        int rc = have_tab ? gb_launch_pack_tiled(d_anm, p->d_x, L, E, p->d_ptab_roff, tn, n_coltiles, st, d_wn)
-                          : gb_launch_pack(d_anm, p->d_x, L, E, st, d_wn);
+        int rc = simple1 ? gb_launch_pack(d_anm, p->d_x, L, E, st, d_wn)
+                         : gb_launch_pack_tiled(d_anm, p->d_x, L, E, p->d_ptab_roff, tn, n_coltiles, st, d_wn);
         if (rc) return rc;
     }
     if (prof) GB_CUDA(cudaEventRecord(prof[1], st));
@@ -1600,37 +1409,15 @@ static int launch_synthesis(gb_plan* p, const double* d_anm, int E, double* d_ou
         GB_LAUNCH_CHECK();
     } else {
         // the polar caps (parallels whose mirror image is not close enough in the reference's tables) run the unfolded
-        // kernel on tiles of 32 northern parallels + their 32 mirror images (polar = 1); tiling.nwn is 2 or 6 outside
-        // the first branch
-        const S1Launch a{p, d_krow, E, n_coltiles, st};
+        // kernel on tiles of 32 northern parallels + their 32 mirror images (kind 1, polar = 1)
+        const S1Launch a{p, d_krow, tiling, E, n_coltiles, st};
         const bool pairs = p->nlat % 2 == 0;
-        const bool nw2 = tiling.nwn == 2;
-        int rc;
-        if (have_tab && fold) {
-            rc = tiling.mi == 4 ? launch_tab<true, 2, true, 4>(a, 0, n_lattiles, n_items, cap_tiles)
-                 : nw2 ? launch_tab<true, 2, true>(a, 0, n_lattiles, n_items, cap_tiles)
-                 : tiling.nwn == 3 ? launch_tab<true, 3, true>(a, 0, n_lattiles, n_items, cap_tiles)
-                                   : launch_tab<true, 6, true>(a, 0, n_lattiles, n_items, cap_tiles);
-            if (!rc && cap_tiles > 0)
-                rc = nw2 ? launch_tab<true, 2, false>(a, 1, cap_tiles, cap_items, 1)
-                         : launch_tab<true, 6, false>(a, 1, cap_tiles, cap_items, 1);
-        } else if (have_tab) {
-            rc = nw2 ? (pairs ? launch_tab<true, 2, false>(a, 2, n_lattiles, n_items, 0)
-                              : launch_tab<false, 2, false>(a, 2, n_lattiles, n_items, 0))
-                     : (pairs ? launch_tab<true, 6, false>(a, 2, n_lattiles, n_items, 0)
-                              : launch_tab<false, 6, false>(a, 2, n_lattiles, n_items, 0));
-        } else if (fold) {              // implies an even number of parallels
-            rc = nw2 ? launch_otf<true, 2, true>(a, n_lattiles, n_items, cap_tiles)
-                     : launch_otf<true, 6, true>(a, n_lattiles, n_items, cap_tiles);
-            if (!rc && cap_tiles > 0)
-                rc = nw2 ? launch_otf<true, 2, false>(a, cap_tiles, cap_items, 1)
-                         : launch_otf<true, 6, false>(a, cap_tiles, cap_items, 1);
-        } else {
-            rc = nw2 ? (pairs ? launch_otf<true, 2, false>(a, n_lattiles, n_items, 0)
-                              : launch_otf<false, 2, false>(a, n_lattiles, n_items, 0))
-                     : (pairs ? launch_otf<true, 6, false>(a, n_lattiles, n_items, 0)
-                              : launch_otf<false, 6, false>(a, n_lattiles, n_items, 0));
-        }
+        auto stage1 = [&](bool f, int kind, int lattiles, int items, int polar) {
+            return have_tab ? dispatch_stage1<S1Source::Table>(a, f, pairs, kind, lattiles, items, polar)
+                            : dispatch_stage1<S1Source::Recursion>(a, f, pairs, kind, lattiles, items, polar);
+        };
+        int rc = stage1(fold, fold ? 0 : 2, n_lattiles, n_items, cap_tiles);
+        if (!rc && cap_tiles > 0) rc = stage1(false, 1, cap_tiles, cap_items, 1);
         if (rc) return rc;
     }
     if (prof) GB_CUDA(cudaEventRecord(prof[2], st));

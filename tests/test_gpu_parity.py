@@ -174,7 +174,7 @@ def test_synthesis_equator_fold_vs_unfolded(gb, orc, monkeypatch, nmax, dlat, E)
         assert maxnorm_err(folded[e], plain[e]) < 5e-13
 
 
-def test_equator_fold_is_gated_on_measured_asymmetry(gb):
+def test_equator_fold_is_gated_on_measured_asymmetry(gb, orc):
     """On a 0.25 degree grid one parallel next to the pole fails the gate (the reference's colatitudes there differ
     between the hemispheres by more than it allows): its tile of 32 parallels per hemisphere stays with the unfolded
     stage, the rest is folded.  Grids that are not mirror images are not folded at all."""
@@ -187,6 +187,50 @@ def test_equator_fold_is_gated_on_measured_asymmetry(gb):
     par[3] += 1e-9
     assert not gb.get_plan(gb.RegularGrid(gb.GeographicGrid(10.0, 10.0).meridians, par), 8, "ewh").folded
     assert not gb.get_plan(gb.RegularGrid(gb.GeographicGrid(10.0, 10.0).meridians, par[:-1]), 8, "ewh").folded   # odd count
+    # a parallel in the second tile of 32 that fails the gate: two polar-cap tiles per pole, still exact
+    grid, og = _two_cap_grid(gb, orc)
+    assert lib.gb_plan_is_folded(gb.get_plan(grid, 60, "ewh")._handle) == 3
+    anm = np.stack([orc.synthetic_coefficients(60, e) for e in range(2)])
+    ref = np.stack([orc.synthesis(a, og, "ewh") for a in anm])
+    assert maxnorm_err(gb.to_grid_batch(anm, grid, "ewh"), ref) < TOL
+
+
+def _two_cap_grid(gb, orc):
+    """0.5 degree parallels (1 degree meridians) with parallel 40 moved by 1e-9: it fails the fold gate, so the first
+    two tiles of 32 parallels per hemisphere run unfolded (gb_plan_is_folded == 3).  Returns the grid and its oracle."""
+    base = gb.GeographicGrid(1.0, 0.5)
+    par = base.parallels.copy()
+    par[40] += 1e-9
+    return gb.RegularGrid(base.meridians, par), orc.OracleGrid(base.meridians, par)
+
+
+@pytest.mark.parametrize("E", [11, 55, 70, 100])         # the 64-, 120-, 80- and 240-column tilings
+def test_stage1_recursion_matches_table(gb, orc, monkeypatch, E):
+    """Without the plan's Legendre table (over its memory budget; GB_S1_ONTHEFLY=1 forces it) the Legendre stage runs the
+    recursion inside the kernel and lays its ring stages out like the table: the results are bit-identical on folded
+    grids with and without polar caps and on unfolded grids with an even and an odd number of parallels."""
+    lib = gb._lib.load()
+    geo3 = gb.GeographicGrid(3.0, 3.0)
+    # grid, degree, GB_NO_FOLD, gb_plan_is_folded (1: folded, 2 / 3: folded with one / two polar-cap tiles per pole)
+    cases = ((geo3, 40, False, 1), (gb.GeographicGrid(1.0, 0.25), 60, False, 2), (_two_cap_grid(gb, orc)[0], 60, False, 3),
+             (geo3, 40, True, 1), (gb.RegularGrid(geo3.meridians, geo3.parallels[:-1]), 40, False, 0))
+    rng = np.random.default_rng(E)
+    for grid, N, no_fold, folded in cases:
+        assert lib.gb_plan_is_folded(gb.get_plan(grid, N, "ewh")._handle) == folded
+        x = torch.as_tensor(rng.standard_normal((E, N + 1, N + 1))).cuda()
+        if no_fold:
+            monkeypatch.setenv("GB_NO_FOLD", "1")
+        table = gb.to_grid_batch(x, grid, "ewh")
+        monkeypatch.setenv("GB_S1_ONTHEFLY", "1")
+        rec = gb.to_grid_batch(x, grid, "ewh")
+        monkeypatch.delenv("GB_S1_ONTHEFLY")
+        monkeypatch.delenv("GB_NO_FOLD", raising=False)
+        assert torch.equal(table, rec), (grid.parallels.size, N, no_fold)
+    flt = gb.OrderWiseFilter(orc.synthetic_filter_blocks(40))
+    x = torch.as_tensor(rng.standard_normal((E, 41, 41))).cuda()
+    table = gb.to_grid_batch(x, geo3, "ewh", orderwise_filter=flt)
+    monkeypatch.setenv("GB_S1_ONTHEFLY", "1")
+    assert torch.equal(gb.to_grid_batch(x, geo3, "ewh", orderwise_filter=flt), table)
 
 
 @pytest.mark.parametrize("nmax,dlon,dlat,E", [(1, 30.0, 30.0, 1), (2, 90.0, 45.0, 2), (17, 7.5, 4.0, 7),
@@ -972,9 +1016,9 @@ def test_orderwise_filter_batch_then_synthesis(gb, orc):
     vals = gb.to_grid_batch(dev, grid, "ewh").cpu().numpy()
     og = orc.geographic_grid(3.0, 3.0)
     assert maxnorm_err(vals, np.stack([orc.synthesis(a, og, "ewh") for a in ref])) < TOL
-    # fused: the filter writes into the synthesis workspace (tiled layout of the table-fed Legendre stage, or the
-    # order-wise layout of the on-the-fly stage); bit-identical to the two calls, on folded and unfolded grids,
-    # batches above and below the narrow-tile limit, a filter of higher degree than the data
+    # fused: the filter writes into the synthesis workspace (the tiled layout the Legendre stage reads, whether it is fed
+    # from the table or runs the recursion); bit-identical to the two calls, on folded and unfolded grids, batches above
+    # and below the narrow-tile limit, a filter of higher degree than the data
     x = torch.as_tensor(anm).cuda()
     for g2 in (grid, gb.GeographicGrid(7.0, 5.0), gb.GaussGrid(19)):
         for xe in (x, x[:3], torch.cat([x] * 5), torch.cat([x] * 9)):      # 64-, 120- (55 epochs) and 240-column items

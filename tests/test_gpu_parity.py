@@ -952,7 +952,7 @@ def test_radial_basis_functions_golden_and_batch(gb, orc, golden):
     aout = abf.to_grid(gb.GeographicGrid(10.0, 10.0), "ewh")
     assert maxnorm_err(aout.value_array, g["aniso_grid_ewh"]) < TOL
     rng = np.random.default_rng(8)
-    N, P, E = 45, 5000, 130                     # 17 coefficient tiles, two epoch tiles, ragged last point block
+    N, P, E = 45, 5000, 130                     # 17 coefficient tiles, two epoch tiles, one block of points (16 384 max)
     lon = rng.uniform(-np.pi, np.pi, P)
     lat = np.arcsin(rng.uniform(-1, 1, P))
     K = rng.uniform(0.5, 1.5, (N + 1, N + 1))

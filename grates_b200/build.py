@@ -13,7 +13,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIBDIR, "libgrates_b200.so")
-SOURCES = ["gb_plan.cu", "gb_pack.cu", "gb_synthesis.cu", "gb_analysis.cu", "gb_covprop.cu", "gb_filter.cu", "gb_points.cu", "gb_matrices.cu", "gb_reduce.cu", "gb_densefilter.cu", "gb_linalg.cu"]
+SOURCES = ["gb_plan.cu", "gb_pack.cu", "gb_synthesis.cu", "gb_analysis.cu", "gb_covprop.cu", "gb_filter.cu", "gb_points.cu", "gb_matrices.cu", "gb_reduce.cu", "gb_densefilter.cu", "gb_linalg.cu", "gb_gradient.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-extended-lambda"]
 

@@ -466,6 +466,94 @@ def to_grid_batch(anm, grid=None, kernel='ewh', GM=GM_DEFAULT, R=R_DEFAULT, devi
     return p.synthesis_host(anm, out=out)
 
 
+_FRAMES = ('cartesian', 'local')
+
+
+def _gradient_input(anm, frame):
+    """Checks that need no device: the frame name, the shape [E, L, L] and, for a tensor, float64 on a CUDA device."""
+    if frame not in _FRAMES:
+        raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
+    x = anm if isinstance(anm, torch.Tensor) else np.ascontiguousarray(anm, dtype=float)
+    if x.ndim != 3 or x.shape[1] != x.shape[2]:
+        raise ValueError("coefficients must have shape [epochs, L, L] (got {0})".format(tuple(x.shape)))
+    if isinstance(x, torch.Tensor) and (x.dtype != torch.float64 or not x.is_cuda):
+        raise ValueError("coefficients must be a float64 CUDA tensor")
+    return x
+
+
+def _gradient(x, p, frame, shape, device_output, out):
+    """Transform (gb_gradient_coefficients), one synthesis of the 3E sets on the gradient plan p, and for frame='local'
+    the rotation (gb_rotate_to_local) -> [E, 3, *shape]."""
+    on_device = isinstance(x, torch.Tensor)
+    dev = torch.device("cuda", p.device)
+    if on_device and x.device.index != p.device:
+        raise ValueError("coefficients must be a float64 CUDA tensor on device {0}".format(p.device))
+    x = x.contiguous() if on_device else torch.as_tensor(x).to(dev)
+    E, L = x.shape[0], x.shape[-1]
+    full = (E, 3) + tuple(shape)
+    to_host = not (on_device or device_output)
+    if out is not None and to_host:
+        _plan._check_out_host(out, full)
+    if out is not None and not to_host:
+        res = _plan._check_out(out, full, p.device)
+    else:
+        res = torch.empty(full, dtype=torch.float64, device=dev)
+    lib, st = _lib.load(), _plan._stream_handle(p.device)
+    g = torch.empty((E, 3, L + 1, L + 1), dtype=torch.float64, device=dev)
+    _lib.check(lib.gb_gradient_coefficients(ctypes.c_void_p(x.data_ptr()), E, L - 1, ctypes.c_void_p(g.data_ptr()),
+                                            p.device, st))
+    p.synthesis(g.view(3 * E, L + 1, L + 1), out=res.view((3 * E,) + tuple(shape)))
+    if frame == 'local':
+        _lib.check(lib.gb_rotate_to_local(ctypes.c_void_p(res.data_ptr()), ctypes.c_void_p(p.frame.data_ptr()), E,
+                                          int(np.prod(shape)), p.device, st))
+    if not to_host:
+        return res
+    if out is None:
+        return res.cpu().numpy()
+    torch.from_numpy(out).copy_(res)
+    return out
+
+
+def gradient_batch(anm, grid=None, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian', device_output=False, out=None):
+    """Gravitational acceleration grad V of a batch of coefficient sets on a grid, in m/s^2.
+
+    anm: [E, L, L] packed coefficients (numpy array or CUDA float64 tensor).  Returns [E, 3, nlat, nlon] on a regular
+    grid, [E, 3, points] on a grid with longitude / latitude (IrregularGrid), at the geocentric radius of the ellipsoid.
+    frame='cartesian': components (x, y, z) Earth-fixed; frame='local': (east, north, up) of the GEOCENTRIC SPHERICAL
+    frame at each point (up along the geocentric radius, not the ellipsoidal normal).  The gradient of the potential
+    only: no kernel and no centrifugal term.  Host / device behaviour as ``to_grid_batch``: with a CUDA tensor input
+    (or device_output=True) the result is a CUDA tensor, otherwise a numpy array (``out`` of the matching kind).
+
+    Each component is a scalar synthesis at degree N + 1 of linearly transformed coefficients (Cunningham's relation,
+    gb_gradient_coefficients), so the 3E sets run through the same synthesis kernels as ``to_grid_batch``."""
+    x = _gradient_input(anm, frame)
+    grid = GeographicGrid() if grid is None else grid
+    if _plan.is_regular(grid):
+        p = _plan.get_gradient_plan(grid, x.shape[-1] - 1, GM, R)
+        shape = (p.nlat, p.nlon)
+    elif hasattr(grid, "longitude") and hasattr(grid, "latitude"):
+        lon = np.asarray(grid.longitude, dtype=float)
+        lat = np.asarray(grid.latitude, dtype=float)
+        a, f = grid.semimajor_axis, grid.flattening
+        p = _plan.get_gradient_points_plan(utilities.geocentric_radius(lat, a, f), utilities.colatitude(lat, a, f), lon,
+                                           x.shape[-1] - 1, GM, R)
+        shape = (p.npts,)
+    else:
+        raise TypeError("grid must expose parallels/meridians or longitude/latitude")
+    return _gradient(x, p, frame, shape, device_output, out)
+
+
+def gradient_at_positions(anm, positions, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian', device_output=False, out=None):
+    """Gravitational acceleration grad V of a batch of coefficient sets at Earth-fixed Cartesian positions [P, 3] in
+    metres (any radius, e.g. along an orbit) -> [E, 3, P] in m/s^2.  frame, the result's kind and ``out`` as for
+    ``gradient_batch``; the local frame is geocentric spherical at each position (longitude 0 on the polar axis).
+    Non-finite positions and the origin raise ValueError."""
+    x = _gradient_input(anm, frame)
+    r, colat, lon = utilities.cartesian_to_spherical(positions)
+    p = _plan.get_gradient_points_plan(r, colat, lon, x.shape[-1] - 1, GM, R)
+    return _gradient(x, p, frame, (p.npts,), device_output, out)
+
+
 def gridded_rms(temporal_gravityfield, epochs, kernel='ewh', base_grid=None):
     """Temporal RMS of gridded values over ``epochs`` (reference gravityfield.py:1143-1172).
     The reference synthesises epoch by epoch; here all epochs go through one batched GPU

@@ -629,14 +629,7 @@ def get_points_plan(grid, max_degree, kernel='ewh', GM=3.9860044150e+14, R=6.378
     lat = np.asarray(grid.latitude, dtype=float)
     key = ("points", lon.tobytes(), lat.tobytes(), float(grid.semimajor_axis), float(grid.flattening),
            int(max_degree), kernel.lower(), float(GM), float(R), dev)
-    with _cache_lock:
-        plan = _cache.get(key)
-        if plan is None:
-            plan = PointsPlan(lon, lat, grid.semimajor_axis, grid.flattening, max_degree, kernel, GM, R, dev)
-            if len(_cache) >= _MAX_CACHED_PLANS:
-                _cache.pop(next(iter(_cache)))       # destroyed by __del__ once no caller holds it any more
-            _cache[key] = plan
-        return plan
+    return _cached(key, lambda: PointsPlan(lon, lat, grid.semimajor_axis, grid.flattening, max_degree, kernel, GM, R, dev))
 
 
 def is_regular(grid):
@@ -655,14 +648,70 @@ def get_plan(grid, max_degree, kernel='ewh', GM=3.9860044150e+14, R=6.3781363000
     key = (np.asarray(meridians, dtype=float).tobytes(), np.asarray(parallels, dtype=float).tobytes(),
            float(grid.semimajor_axis), float(grid.flattening), int(max_degree), kernel.lower(), float(GM), float(R), dev,
            variant)
+    return _cached(key, lambda: SHPlan(meridians, parallels, grid.semimajor_axis, grid.flattening, max_degree, kernel, GM,
+                                       R, dev))
+
+
+def _cached(key, make):
     with _cache_lock:
         plan = _cache.get(key)
         if plan is None:
-            plan = SHPlan(meridians, parallels, grid.semimajor_axis, grid.flattening, max_degree, kernel, GM, R, dev)
+            plan = make()
             if len(_cache) >= _MAX_CACHED_PLANS:
                 _cache.pop(next(iter(_cache)))       # destroyed by __del__ once no caller holds it any more
             _cache[key] = plan
         return plan
+
+
+def gradient_degree_factors(radius, max_degree, GM, R):
+    """Degree factors kn'[p, n'] = GM/R^2 (R/r_p)^(n'+1), n' = 0..max_degree + 1, of the syntheses that turn the output of
+    gb_gradient_coefficients into the components of grad V; column 0 is zero (degree 0 of those coefficients is)."""
+    kn = np.power((R / np.asarray(radius, dtype=float))[:, None], np.arange(max_degree + 2, dtype=int) + 1) * (GM / R ** 2)
+    kn[:, 0] = 0.0
+    return kn
+
+
+def _frame_table(colat, lon, device):
+    """[4, P] device table (cos theta, sin theta, cos lon, sin lon) that gb_rotate_to_local reads."""
+    table = np.stack((np.cos(colat), np.sin(colat), np.cos(lon), np.sin(lon)))
+    return torch.as_tensor(np.ascontiguousarray(table)).to(torch.device("cuda", device))
+
+
+def get_gradient_plan(grid, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
+    """Cached SHPlan at degree max_degree + 1 for the gradient of degree-max_degree coefficients on a regular grid:
+    the grid's geocentric colatitudes, the degree factors of gradient_degree_factors at the geocentric radius of each
+    parallel, and ``plan.frame`` [4, nlat * nlon], the per-point table of the rotation to (east, north, up).  Its cache
+    key carries a 'gradient' variant: it is never mistaken for a potential plan of the same grid and degree."""
+    dev = _current_device(device)
+    meridians = np.asarray(grid.meridians, dtype=float)
+    parallels = np.asarray(grid.parallels, dtype=float)
+    a, f = float(grid.semimajor_axis), float(grid.flattening)
+    key = (meridians.tobytes(), parallels.tobytes(), a, f, int(max_degree), float(GM), float(R), dev, "gradient")
+
+    def make():
+        kn = gradient_degree_factors(utilities.geocentric_radius(parallels, a, f), int(max_degree), GM, R)
+        plan = SHPlan(meridians, parallels, a, f, int(max_degree) + 1, "gradient", GM, R, dev, degree_factors=kn)
+        nlat, nlon = plan.nlat, plan.nlon
+        plan.frame = _frame_table(np.repeat(plan.colat, nlon), np.tile(meridians, nlat), dev)
+        return plan
+    return _cached(key, make)
+
+
+def get_gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
+    """Cached PointsPlan at degree max_degree + 1 for the gradient at points of geocentric radius / colatitude /
+    longitude (any radius: on the ellipsoid for an IrregularGrid, anywhere for Cartesian positions), with ``plan.frame``
+    [4, P] as for get_gradient_plan."""
+    dev = _current_device(device)
+    radius, colat, lon = (np.ascontiguousarray(v, dtype=float) for v in (radius, colat, lon))
+    key = ("gradient points", radius.tobytes(), colat.tobytes(), lon.tobytes(), int(max_degree), float(GM), float(R), dev)
+
+    def make():
+        kn = gradient_degree_factors(radius, int(max_degree), GM, R)
+        plan = PointsPlan(lon, 0.5 * np.pi - colat, utilities.A_GRS80, utilities.F_GRS80, int(max_degree) + 1, "gradient",
+                          GM, R, dev, degree_factors=kn, colatitude=colat)
+        plan.frame = _frame_table(colat, lon, dev)
+        return plan
+    return _cached(key, make)
 
 
 def clear_plan_cache():

@@ -25,6 +25,23 @@ def colatitude(latitude, a=A_GRS80, f=F_GRS80):
     return np.arccos(nu * (1 - e2) * np.sin(latitude) / geocentric_radius(latitude, a, f))
 
 
+def cartesian_to_spherical(positions):
+    """Earth-fixed Cartesian positions [P, 3] in metres -> geocentric (radius, colatitude, longitude), each [P]:
+    r = |x|, theta = atan2(sqrt(x^2 + y^2), z), lon = atan2(y, x), with lon = 0 on the polar axis.
+    Non-finite positions and the origin (r = 0) raise ValueError."""
+    x = np.asarray(positions, dtype=float)
+    if x.ndim != 2 or x.shape[1] != 3:
+        raise ValueError("positions must have shape [points, 3] (got {0})".format(x.shape))
+    if not np.all(np.isfinite(x)):
+        raise ValueError("positions must be finite")
+    rho = np.sqrt(x[:, 0] ** 2 + x[:, 1] ** 2)
+    r = np.sqrt(x[:, 0] ** 2 + x[:, 1] ** 2 + x[:, 2] ** 2)
+    if np.any(r == 0):
+        raise ValueError("positions must not be the origin (r = 0)")
+    lon = np.where(rho > 0, np.arctan2(x[:, 1], x[:, 0]), 0.0)
+    return r, np.arctan2(rho, x[:, 2]), lon
+
+
 _INDEX_CACHE = {}
 
 

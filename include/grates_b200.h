@@ -53,7 +53,7 @@ typedef struct gb_plan gb_plan;
 
 /* Library version (major*10000 + minor*100 + patch); bumped with every change of this header.  The Python binding
  * refuses a library whose version differs from the one it was written for (grates_b200/_lib.py). */
-#define GB_VERSION 202
+#define GB_VERSION 203
 int gb_version(void);
 
 /* Thread-local description of the last error returned on this thread. */
@@ -304,6 +304,30 @@ int gb_ravel_coefficients(const double* d_anm, int n_sets, int nmax, int nmin, d
                           void* stream);
 int gb_quadratic_forms(const double* d_sigma, int64_t k, const double* d_vec, int n_vec, double* d_out,
                        int device, void* stream);
+
+/*
+ * Gravitational acceleration (gradient of the potential, no centrifugal term) as three scalar syntheses.  The general
+ * form of the zonal gradient of PotentialCoefficients.gravitational_acceleration (gravityfield.py:423-481, restated for
+ * GRS80 normal gravity in kernel.py): each Cartesian component of grad V of a degree-nmax field is a synthesis at degree
+ * nmax + 1 of linearly transformed coefficients, with degree factors GM/R^2 (R/r)^(n'+1) (Cunningham's relation).
+ *   gb_gradient_coefficients   d_anm [n_sets][L][L] packed -> d_out [n_sets][3][L+1][L+1] packed, components (x, y, z)
+ *                              Earth-fixed; with q = (2n+1)/(2n+3), (C_nm, S_nm) contributes
+ *                                Z[n+1][m]   -sqrt((n-m+1)(n+m+1) q) (C, S)
+ *                                X[n+1][m+1] -fp (C, S),  Y[n+1][m+1] (+fp S, -fp C)
+ *                                X[n+1][m-1] +fm (C, S),  Y[n+1][m-1] (+fm S, -fm C)   (m >= 1)
+ *                              fp = sqrt((n+m+1)(n+m+2) q)/2 (x sqrt 2 at m = 0), fm = sqrt((n-m+1)(n-m+2) q)/2
+ *                              (x sqrt 2 at m = 1); sines of order 0 dropped; degree 0 of d_out is zero.  Deterministic
+ *                              (a gather, no atomics).
+ *   gb_rotate_to_local         d_xyz [n_sets][3][n_points] (gx, gy, gz) -> (east, north, up) in place, with
+ *                              d_frame [4][n_points] = (cos theta, sin theta, cos lon, sin lon) of each point:
+ *                                east  = -sin lon gx + cos lon gy
+ *                                north = -cos theta cos lon gx - cos theta sin lon gy + sin theta gz
+ *                                up    =  sin theta cos lon gx + sin theta sin lon gy + cos theta gz
+ *                              theta is the GEOCENTRIC colatitude: the frame is geocentric spherical, not the ellipsoidal
+ *                              normal.  Grid values are the [nlat][nlon] points flattened row by row.
+ */
+int gb_gradient_coefficients(const double* d_anm, int n_sets, int nmax, double* d_out, int device, void* stream);
+int gb_rotate_to_local(double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device, void* stream);
 
 /* Pinned host memory for the *_host entry points. */
 int gb_host_alloc(void** ptr, uint64_t bytes);

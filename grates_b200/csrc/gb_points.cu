@@ -11,10 +11,17 @@
 //                          GEMM (gb_gemm.cuh) with Sigma as the A operand and F' as the B operand, and
 //                          the product with F folded into the epilogue with warp shuffles.
 //                          2 P K^2 flops, nothing assumed about the point geometry.
+//   gb_points_gradient_covariance
+//                          the 3 x 3 covariance of grad V per point, J_p sym(Sigma) J_p' with the Jacobian
+//                          J_p = F'_p T of the gradient (Cunningham's transform T, gb_gradient.cuh, followed by the
+//                          degree-(N+1) synthesis row F'_p of a gradient point set): the same blocked GEMM with the
+//                          three components of 40 points in a 120-column tile, the doubled lower triangle of the
+//                          symmetric part of Sigma, and the three cross products of a point folded in the epilogue.
 #include <vector>
 #include <cmath>
 #include "gb_common.cuh"
 #include "gb_gemm.cuh"
+#include "gb_gradient.cuh"
 
 struct gb_points {
     int device = 0, nmax = 0, L = 0, npts = 0, sm_count = 0;
@@ -452,14 +459,19 @@ extern "C" int gb_points_synthesis_matrix(gb_points* p, int nmin, double* d_out,
 // consecutive entries of the rows of Sigma), zero beyond K' in a and b.  For a symmetric Sigma only its lower triangle is
 // kept, the off-diagonal entries doubled:  x' S x = sum_b S_bb x_b^2 + 2 sum_{a>b} S_ab x_a x_b, so that row tile j only
 // needs k = a >= 128 j.
+enum SigmaTiles { SIGMA_FULL = 0, SIGMA_LOWER = 1, SIGMA_SYMMETRISED_LOWER = 2 };
+// SIGMA_LOWER: Sigma is stated symmetric, below the diagonal 2 Sigma_ab.  SIGMA_SYMMETRISED_LOWER: the same for the
+// symmetric part (Sigma + Sigma') / 2 of any Sigma, Sigma_ab + Sigma_ba below the diagonal; bit-identical to SIGMA_LOWER
+// for an exactly symmetric Sigma.
 __global__ void __launch_bounds__(GB_TM)
-gb_points_sigma_tiles(const double* __restrict__ sigma, double* __restrict__ St, long long Kc, int Kp, int lower) {
+gb_points_sigma_tiles(const double* __restrict__ sigma, double* __restrict__ St, long long Kc, int Kp, int mode) {
     const long long a = blockIdx.x;
     const long long b = (long long)blockIdx.y * GB_TM + threadIdx.x;
     double v = 0.0;
     if (a < Kc && b < Kc) {
         v = sigma[(size_t)a * Kc + b];
-        if (lower) v = (a > b) ? v + v : (a == b ? v : 0.0);
+        if (mode != SIGMA_FULL)
+            v = (a > b) ? v + (mode == SIGMA_LOWER ? v : sigma[(size_t)b * Kc + a]) : (a == b ? v : 0.0);
     }
     St[gb_ab_offset(b, (int)a, Kp)] = v;
 }
@@ -467,7 +479,7 @@ gb_points_sigma_tiles(const double* __restrict__ sigma, double* __restrict__ St,
 extern "C" int gb_points_covariance(gb_points* p, const double* d_sigma, int nmin, double* d_out, int flags,
                                     void* stream) {
     const int take_sqrt = flags & GB_COV_SQRT;
-    const int lower = (flags & GB_COV_SYMMETRIC) ? 1 : 0;
+    const int lower = (flags & GB_COV_SYMMETRIC) ? SIGMA_LOWER : SIGMA_FULL;
     GB_REQUIRE(p != nullptr, "gb_points_covariance: point set is NULL");
     GB_REQUIRE(nmin >= 0 && nmin <= p->nmax, "gb_points_covariance: min_degree=%d outside [0, %d]", nmin, p->nmax);
     GB_REQUIRE(d_sigma && d_out, "gb_points_covariance: NULL device pointer");
@@ -518,6 +530,227 @@ extern "C" int gb_points_covariance(gb_points* p, const double* d_sigma, int nmi
         int rc = gbgemm::launch(sh, PointQuadForm{d_ft, d_part, Kc, Kp, count, nslots}, p->sm_count, st);
         if (rc) return rc;
         gb_points_finish<<<(count + 255) / 256, 256, 0, st>>>(d_part, d_out + p0, nslots, count, take_sqrt ? 1 : 0);
+        GB_LAUNCH_CHECK();
+    }
+    return GB_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// covariance of grad V at the points of a gradient point set (degree N + 1, factors GM/R^2 (R/r)^(n'+1))
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int GP_TP = GB_S2_TN / gbgemm::WN;     // 40 points per 120-column tile, one warp column per component
+
+// Jacobian J_c[p][a] = sum_a' F'_p[a'] T_c[a'][a] of a block of points as GEMM B tiles [point tile][Kp][GB_S2_LDB]: tile
+// column 40 c + j holds component c of point j of the tile; padding rows (a >= K'), padding points and the four pad
+// columns are written as zeros.  fr: the dense degree-(N+1) rows F' of the block, [count][kf] from degree nmin + 1 on.
+// An input (n, m, cs) reaches degree n + 1 through the gather of gb_gradient.cu read backwards (fp term, then fm term):
+//   z  -fz (n+1, m, cs)
+//   x  -fp (n+1, m+1, cs)  + fm (n+1, m-1, cs)            (m >= 1; a sine of order 0 does not exist)
+//   y  cosine: -fp (n+1, m+1, S) - fm (n+1, m-1, S)      sine: +fp (n+1, m+1, C) + fm (n+1, m-1, C)
+__global__ void __launch_bounds__(256)
+gb_points_gradient_design(double* __restrict__ Jt, const double* __restrict__ fr, long long kf, int nmin, long long Kc,
+                          int Kp, int count, long long total) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;      // = ((tile * Kp) + a) * LDB + col
+    if (idx >= total) return;
+    const int col = (int)(idx % GB_S2_LDB);
+    const long long ta = idx / GB_S2_LDB;
+    const int a = (int)(ta % Kp);
+    const int c = col / GP_TP;
+    const int pp = (int)(ta / Kp) * GP_TP + (col - c * GP_TP);
+    double v = 0.0;
+    if (col < GB_S2_TN && a < Kc && pp < count) {
+        const long long ad = a + (long long)nmin * nmin;                          // degree-wise index from degree 0
+        int n = (int)sqrt((double)ad);
+        if ((long long)n * n > ad) --n;
+        if ((long long)(n + 1) * (n + 1) <= ad) ++n;
+        const int j = (int)(ad - (long long)n * n);                               // 0: C_n0, 2m-1: C_nm, 2m: S_nm
+        const int m = (j + 1) >> 1;
+        const int s = (j > 0 && (j & 1) == 0) ? 1 : 0;
+        const double* f = fr + (size_t)pp * kf + ((long long)(n + 1) * (n + 1) - (long long)(nmin + 1) * (nmin + 1));
+        auto at = [&](int mp, int sp) { return f[mp == 0 ? 0 : 2 * mp - 1 + sp]; };    // F' of (n + 1, mp, sp)
+        const double q = gbgrad::grad_q(n);
+        if (c == 2) {
+            v = __dmul_rn(-gbgrad::grad_fz(n, m, q), at(m, s));
+        } else {
+            const double fp = gbgrad::grad_fp(n, m, q);
+            if (c == 0) {
+                v = __dmul_rn(-fp, at(m + 1, s));
+                if (m >= 1 && (s == 0 || m >= 2)) v = __dadd_rn(v, __dmul_rn(gbgrad::grad_fm(n, m, q), at(m - 1, s)));
+            } else if (s == 0) {
+                v = __dmul_rn(-fp, at(m + 1, 1));
+                if (m >= 2) v = __dadd_rn(v, __dmul_rn(-gbgrad::grad_fm(n, m, q), at(m - 1, 1)));
+            } else {
+                v = __dmul_rn(fp, at(m + 1, 0));
+                v = __dadd_rn(v, __dmul_rn(gbgrad::grad_fm(n, m, q), at(m - 1, 0)));
+            }
+        }
+    }
+    Jt[idx] = v;
+}
+
+// Epilogue of the gradient covariance: the GEMM rows are the columns b of S2 (the doubled lower triangle of sym(Sigma)),
+// its columns (component c, point) of a block, so that C[b][(c, p)] = (J_c S2)[p][b].  The warp of component c folds its
+// 32 rows with J_0, J_1 and J_2 of the same points, read back from the Jacobian tiles, one c' and one column pair at a
+// time (the 40 accumulators stay live beside two sums; ten sums per c' spill at 128 registers), and writes part[p][c][c'][slot] = sum_b (J_c S2)[p][b] J_c'[p][b] over its rows;
+// slot = (row tile, warp row), one writer per slot.  gb_points_gradient_finish adds the slots in order.
+struct PointGradientQuadForm {
+    static constexpr bool whole_tile = true;
+    const double* jt;    // Jacobian tiles [point tile][rows][GB_S2_LDB]
+    double* part;        // [count][3][3][nslots]
+    long long K;         // coefficients (rows b >= K are padding)
+    int rows, count, nslots;
+    // the tile's row 0 at the thread's first column of component 0 (the component and the point follow from col_base
+    // after the K loop: nothing else stays live across it)
+    __device__ __forceinline__ const double* prepare(long long, int nt, int col_base) const {
+        return jt + (size_t)nt * rows * GB_S2_LDB + (col_base - nt * GB_S2_TN) % GP_TP;
+    }
+    __device__ __forceinline__ void tile(const double* f, long long row_base, int col_base, double (&acc)[4][5][2]) const {
+        const int nt = col_base / GB_S2_TN;
+        const int c = (col_base - nt * GB_S2_TN) / GP_TP;                 // the warp's component
+        const int pp0 = col_base - nt * GB_S2_TN - c * GP_TP + nt * GP_TP;  // the thread's first point in the block
+        const int slot = (int)(row_base >> 5);
+#pragma unroll
+        for (int c2 = 0; c2 < 3; ++c2) {
+#pragma unroll
+            for (int ni = 0; ni < 5; ++ni) {        // one column pair at a time: two sums live beside the accumulators
+                double s0 = 0.0, s1 = 0.0;
+#pragma unroll
+                for (int mi = 0; mi < 4; ++mi) {
+                    const long long b = row_base + mi * 8;
+                    const double2 jb = b < K ? __ldg(reinterpret_cast<const double2*>(f + (size_t)b * GB_S2_LDB +
+                                                                                       c2 * GP_TP + ni * 8))
+                                             : make_double2(0.0, 0.0);
+                    s0 = mi ? fma(acc[mi][ni][0], jb.x, s0) : acc[mi][ni][0] * jb.x;
+                    s1 = mi ? fma(acc[mi][ni][1], jb.y, s1) : acc[mi][ni][1] * jb.y;
+                }
+#pragma unroll
+                for (int o = 4; o < 32; o <<= 1) {
+                    s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+                    s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+                }
+                const int pp = pp0 + ni * 8;
+                if ((threadIdx.x & 31) < 4) {      // g = 0
+                    if (pp < count) part[((size_t)(pp * 3 + c) * 3 + c2) * nslots + slot] = s0;
+                    if (pp + 1 < count) part[((size_t)((pp + 1) * 3 + c) * 3 + c2) * nslots + slot] = s1;
+                }
+            }
+        }
+    }
+};
+
+// Per point of the block: M[c][c'] = sum of the slots in order (bit-identical from run to run), the symmetric covariance
+// C_cc = M_cc, C_cc' = (M_cc' + M_c'c) / 2, optionally Q C Q' in (east, north, up) (gbgrad::rotate on the columns, then
+// on the rows, then made symmetric again); out [npts][3][3], or with take_sqrt [3][npts] square roots of the diagonal.
+__global__ void __launch_bounds__(256)
+gb_points_gradient_finish(const double* __restrict__ part, const double* __restrict__ frame, double* __restrict__ out,
+                          int nslots, int count, int p0, long long npts, int take_sqrt) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    double M[3][3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+#pragma unroll
+        for (int c2 = 0; c2 < 3; ++c2) {
+            const double* pt = part + ((size_t)(i * 3 + c) * 3 + c2) * nslots;
+            double v = 0.0;
+            for (int s = 0; s < nslots; ++s) v += pt[s];
+            M[c][c2] = v;
+        }
+    double C[3][3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+#pragma unroll
+        for (int c2 = 0; c2 < 3; ++c2) C[c][c2] = c == c2 ? M[c][c] : __dmul_rn(0.5, __dadd_rn(M[c][c2], M[c2][c]));
+    const long long p = p0 + (long long)i;
+    if (frame) {
+        const gbgrad::Frame f{frame[p], frame[npts + p], frame[2 * npts + p], frame[3 * npts + p]};
+#pragma unroll
+        for (int j = 0; j < 3; ++j) gbgrad::rotate(f, C[0][j], C[1][j], C[2][j]);
+#pragma unroll
+        for (int j = 0; j < 3; ++j) gbgrad::rotate(f, C[j][0], C[j][1], C[j][2]);
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+#pragma unroll
+            for (int c2 = c + 1; c2 < 3; ++c2) C[c][c2] = C[c2][c] = __dmul_rn(0.5, __dadd_rn(C[c][c2], C[c2][c]));
+    }
+    if (take_sqrt) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) out[c * npts + p] = sqrt(C[c][c]);
+    } else {
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+#pragma unroll
+            for (int c2 = 0; c2 < 3; ++c2) out[(size_t)p * 9 + 3 * c + c2] = C[c][c2];
+    }
+}
+
+}  // namespace
+
+extern "C" int gb_points_gradient_covariance(gb_points* p, const double* d_sigma, int nmin, const double* d_frame,
+                                             double* d_out, int flags, void* stream) {
+    GB_REQUIRE(p != nullptr, "gb_points_gradient_covariance: point set is NULL");
+    GB_REQUIRE((flags & ~GB_COV_SQRT) == 0, "gb_points_gradient_covariance: flags=%d; only GB_COV_SQRT is accepted",
+               flags);
+    GB_REQUIRE(p->nmax >= 1, "gb_points_gradient_covariance: a gradient point set has degree nmax + 1 >= 1 (got %d)",
+               p->nmax);
+    const int nmax = p->nmax - 1;                                      // degree of the field
+    GB_REQUIRE(nmin >= 0 && nmin <= nmax, "gb_points_gradient_covariance: min_degree=%d outside [0, %d]", nmin, nmax);
+    GB_REQUIRE(d_sigma && d_out, "gb_points_gradient_covariance: NULL device pointer");
+    GB_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const long long Kc = (long long)(nmax + 1) * (nmax + 1) - (long long)nmin * nmin;   // coefficients of the field
+    const int Kp = (int)((Kc + 3) / 4 * 4);
+    const long long kf = (long long)p->L * p->L - (long long)(nmin + 1) * (nmin + 1);     // F' from degree nmin + 1
+    const int n_btiles = (int)((Kc + GB_TM - 1) / GB_TM);
+    const int n_ptiles_all = (p->npts + GP_TP - 1) / GP_TP;
+    // point blocks as for gb_points_covariance: several waves of GEMM tiles, the Jacobian only ever for one block
+    int tiles_per_block = 4 * p->sm_count / n_btiles;
+    if (tiles_per_block < 16) tiles_per_block = 16;
+    if (tiles_per_block > n_ptiles_all) tiles_per_block = n_ptiles_all;
+    const int nslots = n_btiles * gbgemm::WM;
+    const int max_count = tiles_per_block * GP_TP;
+    double *d_st = nullptr, *d_fr = nullptr, *d_jt = nullptr, *d_part = nullptr;
+    gb_retain_pool_memory(p->device);
+    gb_scratch scratch(st);
+    GB_CUDA(scratch.alloc(&d_st, (size_t)n_btiles * Kp * GB_LDA));
+    GB_CUDA(scratch.alloc(&d_fr, (size_t)max_count * kf));
+    GB_CUDA(scratch.alloc(&d_jt, (size_t)tiles_per_block * Kp * GB_S2_LDB));
+    GB_CUDA(scratch.alloc(&d_part, (size_t)max_count * 9 * nslots));
+    gb_points_sigma_tiles<<<dim3((unsigned)Kp, (unsigned)n_btiles), GB_TM, 0, st>>>(d_sigma, d_st, Kc, Kp,
+                                                                                    SIGMA_SYMMETRISED_LOWER);
+    GB_LAUNCH_CHECK();
+    gbgemm::Shape sh;
+    sh.A_t = d_st;
+    sh.a_rows = Kp;
+    sh.a_koff_mul = 0;
+    sh.tiles_per_group = 1;
+    sh.B_t = d_jt;
+    sh.b_rows = Kp;
+    sh.klen = Kp;
+    sh.n_mtiles = n_btiles;
+    sh.mt_kstart_mod = n_btiles;        // row tile j starts its contraction at k = 128 j (the rows above are zeros)
+    sh.mt_kstart_mul = GB_TM;
+    const int L = p->L;
+    const int threads = L >= 1024 ? 1024 : (L + 31) / 32 * 32;
+    for (int t0 = 0; t0 < n_ptiles_all; t0 += tiles_per_block) {
+        const int n_ptiles = (n_ptiles_all - t0 < tiles_per_block) ? (n_ptiles_all - t0) : tiles_per_block;
+        const int p0 = t0 * GP_TP;
+        const int count = (p->npts - p0 < n_ptiles * GP_TP) ? (p->npts - p0) : n_ptiles * GP_TP;
+        gb_points_design_rows<<<count, threads, 0, st>>>(DenseRows{d_fr, kf, (long long)(nmin + 1) * (nmin + 1)},
+                                                         p->d_ct, p->d_kn, p->d_pmm, p->d_cml, p->d_sml, p->d_ra,
+                                                         p->d_rb, p->d_rc, L, nmin + 1, p0 + count, p0);
+        GB_LAUNCH_CHECK();
+        const long long total = (long long)n_ptiles * Kp * GB_S2_LDB;
+        gb_points_gradient_design<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d_jt, d_fr, kf, nmin, Kc, Kp, count,
+                                                                                   total);
+        GB_LAUNCH_CHECK();
+        sh.n_ntiles = n_ptiles;
+        int rc = gbgemm::launch(sh, PointGradientQuadForm{d_jt, d_part, Kc, Kp, count, nslots}, p->sm_count, st);
+        if (rc) return rc;
+        gb_points_gradient_finish<<<(count + 255) / 256, 256, 0, st>>>(d_part, d_frame, d_out, nslots, count, p0,
+                                                                       p->npts, (flags & GB_COV_SQRT) ? 1 : 0);
         GB_LAUNCH_CHECK();
     }
     return GB_OK;

@@ -554,6 +554,67 @@ def gradient_at_positions(anm, positions, GM=GM_DEFAULT, R=R_DEFAULT, frame='car
     return _gradient(x, p, frame, (p.npts,), device_output, out)
 
 
+def _gradient_covariance_input(covariance_matrix, min_degree, max_degree, frame, full):
+    """Checks that need no device: the frame name, full, the degree range and the shape of Sigma."""
+    if frame not in _FRAMES:
+        raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
+    if not isinstance(full, (bool, np.bool_)):
+        raise ValueError("full must be True or False (got {0!r})".format(full))
+    if not 0 <= int(min_degree) <= int(max_degree):
+        raise ValueError("degree range [{0}, {1}] is empty or negative".format(min_degree, max_degree))
+    kp = (int(max_degree) + 1) ** 2 - int(min_degree) ** 2
+    if tuple(np.shape(covariance_matrix)) != (kp, kp):
+        raise ValueError("covariance matrix must have shape [{0}, {0}] for degrees {1}..{2} (got {3})".format(
+            kp, min_degree, max_degree, tuple(np.shape(covariance_matrix))))
+
+
+def _gradient_covariance(covariance_matrix, p, min_degree, frame, full, device_output):
+    from .grid import _device_matrix
+    out = p.gradient_covariance(_device_matrix(covariance_matrix, p.device), int(min_degree), frame, bool(full))
+    return out if device_output else out.cpu().numpy()
+
+
+def gradient_covariance_propagation(covariance_matrix, grid, min_degree, max_degree, GM=GM_DEFAULT, R=R_DEFAULT,
+                                    frame='cartesian', full=False, device_output=False):
+    """Uncertainty of the gravitational acceleration grad V on a grid, given the covariance matrix Sigma [K', K'] of the
+    degree-wise coefficients from min_degree to max_degree (numpy array or CUDA tensor; contracted as its symmetric part
+    (Sigma + Sigma') / 2).  Points at the geocentric radius of the ellipsoid, as ``gradient_batch``; frame as there.
+
+    Returns standard deviations in m/s^2, [3, points] on a grid with longitude / latitude and [3, nlat, nlon] on a
+    regular grid (its points row by row), or with full=True the 3 x 3 covariances in (m/s^2)^2, [points, 3, 3] or
+    [nlat, nlon, 3, 3].  numpy arrays, or CUDA tensors with device_output=True.  Work: 3 P K'^2 flops executed
+    (gb_points_gradient_covariance, the lower triangle of the symmetric part)."""
+    _gradient_covariance_input(covariance_matrix, min_degree, max_degree, frame, full)
+    if _plan.is_regular(grid):
+        parallels = np.asarray(grid.parallels, dtype=float)
+        meridians = np.asarray(grid.meridians, dtype=float)
+        lat, lon = np.repeat(parallels, meridians.size), np.tile(meridians, parallels.size)
+        shape = (parallels.size, meridians.size)
+    elif hasattr(grid, "longitude") and hasattr(grid, "latitude"):
+        lat, lon = np.asarray(grid.latitude, dtype=float), np.asarray(grid.longitude, dtype=float)
+        shape = None
+    else:
+        raise TypeError("grid must expose parallels/meridians or longitude/latitude")
+    a, f = grid.semimajor_axis, grid.flattening
+    p = _plan.get_gradient_points_plan(utilities.geocentric_radius(lat, a, f), utilities.colatitude(lat, a, f), lon,
+                                       int(max_degree), GM, R)
+    out = _gradient_covariance(covariance_matrix, p, min_degree, frame, full, device_output)
+    if shape is None:
+        return out
+    return out.reshape(shape + (3, 3)) if full else out.reshape((3,) + shape)
+
+
+def gradient_covariance_at_positions(covariance_matrix, positions, min_degree, max_degree, GM=GM_DEFAULT, R=R_DEFAULT,
+                                     frame='cartesian', full=False, device_output=False):
+    """``gradient_covariance_propagation`` at Earth-fixed Cartesian positions [P, 3] in metres (any radius, e.g. along an
+    orbit; the local frame as for ``gradient_at_positions``) -> [3, P] standard deviations in m/s^2, or [P, 3, 3]
+    covariances in (m/s^2)^2 with full=True.  Non-finite positions and the origin raise ValueError."""
+    _gradient_covariance_input(covariance_matrix, min_degree, max_degree, frame, full)
+    r, colat, lon = utilities.cartesian_to_spherical(positions)
+    p = _plan.get_gradient_points_plan(r, colat, lon, int(max_degree), GM, R)
+    return _gradient_covariance(covariance_matrix, p, min_degree, frame, full, device_output)
+
+
 def gridded_rms(temporal_gravityfield, epochs, kernel='ewh', base_grid=None):
     """Temporal RMS of gridded values over ``epochs`` (reference gravityfield.py:1143-1172).
     The reference synthesises epoch by epoch; here all epochs go through one batched GPU

@@ -621,6 +621,33 @@ class PointsPlan:
                                                   _stream_handle(self.device)))
         return out
 
+    def gradient_covariance(self, sigma, min_degree, frame='cartesian', full=False):
+        """Covariance of grad V at the points of a gradient point plan (get_gradient_points_plan: degree N + 1 for a
+        degree-N field): sigma CUDA tensor [K', K'], K' = (N + 1)^2 - min_degree^2 in degree-wise order, contracted as
+        its symmetric part (Sigma + Sigma') / 2.  frame 'cartesian' (x, y, z) or 'local' (east, north, up).  Returns a
+        CUDA tensor [npts, 3, 3] of covariances in (m/s^2)^2 with full=True, else [3, npts] standard deviations in m/s^2
+        (gb_points_gradient_covariance)."""
+        if frame not in ('cartesian', 'local'):
+            raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
+        if not hasattr(self, "frame"):
+            raise ValueError("gradient_covariance needs a gradient point plan (get_gradient_points_plan)")
+        nmax = self.max_degree - 1
+        if not 0 <= min_degree <= nmax:
+            raise ValueError("min_degree={0} outside [0, {1}]".format(min_degree, nmax))
+        kp = (nmax + 1) ** 2 - min_degree ** 2
+        if sigma.dim() != 2 or tuple(sigma.shape) != (kp, kp):
+            raise ValueError("covariance matrix must have shape [{0}, {0}] (got {1})".format(kp, tuple(sigma.shape)))
+        if sigma.dtype != torch.float64 or not sigma.is_cuda or sigma.device.index != self.device:
+            raise ValueError("covariance matrix must be a float64 CUDA tensor on device {0}".format(self.device))
+        sigma = sigma.contiguous()
+        shape = (self.npts, 3, 3) if full else (3, self.npts)
+        out = torch.empty(shape, dtype=torch.float64, device=sigma.device)
+        fr = ctypes.c_void_p(self.frame.data_ptr()) if frame == 'local' else None
+        _lib.check(self._lib.gb_points_gradient_covariance(self._handle, ctypes.c_void_p(sigma.data_ptr()),
+                                                           int(min_degree), fr, ctypes.c_void_p(out.data_ptr()),
+                                                           0 if full else 1, _stream_handle(self.device)))   # GB_COV_SQRT
+        return out
+
 
 def get_points_plan(grid, max_degree, kernel='ewh', GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
     """Cached PointsPlan for a grid object exposing .longitude/.latitude/.semimajor_axis/.flattening."""

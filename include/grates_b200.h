@@ -53,7 +53,7 @@ typedef struct gb_plan gb_plan;
 
 /* Library version (major*10000 + minor*100 + patch); bumped with every change of this header.  The Python binding
  * refuses a library whose version differs from the one it was written for (grates_b200/_lib.py). */
-#define GB_VERSION 203
+#define GB_VERSION 204
 int gb_version(void);
 
 /* Thread-local description of the last error returned on this thread. */
@@ -276,6 +276,16 @@ int gb_points_adjoint(gb_points* points, const double* d_values, int n_epochs, d
 /* Dense synthesis operator of the point set: d_out [npts][K'], K' = (nmax+1)^2 - nmin^2, degree-wise order
  * (Grid.synthesis_matrix, grid.py:412-443, with IrregularGrid.synthesis_matrix_per_order, grid.py:957-991). */
 int gb_points_synthesis_matrix(gb_points* points, int nmin, double* d_out, void* stream);
+/* Covariance of grad V at the points of a GRADIENT point set (degree nmax + 1, factors GM/R^2 (R/r)^(n'+1)):
+ *   d_sigma [K'][K'] degree-wise from nmin, K' = (nmax + 1)^2 - nmin^2 of the degree-nmax field (contracted as (S + S')/2)
+ *   d_frame [4][npts] (cos theta, sin theta, cos lon, sin lon) for (east, north, up), or NULL for Earth-fixed (x, y, z)
+ *   d_out   [npts][3][3] covariances, or [3][npts] standard deviations with GB_COV_SQRT; other flags are refused
+ * C_p = J_p sym(Sigma) J_p' with the Jacobian J_p = F'_p T (T: the transform of gb_gradient_coefficients, F'_p: the
+ * point's degree-(nmax+1) synthesis row), on the DMMA GEMM of gb_points_covariance with the doubled lower triangle of
+ * sym(Sigma) (the entries Sigma_ab + Sigma_ba below the diagonal): 3 npts K'^2 flops executed.  In the local frame the
+ * result is Q C Q' with the rotation of gb_rotate_to_local.  Bit-reproducible from run to run. */
+int gb_points_gradient_covariance(gb_points* points, const double* d_sigma, int nmin, const double* d_frame,
+                                  double* d_out, int flags, void* stream);
 
 /*
  * Consumers of gridded epoch batches that keep the grids on the device.

@@ -1,6 +1,7 @@
 // Persistent FP64 tensor-core GEMM building block (sm_100a).  Users: synthesis stage 2 (direct path), both analysis
 // stages (longitude and latitude), the dense filter, the covariance longitude form of grids without four-fold symmetric
-// meridians, and at arbitrary points the synthesis, the adjoint and the covariance diag(F Sigma F').
+// meridians, and at arbitrary points the synthesis, the adjoint, the covariance diag(F Sigma F') and the normal
+// equations J'WJ of the acceleration (upper_only: the tiles of the upper triangle only).
 //
 //   C[row, col] = sum_k A[k, row] * B[k, col]
 //
@@ -56,7 +57,14 @@ struct Shape {
                                         // (operand rows below are known zeros: triangular A blocks)
     const int* mt_bgroup = nullptr;     // optional: row tile mt multiplies B tile mt_bgroup[mt] * n_ntiles + nt
                                         // (block-diagonal batches: the analysis latitude stage, one group per order)
+    bool upper_only = false;            // optional: tiles whose columns all lie below their first row (col < row
+                                        // everywhere) are skipped -- the upper triangle of a symmetric product
 };
+
+// the tile (mt, nt) of a column tile width tn holds no entry with col >= row
+__host__ __device__ __forceinline__ bool below_diagonal(const Shape& sh, int mt, int nt, int tn) {
+    return sh.upper_only && (long long)(nt + 1) * tn <= (long long)mt * TM;
+}
 
 template <class E, class = void>
 struct wants_whole_tile { static constexpr bool value = false; };
@@ -92,6 +100,7 @@ __global__ void __launch_bounds__(THREADS, 1) kernel(Shape sh, Epilogue epi) {
         if (lane == 0) {
             for (; mt < sh.n_mtiles; mt += step_m, nt += step_n) {
                 if (nt >= sh.n_ntiles) { nt -= sh.n_ntiles; ++mt; if (mt >= sh.n_mtiles) break; }
+                if (below_diagonal(sh, mt, nt, TN)) continue;
                 const int a_koff = (nt / sh.tiles_per_group) * sh.a_koff_mul;
                 const int kstart = sh.mt_kstart_mod ? (mt % sh.mt_kstart_mod) * sh.mt_kstart_mul : 0;
                 for (int k0 = kstart; k0 < sh.klen; k0 += KC) {
@@ -116,6 +125,7 @@ __global__ void __launch_bounds__(THREADS, 1) kernel(Shape sh, Epilogue epi) {
         const int q = lane & 3;
         for (; mt < sh.n_mtiles; mt += step_m, nt += step_n) {
             if (nt >= sh.n_ntiles) { nt -= sh.n_ntiles; ++mt; if (mt >= sh.n_mtiles) break; }
+            if (below_diagonal(sh, mt, nt, TN)) continue;
             double acc[4][NI][2];
 #pragma unroll
             for (int mi = 0; mi < 4; ++mi)

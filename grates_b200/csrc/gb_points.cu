@@ -17,6 +17,10 @@
 //                          degree-(N+1) synthesis row F'_p of a gradient point set): the same blocked GEMM with the
 //                          three components of 40 points in a 120-column tile, the doubled lower triangle of the
 //                          symmetric part of Sigma, and the three cross products of a point folded in the epilogue.
+//   gb_points_gradient_normals
+//                          the normal equations sum_p J~_p' W_p J~_p of acceleration observations (J~_p = Q_p J_p): the
+//                          weighted, rotated Jacobian rows as both GEMM operands, contracted over observations on the
+//                          tiles of the upper triangle only, added into N and mirrored.
 #include <vector>
 #include <cmath>
 #include "gb_common.cuh"
@@ -545,10 +549,7 @@ constexpr int GP_TP = GB_S2_TN / gbgemm::WN;     // 40 points per 120-column til
 // Jacobian J_c[p][a] = sum_a' F'_p[a'] T_c[a'][a] of a block of points as GEMM B tiles [point tile][Kp][GB_S2_LDB]: tile
 // column 40 c + j holds component c of point j of the tile; padding rows (a >= K'), padding points and the four pad
 // columns are written as zeros.  fr: the dense degree-(N+1) rows F' of the block, [count][kf] from degree nmin + 1 on.
-// An input (n, m, cs) reaches degree n + 1 through the gather of gb_gradient.cu read backwards (fp term, then fm term):
-//   z  -fz (n+1, m, cs)
-//   x  -fp (n+1, m+1, cs)  + fm (n+1, m-1, cs)            (m >= 1; a sine of order 0 does not exist)
-//   y  cosine: -fp (n+1, m+1, S) - fm (n+1, m-1, S)      sine: +fp (n+1, m+1, C) + fm (n+1, m-1, C)
+// An input (n, m, cs) reaches degree n + 1 through the gather of gb_gradient.cu read backwards (gbgrad::grad_terms).
 __global__ void __launch_bounds__(256)
 gb_points_gradient_design(double* __restrict__ Jt, const double* __restrict__ fr, long long kf, int nmin, long long Kc,
                           int Kp, int count, long long total) {
@@ -570,22 +571,7 @@ gb_points_gradient_design(double* __restrict__ Jt, const double* __restrict__ fr
         const int s = (j > 0 && (j & 1) == 0) ? 1 : 0;
         const double* f = fr + (size_t)pp * kf + ((long long)(n + 1) * (n + 1) - (long long)(nmin + 1) * (nmin + 1));
         auto at = [&](int mp, int sp) { return f[mp == 0 ? 0 : 2 * mp - 1 + sp]; };    // F' of (n + 1, mp, sp)
-        const double q = gbgrad::grad_q(n);
-        if (c == 2) {
-            v = __dmul_rn(-gbgrad::grad_fz(n, m, q), at(m, s));
-        } else {
-            const double fp = gbgrad::grad_fp(n, m, q);
-            if (c == 0) {
-                v = __dmul_rn(-fp, at(m + 1, s));
-                if (m >= 1 && (s == 0 || m >= 2)) v = __dadd_rn(v, __dmul_rn(gbgrad::grad_fm(n, m, q), at(m - 1, s)));
-            } else if (s == 0) {
-                v = __dmul_rn(-fp, at(m + 1, 1));
-                if (m >= 2) v = __dadd_rn(v, __dmul_rn(-gbgrad::grad_fm(n, m, q), at(m - 1, 1)));
-            } else {
-                v = __dmul_rn(fp, at(m + 1, 0));
-                v = __dadd_rn(v, __dmul_rn(gbgrad::grad_fm(n, m, q), at(m - 1, 0)));
-            }
-        }
+        v = gbgrad::apply(gbgrad::grad_terms(c, n, m, s, gbgrad::grad_q(n)), at);
     }
     Jt[idx] = v;
 }
@@ -753,5 +739,152 @@ extern "C" int gb_points_gradient_covariance(gb_points* p, const double* d_sigma
                                                                        p->npts, (flags & GB_COV_SQRT) ? 1 : 0);
         GB_LAUNCH_CHECK();
     }
+    return GB_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// normal equations of acceleration observations at the points of a gradient point set: N += J~' W J~ (upper triangle,
+// then mirrored), J~_p = Q_p J_p the rotated Jacobian rows of gb_points_gradient_covariance
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+// The rows sqrt(w_pc) J~_p[c] of a block of points, observation o = 3 pp + c, straight into the two GEMM operands: A
+// tiles [coefficient tile of 128][o][GB_LDA] and B tiles [coefficient tile of 120][o][GB_S2_LDB] (k = observation, like
+// the point adjoint).  Thread = (coefficient a, point pp) with a fastest, so the stores of both layouts coalesce; the
+// three Cartesian entries of the point come from the same gbgrad::grad_terms as gb_points_gradient_design, then
+// gbgrad::rotate for the local frame, then the weights.  Coefficients a >= K' (up to am / bm) and observation rows
+// 3 count .. rows - 1 are written as zeros; the pad columns of the tiles are never read by the GEMM.
+__global__ void __launch_bounds__(256)
+gb_points_gradient_normal_rows(double* __restrict__ At, double* __restrict__ Bt, const double* __restrict__ fr, long long kf,
+                               int nmin, long long Kc, int am, int bm, int rows, int count,
+                               const double* __restrict__ weights, const double* __restrict__ frame, long long npts, int p0) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x;
+    const int pp = blockIdx.y;
+    if (a >= am && a >= bm) return;
+    double v[3] = {0.0, 0.0, 0.0};
+    if (a < Kc && pp < count) {
+        const long long ad = a + (long long)nmin * nmin;                          // degree-wise index from degree 0
+        int n = (int)sqrt((double)ad);
+        if ((long long)n * n > ad) --n;
+        if ((long long)(n + 1) * (n + 1) <= ad) ++n;
+        const int j = (int)(ad - (long long)n * n);                               // 0: C_n0, 2m-1: C_nm, 2m: S_nm
+        const int m = (j + 1) >> 1;
+        const int s = (j > 0 && (j & 1) == 0) ? 1 : 0;
+        const double* f = fr + (size_t)pp * kf + ((long long)(n + 1) * (n + 1) - (long long)(nmin + 1) * (nmin + 1));
+        auto at = [&](int mp, int sp) { return f[mp == 0 ? 0 : 2 * mp - 1 + sp]; };    // F' of (n + 1, mp, sp)
+        const double q = gbgrad::grad_q(n);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) v[c] = gbgrad::apply(gbgrad::grad_terms(c, n, m, s, q), at);
+        const long long p = p0 + (long long)pp;
+        if (frame) {
+            const gbgrad::Frame fq{frame[p], frame[npts + p], frame[2 * npts + p], frame[3 * npts + p]};
+            gbgrad::rotate(fq, v[0], v[1], v[2]);
+        }
+        if (weights) {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) v[c] = __dmul_rn(__dsqrt_rn(weights[c * npts + p]), v[c]);
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const int o = 3 * pp + c;
+        if (o >= rows) break;
+        if (a < am) At[gb_ab_offset(a, o, rows)] = v[c];
+        if (a < bm) Bt[((size_t)(a / GB_S2_TN) * rows + o) * GB_S2_LDB + a % GB_S2_TN] = v[c];
+    }
+}
+
+// Epilogue of the normals: C[a][b] = sum_o J~[o][a] J~[o][b] over the block's observations, added to N[a][b] for b >= a
+// (upper triangle).  One thread per entry per launch and the launches in stream order: bit-reproducible.
+struct NormalsAddUpper {
+    double* out;
+    long long K;
+    __device__ __forceinline__ void operator()(long long row, int col, double v0, double v1) const {
+        if (row >= K) return;
+        double* o = out + (size_t)row * K + col;
+        if (col >= row && col < K) *o += v0;
+        if (col + 1 >= row && col + 1 < K) o[1] += v1;
+    }
+};
+
+// N[r][c] = N[c][r] for r > c, through 32 x 32 tiles in shared memory (both accesses coalesce).  The block of the lower
+// tile (bi, bj), bi >= bj, reads the upper tile (bj, bi), which no block writes.
+__global__ void __launch_bounds__(256)
+gb_mirror_upper(double* __restrict__ N, long long K) {
+    __shared__ double t[32][33];
+    const int bi = blockIdx.y, bj = blockIdx.x;
+    if (bi < bj) return;
+    for (int y = threadIdx.y; y < 32; y += 8) {
+        const long long r = (long long)bj * 32 + y, c = (long long)bi * 32 + threadIdx.x;
+        if (r < K && c < K) t[y][threadIdx.x] = N[(size_t)r * K + c];
+    }
+    __syncthreads();
+    for (int y = threadIdx.y; y < 32; y += 8) {
+        const long long r = (long long)bi * 32 + y, c = (long long)bj * 32 + threadIdx.x;
+        if (r < K && c < K && r > c) N[(size_t)r * K + c] = t[threadIdx.x][y];
+    }
+}
+
+}  // namespace
+
+extern "C" int gb_points_gradient_normals(gb_points* p, int nmin, const double* d_weights, const double* d_frame,
+                                          double* d_normals, void* stream) {
+    GB_REQUIRE(p != nullptr, "gb_points_gradient_normals: point set is NULL");
+    GB_REQUIRE(p->nmax >= 1, "gb_points_gradient_normals: a gradient point set has degree nmax + 1 >= 1 (got %d)",
+               p->nmax);
+    const int nmax = p->nmax - 1;                                      // degree of the field
+    GB_REQUIRE(nmin >= 0 && nmin <= nmax, "gb_points_gradient_normals: min_degree=%d outside [0, %d]", nmin, nmax);
+    GB_REQUIRE(d_normals != nullptr, "gb_points_gradient_normals: NULL device pointer");
+    GB_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const long long Kc = (long long)(nmax + 1) * (nmax + 1) - (long long)nmin * nmin;   // coefficients of the field
+    const long long kf = (long long)p->L * p->L - (long long)(nmin + 1) * (nmin + 1);     // F' from degree nmin + 1
+    const int n_mtiles = (int)((Kc + GB_TM - 1) / GB_TM);
+    const int n_ntiles = (int)((Kc + GB_S2_TN - 1) / GB_S2_TN);
+    const int am = n_mtiles * GB_TM, bm = n_ntiles * GB_S2_TN;
+    // points per block: an A operand of about 512 MB (the B operand is as large), a multiple of 4 points so that the 3 pb
+    // observation rows of a full block are whole k4 steps
+    long long pb = (512LL << 20) / ((long long)n_mtiles * GB_LDA * sizeof(double)) / 3;
+    pb = pb / 4 * 4;
+    if (pb < 4) pb = 4;
+    if (pb > 16384) pb = 16384;
+    if (pb > (p->npts + 3) / 4 * 4) pb = (p->npts + 3) / 4 * 4;
+    const int max_rows = (int)(3 * pb);
+    double *d_at = nullptr, *d_bt = nullptr, *d_fr = nullptr;
+    gb_retain_pool_memory(p->device);
+    gb_scratch scratch(st);
+    GB_CUDA(scratch.alloc(&d_at, (size_t)n_mtiles * max_rows * GB_LDA));
+    GB_CUDA(scratch.alloc(&d_bt, (size_t)n_ntiles * max_rows * GB_S2_LDB));
+    GB_CUDA(scratch.alloc(&d_fr, (size_t)pb * kf));
+    gbgemm::Shape sh;
+    sh.A_t = d_at;
+    sh.a_koff_mul = 0;
+    sh.tiles_per_group = 1;
+    sh.B_t = d_bt;
+    sh.n_mtiles = n_mtiles;
+    sh.n_ntiles = n_ntiles;
+    sh.upper_only = true;                // N is symmetric: the tiles below the diagonal are never contracted
+    const int L = p->L;
+    const int threads = L >= 1024 ? 1024 : (L + 31) / 32 * 32;
+    for (int p0 = 0; p0 < p->npts; p0 += (int)pb) {
+        const int count = (p->npts - p0 < pb) ? (p->npts - p0) : (int)pb;
+        const int rows = (3 * count + 3) / 4 * 4;
+        gb_points_design_rows<<<count, threads, 0, st>>>(DenseRows{d_fr, kf, (long long)(nmin + 1) * (nmin + 1)},
+                                                         p->d_ct, p->d_kn, p->d_pmm, p->d_cml, p->d_sml, p->d_ra,
+                                                         p->d_rb, p->d_rc, L, nmin + 1, p0 + count, p0);
+        GB_LAUNCH_CHECK();
+        dim3 grid((unsigned)(((am > bm ? am : bm) + 255) / 256), (unsigned)((rows + 2) / 3));
+        gb_points_gradient_normal_rows<<<grid, 256, 0, st>>>(d_at, d_bt, d_fr, kf, nmin, Kc, am, bm, rows, count,
+                                                             d_weights, d_frame, p->npts, p0);
+        GB_LAUNCH_CHECK();
+        sh.a_rows = rows;
+        sh.b_rows = rows;
+        sh.klen = rows;
+        int rc = gbgemm::launch(sh, NormalsAddUpper{d_normals, Kc}, p->sm_count, st);
+        if (rc) return rc;
+    }
+    const unsigned nt32 = (unsigned)((Kc + 31) / 32);
+    gb_mirror_upper<<<dim3(nt32, nt32), dim3(32, 8), 0, st>>>(d_normals, Kc);
+    GB_LAUNCH_CHECK();
     return GB_OK;
 }

@@ -615,6 +615,126 @@ def gradient_covariance_at_positions(covariance_matrix, positions, min_degree, m
     return _gradient_covariance(covariance_matrix, p, min_degree, frame, full, device_output)
 
 
+def _host_or_cuda(x, name):
+    """numpy float64 array, or the tensor itself when it is a float64 CUDA tensor."""
+    if isinstance(x, torch.Tensor):
+        if x.dtype != torch.float64 or not x.is_cuda:
+            raise ValueError("{0} must be a float64 CUDA tensor".format(name))
+        return x
+    return np.asarray(x, dtype=float)
+
+
+def gradient_adjoint_at_positions(values, positions, max_degree, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian',
+                                  device_output=False):
+    """Transpose of ``gradient_at_positions``: values [E, 3, P] in m/s^2 at Earth-fixed Cartesian positions [P, 3] in
+    metres, components in ``frame`` -> packed coefficients [E, L, L], L = max_degree + 1, with
+    <gradient_at_positions(X), Y> = <X, gradient_adjoint_at_positions(Y)>: the operator J' of an iterative
+    least-squares solver.  With a CUDA tensor input (or device_output=True) the result is a CUDA tensor, otherwise a
+    numpy array.  Non-finite positions and the origin raise ValueError."""
+    if frame not in _FRAMES:
+        raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
+    if int(max_degree) < 0:
+        raise ValueError("max_degree must be >= 0 (got {0})".format(max_degree))
+    v = _host_or_cuda(values, "values")
+    r, colat, lon = utilities.cartesian_to_spherical(positions)
+    if v.ndim != 3 or v.shape[1] != 3 or v.shape[2] != r.size:
+        raise ValueError("values must have shape [sets, 3, {0}] (got {1})".format(r.size, tuple(v.shape)))
+    p = _plan.get_gradient_points_plan(r, colat, lon, int(max_degree), GM, R)
+    on_device = isinstance(v, torch.Tensor)
+    if on_device and v.device.index != p.device:
+        raise ValueError("values must be a float64 CUDA tensor on device {0}".format(p.device))
+    x = v if on_device else torch.as_tensor(np.ascontiguousarray(v)).to(torch.device("cuda", p.device))
+    out = p.gradient_adjoint(x, frame)
+    return out if (on_device or device_output) else out.cpu().numpy()
+
+
+def _positions_per_chunk(max_degree):
+    """Positions whose point-plan tables (four [P, N + 2] tables) take about 1 GB."""
+    return max(1, (1 << 30) // (8 * 4 * (int(max_degree) + 2)))
+
+
+def gradient_normal_equations_at_positions(observations, positions, min_degree, max_degree, GM=GM_DEFAULT, R=R_DEFAULT,
+                                           frame='cartesian', weights=None, block_size=2048, positions_per_chunk=None):
+    """Least-squares normal equations of gravitational-acceleration observations at Earth-fixed Cartesian positions (the
+    acceleration approach of orbit-based gravity recovery), for the degree-wise coefficients from min_degree to
+    max_degree, K' = (max_degree + 1)^2 - min_degree^2 unknowns.
+
+    observations: [E, 3, P] or [3, P] in m/s^2 (numpy or CUDA float64), E sets on the same positions sharing one normal
+    matrix; components in ``frame`` ('cartesian' (x, y, z), or 'local' (east, north, up) as in ``gradient_at_positions``).
+    positions: [P, 3] in metres.  weights: [3, P] positive weights (inverse variances) per observation, or None for 1.
+    With J~ the design matrix of grad V (the Jacobian of ``gradient_at_positions`` in ``frame``) and W = diag(weights):
+
+      matrix                  N = J~' W J~ as a device ``lstsq.BlockMatrix`` with blocks of block_size
+      right_hand_side         n = J~' W l, CUDA tensor [K', E]
+      observation_square_sum  l' W l per set, numpy [E]
+      observation_count       3 P
+
+    returned as an ``lstsq.NormalEquations`` (``solve()``, ``compute_covariance()``).  Everything is formed on the device
+    (gb_points_gradient_normals, ``gradient_adjoint_at_positions``); long position arrays are cut into chunks of
+    positions_per_chunk (None: the positions whose tables take about 1 GB) with point plans of their own, closed after
+    use.  Work: about 3 P K'^2 flops on the FP64 tensor cores (the upper triangle of N)."""
+    from .lstsq import BlockMatrix, NormalEquations
+    if frame not in _FRAMES:
+        raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
+    nmin, nmax = int(min_degree), int(max_degree)
+    if not 0 <= nmin <= nmax:
+        raise ValueError("degree range [{0}, {1}] is empty or negative".format(min_degree, max_degree))
+    if int(block_size) < 1:
+        raise ValueError("block_size must be positive (got {0})".format(block_size))
+    if positions_per_chunk is not None and int(positions_per_chunk) < 1:
+        raise ValueError("positions_per_chunk must be positive (got {0})".format(positions_per_chunk))
+    obs = _host_or_cuda(observations, "observations")
+    w = None if weights is None else _host_or_cuda(weights, "weights")
+    r, colat, lon = utilities.cartesian_to_spherical(positions)
+    P = r.size
+    single = obs.ndim == 2
+    if single:
+        obs = obs[None]
+    if obs.ndim != 3 or obs.shape[1] != 3 or obs.shape[2] != P or obs.shape[0] < 1:
+        raise ValueError("observations must have shape [sets, 3, {0}] or [3, {0}] (got {1})".format(
+            P, tuple(np.shape(observations))))
+    if w is not None:
+        if tuple(w.shape) != (3, P):
+            raise ValueError("weights must have shape [3, {0}] (got {1})".format(P, tuple(w.shape)))
+        ok = bool(torch.isfinite(w).all() and (w > 0).all()) if isinstance(w, torch.Tensor) else \
+            bool(np.all(np.isfinite(w)) and np.all(w > 0))
+        if not ok:
+            raise ValueError("weights must be finite and positive")
+    dev = obs.device.index if isinstance(obs, torch.Tensor) else _plan._current_device(None)
+    tdev = torch.device("cuda", dev)
+
+    def on_device(x, p0, p1):
+        part = x[..., p0:p1]
+        if isinstance(part, torch.Tensor):
+            return part.to(tdev).contiguous()
+        return torch.as_tensor(np.ascontiguousarray(part)).to(tdev)
+
+    E = obs.shape[0]
+    kp = (nmax + 1) ** 2 - nmin ** 2
+    normals = torch.zeros((kp, kp), dtype=torch.float64, device=tdev)
+    anm = torch.zeros((E, nmax + 1, nmax + 1), dtype=torch.float64, device=tdev)
+    lpl = torch.zeros(E, dtype=torch.float64, device=tdev)
+    chunk = _positions_per_chunk(nmax) if positions_per_chunk is None else int(positions_per_chunk)
+    for p0 in range(0, P, chunk):
+        p1 = min(P, p0 + chunk)
+        l = on_device(obs, p0, p1)
+        wc = None if w is None else on_device(w, p0, p1)
+        wl = l if wc is None else l * wc
+        lpl += (wl * l).sum(dim=(1, 2))
+        plan = _plan.gradient_points_plan(r[p0:p1], colat[p0:p1], lon[p0:p1], nmax, GM, R, dev)
+        try:
+            plan.gradient_normals(normals, nmin, frame, wc)
+            anm += plan.gradient_adjoint(wl, frame)
+        finally:
+            plan.close()
+    rhs = ravel_batch(anm, nmin).T.contiguous()
+    del anm
+    row_index, column_index = BlockMatrix.compute_block_index((kp, kp), int(block_size))
+    matrix = BlockMatrix.from_array(normals, row_index, column_index)
+    del normals
+    return NormalEquations(matrix, rhs, lpl.cpu().numpy(), 3 * P)
+
+
 def gridded_rms(temporal_gravityfield, epochs, kernel='ewh', base_grid=None):
     """Temporal RMS of gridded values over ``epochs`` (reference gravityfield.py:1143-1172).
     The reference synthesises epoch by epoch; here all epochs go through one batched GPU

@@ -648,6 +648,64 @@ class PointsPlan:
                                                            0 if full else 1, _stream_handle(self.device)))   # GB_COV_SQRT
         return out
 
+    def _gradient_field_degree(self, frame, min_degree, name):
+        if frame not in ('cartesian', 'local'):
+            raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
+        if not hasattr(self, "frame"):
+            raise ValueError("{0} needs a gradient point plan (get_gradient_points_plan)".format(name))
+        nmax = self.max_degree - 1
+        if not 0 <= min_degree <= nmax:
+            raise ValueError("min_degree={0} outside [0, {1}]".format(min_degree, nmax))
+        return nmax
+
+    def gradient_normals(self, normals, min_degree, frame='cartesian', weights=None):
+        """Adds the normal equations sum_p J~_p' W_p J~_p of acceleration observations at the points of a gradient point
+        plan to ``normals``, a CUDA float64 tensor [K', K'] (K' = (N + 1)^2 - min_degree^2, degree-wise; zeroed by the
+        caller for a fresh matrix), and returns it with both triangles holding the sum.  J~_p: the Jacobian of grad V in
+        ``frame`` ('cartesian' or 'local'); weights: CUDA float64 tensor [3, npts] of positive weights (inverse variances)
+        or None for 1 (gb_points_gradient_normals)."""
+        nmax = self._gradient_field_degree(frame, min_degree, "gradient_normals")
+        kp = (nmax + 1) ** 2 - min_degree ** 2
+        if normals.dim() != 2 or tuple(normals.shape) != (kp, kp) or not normals.is_contiguous():
+            raise ValueError("normal matrix must be a contiguous tensor of shape [{0}, {0}] (got {1})".format(
+                kp, tuple(normals.shape)))
+        if normals.dtype != torch.float64 or not normals.is_cuda or normals.device.index != self.device:
+            raise ValueError("normal matrix must be a float64 CUDA tensor on device {0}".format(self.device))
+        w = None
+        if weights is not None:
+            if tuple(weights.shape) != (3, self.npts):
+                raise ValueError("weights must have shape [3, {0}] (got {1})".format(self.npts, tuple(weights.shape)))
+            if weights.dtype != torch.float64 or not weights.is_cuda or weights.device.index != self.device:
+                raise ValueError("weights must be a float64 CUDA tensor on device {0}".format(self.device))
+            weights = weights.contiguous()
+            w = ctypes.c_void_p(weights.data_ptr())
+        fr = ctypes.c_void_p(self.frame.data_ptr()) if frame == 'local' else None
+        _lib.check(self._lib.gb_points_gradient_normals(self._handle, int(min_degree), w, fr,
+                                                        ctypes.c_void_p(normals.data_ptr()), _stream_handle(self.device)))
+        return normals
+
+    def gradient_adjoint(self, values, frame='cartesian'):
+        """Transpose of the acceleration at the points of a gradient point plan: values CUDA float64 [E, 3, npts] in
+        ``frame`` -> CUDA tensor [E, N + 1, N + 1] packed, sum_p J_p' Q_p' v_p: Q' for 'local' (gb_rotate_from_local), the
+        adjoint synthesis of the 3E component sets (``adjoint``) and T' (gb_gradient_coefficients_adjoint)."""
+        nmax = self._gradient_field_degree(frame, 0, "gradient_adjoint")
+        if values.dim() != 3 or values.shape[1] != 3 or values.shape[2] != self.npts:
+            raise ValueError("values must have shape [sets, 3, {0}] (got {1})".format(self.npts, tuple(values.shape)))
+        if values.dtype != torch.float64 or not values.is_cuda or values.device.index != self.device:
+            raise ValueError("values must be a float64 CUDA tensor on device {0}".format(self.device))
+        E = values.shape[0]
+        st = _stream_handle(self.device)
+        if frame == 'local':
+            values = values.clone(memory_format=torch.contiguous_format)
+            _lib.check(self._lib.gb_rotate_from_local(ctypes.c_void_p(values.data_ptr()),
+                                                      ctypes.c_void_p(self.frame.data_ptr()), E, self.npts, self.device,
+                                                      st))
+        g = self.adjoint(values.contiguous().view(3 * E, self.npts))
+        out = torch.empty((E, nmax + 1, nmax + 1), dtype=torch.float64, device=values.device)
+        _lib.check(self._lib.gb_gradient_coefficients_adjoint(ctypes.c_void_p(g.data_ptr()), E, nmax,
+                                                              ctypes.c_void_p(out.data_ptr()), self.device, st))
+        return out
+
 
 def get_points_plan(grid, max_degree, kernel='ewh', GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
     """Cached PointsPlan for a grid object exposing .longitude/.latitude/.semimajor_axis/.flattening."""
@@ -731,14 +789,18 @@ def get_gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14
     dev = _current_device(device)
     radius, colat, lon = (np.ascontiguousarray(v, dtype=float) for v in (radius, colat, lon))
     key = ("gradient points", radius.tobytes(), colat.tobytes(), lon.tobytes(), int(max_degree), float(GM), float(R), dev)
+    return _cached(key, lambda: gradient_points_plan(radius, colat, lon, max_degree, GM, R, dev))
 
-    def make():
-        kn = gradient_degree_factors(radius, int(max_degree), GM, R)
-        plan = PointsPlan(lon, 0.5 * np.pi - colat, utilities.A_GRS80, utilities.F_GRS80, int(max_degree) + 1, "gradient",
-                          GM, R, dev, degree_factors=kn, colatitude=colat)
-        plan.frame = _frame_table(colat, lon, dev)
-        return plan
-    return _cached(key, make)
+
+def gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
+    """The PointsPlan of get_gradient_points_plan, not cached: the caller closes it (long position arrays in chunks)."""
+    dev = _current_device(device)
+    radius, colat, lon = (np.ascontiguousarray(v, dtype=float) for v in (radius, colat, lon))
+    kn = gradient_degree_factors(radius, int(max_degree), GM, R)
+    plan = PointsPlan(lon, 0.5 * np.pi - colat, utilities.A_GRS80, utilities.F_GRS80, int(max_degree) + 1, "gradient",
+                      GM, R, dev, degree_factors=kn, colatitude=colat)
+    plan.frame = _frame_table(colat, lon, dev)
+    return plan
 
 
 def clear_plan_cache():

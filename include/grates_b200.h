@@ -53,7 +53,7 @@ typedef struct gb_plan gb_plan;
 
 /* Library version (major*10000 + minor*100 + patch); bumped with every change of this header.  The Python binding
  * refuses a library whose version differs from the one it was written for (grates_b200/_lib.py). */
-#define GB_VERSION 204
+#define GB_VERSION 205
 int gb_version(void);
 
 /* Thread-local description of the last error returned on this thread. */
@@ -286,6 +286,19 @@ int gb_points_synthesis_matrix(gb_points* points, int nmin, double* d_out, void*
  * result is Q C Q' with the rotation of gb_rotate_to_local.  Bit-reproducible from run to run. */
 int gb_points_gradient_covariance(gb_points* points, const double* d_sigma, int nmin, const double* d_frame,
                                   double* d_out, int flags, void* stream);
+/* Normal equations of acceleration observations at the points of a GRADIENT point set (as above): ADDS
+ *   N = sum_p J~_p' W_p J~_p,   J~_p = Q_p J_p  (Q_p = I, or the rotation of gb_rotate_to_local with d_frame)
+ * to d_normals [K'][K'], K' = (nmax + 1)^2 - nmin^2 of the degree-nmax field, degree-wise from nmin.  The caller zeroes
+ * d_normals for a fresh matrix; calls on successive point sets (arcs) accumulate.  On return both triangles hold the sum
+ * and the matrix is exactly symmetric (the upper triangle is accumulated, then mirrored; a lower triangle passed in is
+ * overwritten).
+ *   d_weights [3][npts] positive weights (inverse variances) of the three components per point, or NULL for 1
+ *   d_frame   [4][npts] as for gb_points_gradient_covariance: observations in (east, north, up); NULL: (x, y, z)
+ * The rows sqrt(w) J~ of a block of points are the operands of the DMMA GEMM, contracted over observations; only the
+ * tiles of the upper triangle are computed: about 3 npts K'^2 flops, half those of the full product.
+ * Bit-reproducible from run to run. */
+int gb_points_gradient_normals(gb_points* points, int nmin, const double* d_weights, const double* d_frame,
+                               double* d_normals, void* stream);
 
 /*
  * Consumers of gridded epoch batches that keep the grids on the device.
@@ -338,6 +351,14 @@ int gb_quadratic_forms(const double* d_sigma, int64_t k, const double* d_vec, in
  */
 int gb_gradient_coefficients(const double* d_anm, int n_sets, int nmax, double* d_out, int device, void* stream);
 int gb_rotate_to_local(double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device, void* stream);
+/* The transposes, for the adjoint of the acceleration at points (the operator of iterative least-squares solvers):
+ *   gb_gradient_coefficients_adjoint   T': d_in [n_sets][3][L+1][L+1] packed (x, y, z) -> d_anm [n_sets][L][L] packed,
+ *                                      anm = T_x' in_x + T_y' in_y + T_z' in_z with the factors of
+ *                                      gb_gradient_coefficients; degree 0 of d_in is not read.  A gather, no atomics.
+ *   gb_rotate_from_local               Q': d_xyz [n_sets][3][n_points] (east, north, up) -> (gx, gy, gz) in place, with
+ *                                      d_frame as for gb_rotate_to_local. */
+int gb_gradient_coefficients_adjoint(const double* d_in, int n_sets, int nmax, double* d_anm, int device, void* stream);
+int gb_rotate_from_local(double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device, void* stream);
 
 /* Pinned host memory for the *_host entry points. */
 int gb_host_alloc(void** ptr, uint64_t bytes);

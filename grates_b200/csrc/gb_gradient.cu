@@ -19,6 +19,10 @@
 //                              the transposes T' (summed over the three components) and Q', for the adjoint of the
 //                              acceleration at points (PointsPlan.gradient_adjoint): the same factors (gbgrad::grad_terms)
 //                              and the same rotation kernels, templated on the direction.
+//   gb_gravity_gradient_coefficients, gb_rotate_tensor_to_local
+//                              the gravity gradient tensor: applying the transform twice gives every second derivative
+//                              V_ab as a synthesis at degree N + 2 (T_a T_b, in one gather), and the same rotation kernels
+//                              turn its six components into (east, north, up).
 #include "gb_gradient.cuh"
 
 namespace {
@@ -32,23 +36,16 @@ using gbgrad::rotate_dir;
 
 constexpr int GC_EB = 8;      // epochs per thread: the factors of an output coefficient are computed once for them
 
-// out [E][3][L+1][L+1] packed (x, y, z); one thread per output coefficient of one set, for GC_EB sets.  An output
-// coefficient (n', m', sine) of a component is at most two products f1 a[i1] + f2 a[i2]: its fp term (source order
-// m' - 1) first, then its fm term (source order m' + 1); a source index of -1 is a missing term (out of range, or the
-// sine of order 0).
-__global__ void __launch_bounds__(256)
-gb_gradient_coefficients_kernel(const double* __restrict__ anm, double* __restrict__ out, int L, int E) {
-    const int Lo = L + 1;
-    const int per_set = 3 * Lo * Lo;
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= per_set) return;
-    const int comp = idx / (Lo * Lo);
-    const int rc = idx - comp * Lo * Lo;
-    const int r = rc / Lo, c = rc - r * Lo;
-    const bool sine = r < c;                                  // S_{n', m'} = out[m' - 1][n'], C_{n', m'} = out[n'][m']
-    const int np = sine ? c : r, mp = sine ? r + 1 : c;
-    int i1 = -1, i2 = -1;
-    double f1 = 0.0, f2 = 0.0;
+// An output coefficient (n', m', sine) of component comp of the transform of a packed [L][L] set is at most two products
+// f1 a[i1] + f2 a[i2]: its fp term (source order m' - 1) first, then its fm term (source order m' + 1); a source index of
+// -1 is a missing term (out of range, or the sine of order 0).
+struct Gather {
+    int i1, i2;
+    double f1, f2;
+};
+
+__device__ __forceinline__ Gather gather_terms(int comp, int np, int mp, bool sine, int L) {
+    Gather g{-1, -1, 0.0, 0.0};
     if (np > 0) {
         const int n = np - 1;
         const double q = grad_q(n);
@@ -56,41 +53,121 @@ gb_gradient_coefficients_kernel(const double* __restrict__ anm, double* __restri
         auto Ci = [&](int m) { return n * L + m; };
         auto Si = [&](int m) { return m > 0 ? (m - 1) * L + n : -1; };
         if (comp == 2) {
-            if (mp <= n) { i1 = sine ? Si(mp) : Ci(mp); f1 = -grad_fz(n, mp, q); }
+            if (mp <= n) { g.i1 = sine ? Si(mp) : Ci(mp); g.f1 = -grad_fz(n, mp, q); }
         } else if (comp == 0) {
-            if (mp >= 1) { i1 = sine ? Si(mp - 1) : Ci(mp - 1); f1 = -grad_fp(n, mp - 1, q); }
-            if (mp + 1 <= n) { i2 = sine ? Si(mp + 1) : Ci(mp + 1); f2 = grad_fm(n, mp + 1, q); }
+            if (mp >= 1) { g.i1 = sine ? Si(mp - 1) : Ci(mp - 1); g.f1 = -grad_fp(n, mp - 1, q); }
+            if (mp + 1 <= n) { g.i2 = sine ? Si(mp + 1) : Ci(mp + 1); g.f2 = grad_fm(n, mp + 1, q); }
         } else {
             if (mp >= 1) {
                 const double f = grad_fp(n, mp - 1, q);
-                i1 = sine ? Ci(mp - 1) : Si(mp - 1);
-                f1 = sine ? -f : f;
+                g.i1 = sine ? Ci(mp - 1) : Si(mp - 1);
+                g.f1 = sine ? -f : f;
             }
             if (mp + 1 <= n) {
                 const double f = grad_fm(n, mp + 1, q);
-                i2 = sine ? Ci(mp + 1) : Si(mp + 1);
-                f2 = sine ? -f : f;
+                g.i2 = sine ? Ci(mp + 1) : Si(mp + 1);
+                g.f2 = sine ? -f : f;
             }
         }
     }
+    return g;
+}
+
+// The terms of the output coefficient at packed position idx of a [Lo][Lo] component (Lo = L + 1)
+__device__ __forceinline__ Gather gather_at(int comp, int idx, int L) {
+    const int Lo = L + 1;
+    const int r = idx / Lo, c = idx - r * Lo;
+    const bool sine = r < c;                                  // S_{n', m'} = out[m' - 1][n'], C_{n', m'} = out[n'][m']
+    return gather_terms(comp, sine ? c : r, sine ? r + 1 : c, sine, L);
+}
+
+// f1 x(i1) [+ f2 x(i2)] in the order of the transform, each product and sum rounded on its own; x is called for present
+// terms only.
+template <class Read>
+__device__ __forceinline__ double gather(const Gather& g, Read x) {
+    double v = 0.0;
+    if (g.i1 >= 0) v = __dmul_rn(g.f1, x(g.i1));
+    if (g.i2 >= 0) v = __dadd_rn(v, __dmul_rn(g.f2, x(g.i2)));
+    return v;
+}
+
+// out [E][3][L+1][L+1] packed (x, y, z); one thread per output coefficient of one set, for GC_EB sets.
+__global__ void __launch_bounds__(256)
+gb_gradient_coefficients_kernel(const double* __restrict__ anm, double* __restrict__ out, int L, int E) {
+    const int Lo = L + 1;
+    const int per_set = 3 * Lo * Lo;
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= per_set) return;
+    const int comp = idx / (Lo * Lo);
+    const Gather g = gather_at(comp, idx - comp * Lo * Lo, L);
     const int e0 = blockIdx.y * GC_EB;
     const int e1 = e0 + GC_EB < E ? e0 + GC_EB : E;
     for (int e = e0; e < e1; ++e) {
         const double* a = anm + (size_t)e * L * L;
-        double v = 0.0;
-        if (i1 >= 0) v = __dmul_rn(f1, a[i1]);
-        if (i2 >= 0) v = __dadd_rn(v, __dmul_rn(f2, a[i2]));
-        out[(size_t)e * per_set + idx] = v;
+        out[(size_t)e * per_set + idx] = gather(g, [&](int i) { return a[i]; });
+    }
+}
+
+// out [E][6][L+2][L+2] packed, pairs (a, b) = xx, xy, xz, yy, yz, zz: T_a applied to component b of T(anm), with the
+// arithmetic of two gb_gradient_coefficients calls.  One thread per output coefficient of one set, for GC_EB sets: the
+// outer terms (T_a at degree L) name at most two intermediate coefficients of component b, each of them the inner terms
+// (T_b at degree L - 1) of at most two inputs, so an output reads at most four inputs and nothing is stored in between.
+__global__ void __launch_bounds__(256)
+gb_gravity_gradient_coefficients_kernel(const double* __restrict__ anm, double* __restrict__ out, int L, int E) {
+    const int Lo = L + 2;
+    const int per_set = 6 * Lo * Lo;
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= per_set) return;
+    const int pair = idx / (Lo * Lo);
+    const int ca = pair < 3 ? 0 : pair < 5 ? 1 : 2;
+    const int cb = pair < 3 ? pair : pair < 5 ? pair - 2 : 2;
+    const Gather outer = gather_at(ca, idx - pair * Lo * Lo, L + 1);
+    const Gather inner1 = outer.i1 >= 0 ? gather_at(cb, outer.i1, L) : Gather{-1, -1, 0.0, 0.0};
+    const Gather inner2 = outer.i2 >= 0 ? gather_at(cb, outer.i2, L) : Gather{-1, -1, 0.0, 0.0};
+    const int e0 = blockIdx.y * GC_EB;
+    const int e1 = e0 + GC_EB < E ? e0 + GC_EB : E;
+    for (int e = e0; e < e1; ++e) {
+        const double* a = anm + (size_t)e * L * L;
+        auto read = [&](int i) { return a[i]; };
+        const double g1 = gather(inner1, read), g2 = gather(inner2, read);
+        out[(size_t)e * per_set + idx] = gather(outer, [&](int i) { return i == outer.i1 ? g1 : g2; });
     }
 }
 
 constexpr int ROT_EB = 8;     // epochs per thread: the frame of a point is read once for them
 
-// Two points per thread with 16-byte accesses (n_points even, xyz and frame 16-byte aligned), ROT_EB epochs per thread.
-// TO_LOCAL: Q (gbgrad::rotate), else Q' (gbgrad::rotate_back).
+// What the rotation kernels do to the NC values of one point of one set:
+//   ToLocal / FromLocal   a vector (x, y, z) <-> (east, north, up): Q (gbgrad::rotate) or Q' (gbgrad::rotate_back)
+//   TensorToLocal         a symmetric tensor, upper triangle (xx, xy, xz, yy, yz, zz) -> (ee, en, eu, nn, nu, uu) of
+//                         Q V Q' (gbgrad::rotate_matrix: the columns of V, then the rows of the result)
 template <bool TO_LOCAL>
+struct VectorRotation {
+    static constexpr int NC = 3;
+    __device__ static void apply(const Frame& f, double (&v)[NC]) { rotate_dir<TO_LOCAL>(f, v[0], v[1], v[2]); }
+};
+using ToLocal = VectorRotation<true>;
+using FromLocal = VectorRotation<false>;
+
+struct TensorToLocal {
+    static constexpr int NC = 6;
+    __device__ static void apply(const Frame& f, double (&v)[NC]) {
+        double M[3][3] = {{v[0], v[1], v[2]}, {v[1], v[3], v[4]}, {v[2], v[4], v[5]}};
+        gbgrad::rotate_matrix(f, M);
+        v[0] = M[0][0];
+        v[1] = M[0][1];
+        v[2] = M[0][2];
+        v[3] = M[1][1];
+        v[4] = M[1][2];
+        v[5] = M[2][2];
+    }
+};
+
+// Two points per thread with 16-byte accesses (n_points even, values and frame 16-byte aligned), ROT_EB epochs per
+// thread; values [E][Op::NC][P].
+template <class Op>
 __global__ void __launch_bounds__(256)
-gb_rotate_vec2(double* __restrict__ xyz, const double* __restrict__ frame, int E, long long P) {
+gb_rotate_vec2(double* __restrict__ vals, const double* __restrict__ frame, int E, long long P) {
+    constexpr int NC = Op::NC;
     const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;      // point pair
     if (2 * j >= P) return;
     const double2 ct = reinterpret_cast<const double2*>(frame)[j];
@@ -101,38 +178,43 @@ gb_rotate_vec2(double* __restrict__ xyz, const double* __restrict__ frame, int E
     const int e0 = blockIdx.y * ROT_EB;
     const int e1 = e0 + ROT_EB < E ? e0 + ROT_EB : E;
     for (int e = e0; e < e1; ++e) {
-        double2* gx = reinterpret_cast<double2*>(xyz + (size_t)e * 3 * P);
-        double2* gy = reinterpret_cast<double2*>(xyz + (size_t)e * 3 * P + P);
-        double2* gz = reinterpret_cast<double2*>(xyz + (size_t)e * 3 * P + 2 * P);
-        double2 x = gx[j], y = gy[j], z = gz[j];
-        rotate_dir<TO_LOCAL>(f0, x.x, y.x, z.x);
-        rotate_dir<TO_LOCAL>(f1, x.y, y.y, z.y);
-        gx[j] = x;
-        gy[j] = y;
-        gz[j] = z;
+        double2* g = reinterpret_cast<double2*>(vals + (size_t)e * NC * P);
+        double v0[NC], v1[NC];
+#pragma unroll
+        for (int c = 0; c < NC; ++c) {
+            const double2 x = g[c * (P / 2) + j];
+            v0[c] = x.x;
+            v1[c] = x.y;
+        }
+        Op::apply(f0, v0);
+        Op::apply(f1, v1);
+#pragma unroll
+        for (int c = 0; c < NC; ++c) g[c * (P / 2) + j] = make_double2(v0[c], v1[c]);
     }
 }
 
 // Any point count or alignment: one point per thread, the same arithmetic.
-template <bool TO_LOCAL>
+template <class Op>
 __global__ void __launch_bounds__(256)
-gb_rotate_scalar(double* __restrict__ xyz, const double* __restrict__ frame, int E, long long P) {
+gb_rotate_scalar(double* __restrict__ vals, const double* __restrict__ frame, int E, long long P) {
+    constexpr int NC = Op::NC;
     const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
     const Frame f{frame[p], frame[P + p], frame[2 * P + p], frame[3 * P + p]};
     const int e0 = blockIdx.y * ROT_EB;
     const int e1 = e0 + ROT_EB < E ? e0 + ROT_EB : E;
     for (int e = e0; e < e1; ++e) {
-        double* g = xyz + (size_t)e * 3 * P;
-        double x = g[p], y = g[P + p], z = g[2 * P + p];
-        rotate_dir<TO_LOCAL>(f, x, y, z);
-        g[p] = x;
-        g[P + p] = y;
-        g[2 * P + p] = z;
+        double* g = vals + (size_t)e * NC * P;
+        double v[NC];
+#pragma unroll
+        for (int c = 0; c < NC; ++c) v[c] = g[c * P + p];
+        Op::apply(f, v);
+#pragma unroll
+        for (int c = 0; c < NC; ++c) g[c * P + p] = v[c];
     }
 }
 
-template <bool TO_LOCAL>
+template <class Op>
 int rotate_sets(const char* name, double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device,
                 void* stream) {
     GB_REQUIRE(n_sets >= 0 && n_points >= 0, "%s: negative size (n_sets=%d, n_points=%lld)", name, n_sets,
@@ -147,10 +229,10 @@ int rotate_sets(const char* name, double* d_xyz, const double* d_frame, int n_se
                      reinterpret_cast<uintptr_t>(d_frame) % 16 == 0;
     if (vec) {
         dim3 grid((unsigned)((n_points / 2 + 255) / 256), eb);
-        gb_rotate_vec2<TO_LOCAL><<<grid, 256, 0, st>>>(d_xyz, d_frame, n_sets, n_points);
+        gb_rotate_vec2<Op><<<grid, 256, 0, st>>>(d_xyz, d_frame, n_sets, n_points);
     } else {
         dim3 grid((unsigned)((n_points + 255) / 256), eb);
-        gb_rotate_scalar<TO_LOCAL><<<grid, 256, 0, st>>>(d_xyz, d_frame, n_sets, n_points);
+        gb_rotate_scalar<Op><<<grid, 256, 0, st>>>(d_xyz, d_frame, n_sets, n_points);
     }
     GB_LAUNCH_CHECK();
     return GB_OK;
@@ -208,12 +290,12 @@ extern "C" int gb_gradient_coefficients(const double* d_anm, int n_sets, int nma
 
 extern "C" int gb_rotate_to_local(double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device,
                                   void* stream) {
-    return rotate_sets<true>("gb_rotate_to_local", d_xyz, d_frame, n_sets, n_points, device, stream);
+    return rotate_sets<ToLocal>("gb_rotate_to_local", d_xyz, d_frame, n_sets, n_points, device, stream);
 }
 
 extern "C" int gb_rotate_from_local(double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device,
                                     void* stream) {
-    return rotate_sets<false>("gb_rotate_from_local", d_xyz, d_frame, n_sets, n_points, device, stream);
+    return rotate_sets<FromLocal>("gb_rotate_from_local", d_xyz, d_frame, n_sets, n_points, device, stream);
 }
 
 extern "C" int gb_gradient_coefficients_adjoint(const double* d_in, int n_sets, int nmax, double* d_anm, int device,
@@ -231,4 +313,28 @@ extern "C" int gb_gradient_coefficients_adjoint(const double* d_in, int n_sets, 
     gb_gradient_coefficients_adjoint_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_in, d_anm, L, n_sets);
     GB_LAUNCH_CHECK();
     return GB_OK;
+}
+
+extern "C" int gb_gravity_gradient_coefficients(const double* d_anm, int n_sets, int nmax, double* d_out, int device,
+                                                void* stream) {
+    GB_REQUIRE(n_sets >= 0 && nmax >= 0, "gb_gravity_gradient_coefficients: negative size (n_sets=%d, nmax=%d)", n_sets,
+               nmax);
+    if (n_sets == 0) return GB_OK;
+    GB_REQUIRE(d_anm && d_out, "gb_gravity_gradient_coefficients: NULL device pointer");
+    GB_REQUIRE(nmax < 8192, "gb_gravity_gradient_coefficients: nmax=%d too large (at most 8191)", nmax);
+    const int eb = (n_sets + GC_EB - 1) / GC_EB;
+    GB_REQUIRE(eb <= 65535, "gb_gravity_gradient_coefficients: at most %d sets per call", 65535 * GC_EB);
+    GB_CUDA(cudaSetDevice(device));
+    const int L = nmax + 1;
+    const int per_set = 6 * (L + 2) * (L + 2);
+    dim3 grid((per_set + 255) / 256, eb);
+    gb_gravity_gradient_coefficients_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_anm, d_out, L,
+                                                                                                 n_sets);
+    GB_LAUNCH_CHECK();
+    return GB_OK;
+}
+
+extern "C" int gb_rotate_tensor_to_local(double* d_v, const double* d_frame, int n_sets, int64_t n_points, int device,
+                                         void* stream) {
+    return rotate_sets<TensorToLocal>("gb_rotate_tensor_to_local", d_v, d_frame, n_sets, n_points, device, stream);
 }

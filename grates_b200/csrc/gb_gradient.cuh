@@ -1,6 +1,6 @@
-// Factors of Cunningham's relation and the rotation to (east, north, up), shared by the gradient transform and its
-// transpose (gb_gradient.cu) and the Jacobian rows of the gradient covariance and normal equations (gb_points.cu): all
-// must use the same expressions.
+// Factors of Cunningham's relation and the rotation to (east, north, up), shared by the gradient and gravity gradient
+// transforms, their rotations and the transpose (gb_gradient.cu) and the Jacobian rows of the gradient covariance and
+// normal equations (gb_points.cu): all must use the same expressions.
 #pragma once
 #include "gb_common.cuh"
 
@@ -113,6 +113,15 @@ template <bool TO_LOCAL>
 __device__ __forceinline__ void rotate_dir(const Frame& f, double& a, double& b, double& c) {
     if constexpr (TO_LOCAL) rotate(f, a, b, c);
     else rotate_back(f, a, b, c);
+}
+
+// Q M Q' of a 3 x 3 matrix in place: rotate on the three columns of M, then on the three rows of the result.  Even for a
+// symmetric M the result is symmetric only to rounding; callers keep one triangle or symmetrise.
+__device__ __forceinline__ void rotate_matrix(const Frame& f, double (&M)[3][3]) {
+#pragma unroll
+    for (int j = 0; j < 3; ++j) rotate(f, M[0][j], M[1][j], M[2][j]);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) rotate(f, M[j][0], M[j][1], M[j][2]);
 }
 
 }  // namespace gbgrad

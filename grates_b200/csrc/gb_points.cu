@@ -652,10 +652,7 @@ gb_points_gradient_finish(const double* __restrict__ part, const double* __restr
     const long long p = p0 + (long long)i;
     if (frame) {
         const gbgrad::Frame f{frame[p], frame[npts + p], frame[2 * npts + p], frame[3 * npts + p]};
-#pragma unroll
-        for (int j = 0; j < 3; ++j) gbgrad::rotate(f, C[0][j], C[1][j], C[2][j]);
-#pragma unroll
-        for (int j = 0; j < 3; ++j) gbgrad::rotate(f, C[j][0], C[j][1], C[j][2]);
+        gbgrad::rotate_matrix(f, C);
 #pragma unroll
         for (int c = 0; c < 3; ++c)
 #pragma unroll

@@ -481,16 +481,23 @@ def _gradient_input(anm, frame):
     return x
 
 
-def _gradient(x, p, frame, shape, device_output, out):
-    """Transform (gb_gradient_coefficients), one synthesis of the 3E sets on the gradient plan p, and for frame='local'
-    the rotation (gb_rotate_to_local) -> [E, 3, *shape]."""
+# order of the derivative -> (components, coefficient transform, rotation to the local frame)
+_DERIVATIVE_CALLS = {1: (3, "gb_gradient_coefficients", "gb_rotate_to_local"),
+                     2: (6, "gb_gravity_gradient_coefficients", "gb_rotate_tensor_to_local")}
+
+
+def _gradient(x, p, frame, shape, device_output, out, order=1):
+    """Transform (gb_gradient_coefficients, or gb_gravity_gradient_coefficients for order 2), one synthesis of the C*E
+    sets on the plan p of that order, and for frame='local' the rotation (gb_rotate_to_local / gb_rotate_tensor_to_local)
+    -> [E, C, *shape] with C = 3 (order 1) or 6 (order 2) components."""
+    ncomp, transform, rotation = _DERIVATIVE_CALLS[order]
     on_device = isinstance(x, torch.Tensor)
     dev = torch.device("cuda", p.device)
     if on_device and x.device.index != p.device:
         raise ValueError("coefficients must be a float64 CUDA tensor on device {0}".format(p.device))
     x = x.contiguous() if on_device else torch.as_tensor(x).to(dev)
     E, L = x.shape[0], x.shape[-1]
-    full = (E, 3) + tuple(shape)
+    full = (E, ncomp) + tuple(shape)
     to_host = not (on_device or device_output)
     if out is not None and to_host:
         _plan._check_out_host(out, full)
@@ -499,12 +506,13 @@ def _gradient(x, p, frame, shape, device_output, out):
     else:
         res = torch.empty(full, dtype=torch.float64, device=dev)
     lib, st = _lib.load(), _plan._stream_handle(p.device)
-    g = torch.empty((E, 3, L + 1, L + 1), dtype=torch.float64, device=dev)
-    _lib.check(lib.gb_gradient_coefficients(ctypes.c_void_p(x.data_ptr()), E, L - 1, ctypes.c_void_p(g.data_ptr()),
-                                            p.device, st))
-    p.synthesis(g.view(3 * E, L + 1, L + 1), out=res.view((3 * E,) + tuple(shape)))
+    Lo = L + order
+    g = torch.empty((E, ncomp, Lo, Lo), dtype=torch.float64, device=dev)
+    _lib.check(getattr(lib, transform)(ctypes.c_void_p(x.data_ptr()), E, L - 1, ctypes.c_void_p(g.data_ptr()),
+                                       p.device, st))
+    p.synthesis(g.view(ncomp * E, Lo, Lo), out=res.view((ncomp * E,) + tuple(shape)))
     if frame == 'local':
-        _lib.check(lib.gb_rotate_to_local(ctypes.c_void_p(res.data_ptr()), ctypes.c_void_p(p.frame.data_ptr()), E,
+        _lib.check(getattr(lib, rotation)(ctypes.c_void_p(res.data_ptr()), ctypes.c_void_p(p.frame.data_ptr()), E,
                                           int(np.prod(shape)), p.device, st))
     if not to_host:
         return res
@@ -526,21 +534,25 @@ def gradient_batch(anm, grid=None, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian'
 
     Each component is a scalar synthesis at degree N + 1 of linearly transformed coefficients (Cunningham's relation,
     gb_gradient_coefficients), so the 3E sets run through the same synthesis kernels as ``to_grid_batch``."""
+    return _derivative_on_grid(anm, grid, GM, R, frame, device_output, out, 1)
+
+
+def _derivative_on_grid(anm, grid, GM, R, frame, device_output, out, order):
     x = _gradient_input(anm, frame)
     grid = GeographicGrid() if grid is None else grid
     if _plan.is_regular(grid):
-        p = _plan.get_gradient_plan(grid, x.shape[-1] - 1, GM, R)
+        p = _plan._derivative_plan(grid, x.shape[-1] - 1, order, GM, R, None)
         shape = (p.nlat, p.nlon)
     elif hasattr(grid, "longitude") and hasattr(grid, "latitude"):
         lon = np.asarray(grid.longitude, dtype=float)
         lat = np.asarray(grid.latitude, dtype=float)
         a, f = grid.semimajor_axis, grid.flattening
-        p = _plan.get_gradient_points_plan(utilities.geocentric_radius(lat, a, f), utilities.colatitude(lat, a, f), lon,
-                                           x.shape[-1] - 1, GM, R)
+        p = _plan._derivative_points_plan(utilities.geocentric_radius(lat, a, f), utilities.colatitude(lat, a, f), lon,
+                                          x.shape[-1] - 1, order, GM, R, None, True)
         shape = (p.npts,)
     else:
         raise TypeError("grid must expose parallels/meridians or longitude/latitude")
-    return _gradient(x, p, frame, shape, device_output, out)
+    return _gradient(x, p, frame, shape, device_output, out, order)
 
 
 def gradient_at_positions(anm, positions, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian', device_output=False, out=None):
@@ -548,10 +560,40 @@ def gradient_at_positions(anm, positions, GM=GM_DEFAULT, R=R_DEFAULT, frame='car
     metres (any radius, e.g. along an orbit) -> [E, 3, P] in m/s^2.  frame, the result's kind and ``out`` as for
     ``gradient_batch``; the local frame is geocentric spherical at each position (longitude 0 on the polar axis).
     Non-finite positions and the origin raise ValueError."""
+    return _derivative_at_positions(anm, positions, GM, R, frame, device_output, out, 1)
+
+
+def _derivative_at_positions(anm, positions, GM, R, frame, device_output, out, order):
     x = _gradient_input(anm, frame)
     r, colat, lon = utilities.cartesian_to_spherical(positions)
-    p = _plan.get_gradient_points_plan(r, colat, lon, x.shape[-1] - 1, GM, R)
-    return _gradient(x, p, frame, (p.npts,), device_output, out)
+    p = _plan._derivative_points_plan(r, colat, lon, x.shape[-1] - 1, order, GM, R, None, True)
+    return _gradient(x, p, frame, (p.npts,), device_output, out, order)
+
+
+def gravity_gradient_batch(anm, grid=None, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian', device_output=False,
+                           out=None):
+    """Gravity gradient tensor (the second derivatives of the potential) of a batch of coefficient sets on a grid, in
+    s^-2 (1 E = 1 Eotvos = 1e-9 s^-2).
+
+    anm: [E, L, L] packed coefficients (numpy array or CUDA float64 tensor).  Returns the upper triangle of the
+    symmetric tensor, [E, 6, nlat, nlon] on a regular grid, [E, 6, points] on a grid with longitude / latitude, at the
+    geocentric radius of the ellipsoid.  frame='cartesian': (xx, xy, xz, yy, yz, zz) Earth-fixed; frame='local':
+    (ee, en, eu, nn, nu, uu) of Q V Q' in (east, north, up) of the geocentric spherical frame, as for ``gradient_batch``.
+    The potential only: no kernel and no centrifugal term.  The result's kind and ``out`` as for ``gradient_batch``.
+
+    Component (a, b) is a scalar synthesis at degree N + 2 of the coefficients transformed twice by Cunningham's
+    relation (gb_gravity_gradient_coefficients), so the 6E sets run through one synthesis on the same kernels as
+    ``to_grid_batch``; no 1 / sin(theta) is involved, so the poles are regular."""
+    return _derivative_on_grid(anm, grid, GM, R, frame, device_output, out, 2)
+
+
+def gravity_gradient_at_positions(anm, positions, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian', device_output=False,
+                                  out=None):
+    """Gravity gradient tensor of a batch of coefficient sets at Earth-fixed Cartesian positions [P, 3] in metres (any
+    radius, e.g. along an orbit) -> [E, 6, P] in s^-2 (1 E = 1e-9 s^-2).  Components, frame, the result's kind and
+    ``out`` as for ``gravity_gradient_batch``; the local frame as for ``gradient_at_positions``.  Non-finite positions
+    and the origin raise ValueError."""
+    return _derivative_at_positions(anm, positions, GM, R, frame, device_output, out, 2)
 
 
 def _gradient_covariance_input(covariance_matrix, min_degree, max_degree, frame, full):

@@ -748,12 +748,25 @@ def _cached(key, make):
         return plan
 
 
+def _derivative_degree_factors(radius, max_degree, order, GM, R):
+    """kn[p, n] = GM/R^(order+1) (R/r_p)^(n+1), n = 0..max_degree + order; columns 0..order-1 are zero (those degrees of
+    the transformed coefficients are)."""
+    kn = np.power((R / np.asarray(radius, dtype=float))[:, None], np.arange(max_degree + order + 1, dtype=int) + 1) * (
+        GM / R ** (order + 1))
+    kn[:, :order] = 0.0
+    return kn
+
+
 def gradient_degree_factors(radius, max_degree, GM, R):
     """Degree factors kn'[p, n'] = GM/R^2 (R/r_p)^(n'+1), n' = 0..max_degree + 1, of the syntheses that turn the output of
     gb_gradient_coefficients into the components of grad V; column 0 is zero (degree 0 of those coefficients is)."""
-    kn = np.power((R / np.asarray(radius, dtype=float))[:, None], np.arange(max_degree + 2, dtype=int) + 1) * (GM / R ** 2)
-    kn[:, 0] = 0.0
-    return kn
+    return _derivative_degree_factors(radius, max_degree, 1, GM, R)
+
+
+def gravity_gradient_degree_factors(radius, max_degree, GM, R):
+    """Degree factors kn''[p, n''] = GM/R^3 (R/r_p)^(n''+1), n'' = 0..max_degree + 2, of the syntheses that turn the output
+    of gb_gravity_gradient_coefficients into the components of the gravity gradient tensor; columns 0 and 1 are zero."""
+    return _derivative_degree_factors(radius, max_degree, 2, GM, R)
 
 
 def _frame_table(colat, lon, device):
@@ -762,23 +775,58 @@ def _frame_table(colat, lon, device):
     return torch.as_tensor(np.ascontiguousarray(table)).to(torch.device("cuda", device))
 
 
+# order of the derivative -> (name, cache variant of the grid plan, of the point plan)
+_DERIVATIVES = {1: ("gradient", "gradient", "gradient points"),
+                2: ("gravity gradient", "gravity gradient", "gravity gradient points")}
+
+
+def _derivative_plan(grid, max_degree, order, GM, R, device):
+    dev = _current_device(device)
+    meridians = np.asarray(grid.meridians, dtype=float)
+    parallels = np.asarray(grid.parallels, dtype=float)
+    a, f = float(grid.semimajor_axis), float(grid.flattening)
+    name, variant, _ = _DERIVATIVES[order]
+    key = (meridians.tobytes(), parallels.tobytes(), a, f, int(max_degree), float(GM), float(R), dev, variant)
+
+    def make():
+        kn = _derivative_degree_factors(utilities.geocentric_radius(parallels, a, f), int(max_degree), order, GM, R)
+        plan = SHPlan(meridians, parallels, a, f, int(max_degree) + order, name, GM, R, dev, degree_factors=kn)
+        nlat, nlon = plan.nlat, plan.nlon
+        plan.frame = _frame_table(np.repeat(plan.colat, nlon), np.tile(meridians, nlat), dev)
+        return plan
+    return _cached(key, make)
+
+
 def get_gradient_plan(grid, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
     """Cached SHPlan at degree max_degree + 1 for the gradient of degree-max_degree coefficients on a regular grid:
     the grid's geocentric colatitudes, the degree factors of gradient_degree_factors at the geocentric radius of each
     parallel, and ``plan.frame`` [4, nlat * nlon], the per-point table of the rotation to (east, north, up).  Its cache
     key carries a 'gradient' variant: it is never mistaken for a potential plan of the same grid and degree."""
+    return _derivative_plan(grid, max_degree, 1, GM, R, device)
+
+
+def get_gravity_gradient_plan(grid, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
+    """Cached SHPlan at degree max_degree + 2 for the gravity gradient tensor of degree-max_degree coefficients on a
+    regular grid: as get_gradient_plan, with the degree factors of gravity_gradient_degree_factors.  Its cache key
+    carries its own variant: it is never mistaken for the gradient plan of degree max_degree + 1, which has the same
+    degree and other factors."""
+    return _derivative_plan(grid, max_degree, 2, GM, R, device)
+
+
+def _derivative_points_plan(radius, colat, lon, max_degree, order, GM, R, device, cached):
     dev = _current_device(device)
-    meridians = np.asarray(grid.meridians, dtype=float)
-    parallels = np.asarray(grid.parallels, dtype=float)
-    a, f = float(grid.semimajor_axis), float(grid.flattening)
-    key = (meridians.tobytes(), parallels.tobytes(), a, f, int(max_degree), float(GM), float(R), dev, "gradient")
+    radius, colat, lon = (np.ascontiguousarray(v, dtype=float) for v in (radius, colat, lon))
+    name, _, variant = _DERIVATIVES[order]
 
     def make():
-        kn = gradient_degree_factors(utilities.geocentric_radius(parallels, a, f), int(max_degree), GM, R)
-        plan = SHPlan(meridians, parallels, a, f, int(max_degree) + 1, "gradient", GM, R, dev, degree_factors=kn)
-        nlat, nlon = plan.nlat, plan.nlon
-        plan.frame = _frame_table(np.repeat(plan.colat, nlon), np.tile(meridians, nlat), dev)
+        kn = _derivative_degree_factors(radius, int(max_degree), order, GM, R)
+        plan = PointsPlan(lon, 0.5 * np.pi - colat, utilities.A_GRS80, utilities.F_GRS80, int(max_degree) + order, name,
+                          GM, R, dev, degree_factors=kn, colatitude=colat)
+        plan.frame = _frame_table(colat, lon, dev)
         return plan
+    if not cached:
+        return make()
+    key = (variant, radius.tobytes(), colat.tobytes(), lon.tobytes(), int(max_degree), float(GM), float(R), dev)
     return _cached(key, make)
 
 
@@ -786,21 +834,19 @@ def get_gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14
     """Cached PointsPlan at degree max_degree + 1 for the gradient at points of geocentric radius / colatitude /
     longitude (any radius: on the ellipsoid for an IrregularGrid, anywhere for Cartesian positions), with ``plan.frame``
     [4, P] as for get_gradient_plan."""
-    dev = _current_device(device)
-    radius, colat, lon = (np.ascontiguousarray(v, dtype=float) for v in (radius, colat, lon))
-    key = ("gradient points", radius.tobytes(), colat.tobytes(), lon.tobytes(), int(max_degree), float(GM), float(R), dev)
-    return _cached(key, lambda: gradient_points_plan(radius, colat, lon, max_degree, GM, R, dev))
+    return _derivative_points_plan(radius, colat, lon, max_degree, 1, GM, R, device, True)
 
 
 def gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
     """The PointsPlan of get_gradient_points_plan, not cached: the caller closes it (long position arrays in chunks)."""
-    dev = _current_device(device)
-    radius, colat, lon = (np.ascontiguousarray(v, dtype=float) for v in (radius, colat, lon))
-    kn = gradient_degree_factors(radius, int(max_degree), GM, R)
-    plan = PointsPlan(lon, 0.5 * np.pi - colat, utilities.A_GRS80, utilities.F_GRS80, int(max_degree) + 1, "gradient",
-                      GM, R, dev, degree_factors=kn, colatitude=colat)
-    plan.frame = _frame_table(colat, lon, dev)
-    return plan
+    return _derivative_points_plan(radius, colat, lon, max_degree, 1, GM, R, device, False)
+
+
+def get_gravity_gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06,
+                                     device=None):
+    """Cached PointsPlan at degree max_degree + 2 for the gravity gradient tensor at points, as get_gradient_points_plan
+    with the degree factors of gravity_gradient_degree_factors and its own cache variant."""
+    return _derivative_points_plan(radius, colat, lon, max_degree, 2, GM, R, device, True)
 
 
 def clear_plan_cache():

@@ -53,7 +53,7 @@ typedef struct gb_plan gb_plan;
 
 /* Library version (major*10000 + minor*100 + patch); bumped with every change of this header.  The Python binding
  * refuses a library whose version differs from the one it was written for (grates_b200/_lib.py). */
-#define GB_VERSION 205
+#define GB_VERSION 206
 int gb_version(void);
 
 /* Thread-local description of the last error returned on this thread. */
@@ -359,6 +359,20 @@ int gb_rotate_to_local(double* d_xyz, const double* d_frame, int n_sets, int64_t
  *                                      d_frame as for gb_rotate_to_local. */
 int gb_gradient_coefficients_adjoint(const double* d_in, int n_sets, int nmax, double* d_anm, int device, void* stream);
 int gb_rotate_from_local(double* d_xyz, const double* d_frame, int n_sets, int64_t n_points, int device, void* stream);
+/* The gravity gradient tensor (second derivatives of the potential, in s^-2): the transform applied twice makes every
+ * V_ab of a degree-nmax field a synthesis at degree nmax + 2, with degree factors GM/R^3 (R/r)^(n''+1).
+ *   gb_gravity_gradient_coefficients   d_anm [n_sets][L][L] packed -> d_out [n_sets][6][L+2][L+2] packed, components
+ *                                      (xx, xy, xz, yy, yz, zz) Earth-fixed.  Component (a, b) is T_a(T_b(anm)):
+ *                                      bit for bit gb_gradient_coefficients applied to anm, then (nmax + 1) to component
+ *                                      b of its result.  Degrees 0 and 1 of d_out are zero.  A gather, no atomics.
+ *   gb_rotate_tensor_to_local          d_v [n_sets][6][n_points] (xx, xy, xz, yy, yz, zz) -> (ee, en, eu, nn, nu, uu) in
+ *                                      place: the upper triangle of Q V Q', with Q and d_frame as for
+ *                                      gb_rotate_to_local, computed as Q on the three columns of V and then on the three
+ *                                      rows of the result. */
+int gb_gravity_gradient_coefficients(const double* d_anm, int n_sets, int nmax, double* d_out, int device,
+                                     void* stream);
+int gb_rotate_tensor_to_local(double* d_v, const double* d_frame, int n_sets, int64_t n_points, int device,
+                              void* stream);
 
 /* Pinned host memory for the *_host entry points. */
 int gb_host_alloc(void** ptr, uint64_t bytes);

@@ -222,6 +222,8 @@ extern "C" int gb_dgemm(int trans_a, int trans_b, int64_t m, int64_t n, int64_t 
 extern "C" int gb_dpotrf_upper(double* d_a, int64_t n, int64_t lda, int* d_info, int device, void* stream) {
     GB_REQUIRE(n >= 0 && lda >= n, "gb_dpotrf_upper: bad size");
     GB_REQUIRE(d_info != nullptr, "gb_dpotrf_upper: d_info is NULL");
+    // the lower-triangle clear at the end takes one grid row per matrix row (at most 65535): refuse before any write
+    GB_REQUIRE(n <= 65535, "gb_dpotrf_upper: blocks of more than 65535 rows are not supported");
     GB_CUDA(cudaSetDevice(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     GB_CUDA(cudaMemsetAsync(d_info, 0, sizeof(int), st));
@@ -246,7 +248,6 @@ extern "C" int gb_dpotrf_upper(double* d_a, int64_t n, int64_t lda, int* d_info,
         }
     }
     // the strict lower triangle is not referenced above: clear it, scipy.linalg.cholesky(lower=False) returns a clean factor
-    GB_REQUIRE(n <= 65535, "gb_dpotrf_upper: blocks of more than 65535 rows are not supported");
     gb_zero_lower_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)n), 256, 0, st>>>(d_a, n, lda);
     GB_LAUNCH_CHECK();
     return GB_OK;

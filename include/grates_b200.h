@@ -408,7 +408,8 @@ int64_t gb_launch_count(int reset);
  *   gb_dgemm         C[m][n] = alpha * op(A) * op(B) + beta * C; trans_a: A is stored [k][m], trans_b: B is stored
  *                    [n][k]; upper_only: tiles strictly below the diagonal are skipped (symmetric updates)
  *   gb_dpotrf_upper  A = W' W in place, W upper triangular, strict lower triangle zeroed; *d_info (device int) = 0 or
- *                    the 1-based index of the first non-positive pivot (scipy raises LinAlgError there)
+ *                    the 1-based index of the first non-positive pivot (scipy raises LinAlgError there); n > 65535
+ *                    fails with GB_ERR_ARGUMENT before anything is written
  *   gb_dtrsm_upper   solves W X = B (trans = 0) or W' X = B (trans = 1) in place of B[n][m], W upper triangular
  */
 int gb_dgemm(int trans_a, int trans_b, int64_t m, int64_t n, int64_t k, double alpha, const double* d_a, int64_t lda,

@@ -7,7 +7,7 @@ torch.distributed); all arithmetic on the path runs in hand-written CUDA kernels
 C ABI of ``include/grates_b200.h``.  There is no CPU fallback.
 """
 from . import _lib, utilities, kernel, plan, grid, gravityfield, filter, distributed, lstsq, io  # noqa: F401
-from .gravityfield import PotentialCoefficients, SurfaceMasCons, RadialBasisFunctions, AnisotropicBasisFunctions, TimeSeries, to_grid_batch, gridded_rms, grid_statistics, ravel_batch, gradient_batch, gradient_at_positions, gradient_covariance_propagation, gradient_covariance_at_positions, gradient_adjoint_at_positions, gradient_normal_equations_at_positions, gravity_gradient_batch, gravity_gradient_at_positions  # noqa: F401
+from .gravityfield import PotentialCoefficients, SurfaceMasCons, RadialBasisFunctions, AnisotropicBasisFunctions, TimeSeries, to_grid_batch, gridded_rms, grid_statistics, ravel_batch, gradient_batch, gradient_at_positions, gradient_covariance_propagation, gradient_covariance_at_positions, gradient_adjoint_at_positions, gradient_normal_equations_at_positions, gravity_gradient_batch, gravity_gradient_at_positions, gravity_gradient_adjoint_at_positions, gravity_gradient_normal_equations_at_positions  # noqa: F401
 from .grid import (RegularGrid, IrregularGrid, GeographicGrid, GaussGrid, analysis_batch, basin_variances,  # noqa: F401
                    covariance_from_normals)
 from .filter import OrderWiseFilter, Gaussian, Butterworth, GeneralMatrix, VDK, SpatialFilter  # noqa: F401

@@ -12,7 +12,7 @@ _c_int64_p = ctypes.POINTER(ctypes.c_int64)
 _vp = ctypes.c_void_p
 
 GB_OK, GB_ERR_ARGUMENT, GB_ERR_CUDA, GB_ERR_UNSUPPORTED, GB_ERR_MEMORY = 0, 1, 2, 3, 4
-GB_VERSION = 206        # must equal GB_VERSION of include/grates_b200.h: the argtypes below describe THAT header
+GB_VERSION = 207        # must equal GB_VERSION of include/grates_b200.h: the argtypes below describe THAT header
 
 # name -> (restype, argtypes); must list every symbol of include/grates_b200.h
 SIGNATURES = {
@@ -56,6 +56,7 @@ SIGNATURES = {
     "gb_points_synthesis_matrix": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp]),
     "gb_points_gradient_covariance": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, ctypes.c_int, _vp]),
     "gb_points_gradient_normals": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, _vp, _vp]),
+    "gb_points_gravity_gradient_normals": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, _vp, _vp]),
     "gb_temporal_rms": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int64, _vp, ctypes.c_int, _vp]),
     "gb_weighted_moments": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int, ctypes.c_int64, _vp, ctypes.c_int, _vp]),
     "gb_ravel_coefficients": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, _vp]),
@@ -66,6 +67,9 @@ SIGNATURES = {
     "gb_rotate_from_local": (ctypes.c_int, [_vp, _vp, ctypes.c_int, ctypes.c_int64, ctypes.c_int, _vp]),
     "gb_gravity_gradient_coefficients": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, _vp]),
     "gb_rotate_tensor_to_local": (ctypes.c_int, [_vp, _vp, ctypes.c_int, ctypes.c_int64, ctypes.c_int, _vp]),
+    "gb_gravity_gradient_coefficients_adjoint": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int,
+                                                                 _vp]),
+    "gb_rotate_tensor_from_local": (ctypes.c_int, [_vp, _vp, ctypes.c_int, ctypes.c_int64, ctypes.c_int, _vp]),
     "gb_host_alloc":(ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_uint64]),
     "gb_host_free": (ctypes.c_int, [_vp]),
     "gb_probe_fp64_peak": (ctypes.c_int, [ctypes.c_int, _c_double_p, _c_double_p]),

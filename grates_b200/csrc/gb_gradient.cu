@@ -23,6 +23,10 @@
 //                              the gravity gradient tensor: applying the transform twice gives every second derivative
 //                              V_ab as a synthesis at degree N + 2 (T_a T_b, in one gather), and the same rotation kernels
 //                              turn its six components into (east, north, up).
+//   gb_gravity_gradient_coefficients_adjoint, gb_rotate_tensor_from_local
+//                              their transposes, for the adjoint of the gravity gradient at points
+//                              (PointsPlan.gravity_gradient_adjoint): the composed terms of gbgrad::apply_pair and
+//                              gbgrad::rotate_tensor_transpose.
 #include "gb_gradient.cuh"
 
 namespace {
@@ -150,16 +154,13 @@ using FromLocal = VectorRotation<false>;
 
 struct TensorToLocal {
     static constexpr int NC = 6;
-    __device__ static void apply(const Frame& f, double (&v)[NC]) {
-        double M[3][3] = {{v[0], v[1], v[2]}, {v[1], v[3], v[4]}, {v[2], v[4], v[5]}};
-        gbgrad::rotate_matrix(f, M);
-        v[0] = M[0][0];
-        v[1] = M[0][1];
-        v[2] = M[0][2];
-        v[3] = M[1][1];
-        v[4] = M[1][2];
-        v[5] = M[2][2];
-    }
+    __device__ static void apply(const Frame& f, double (&v)[NC]) { gbgrad::rotate_tensor(f, v); }
+};
+
+//   TensorFromLocal       the transpose of TensorToLocal on the 6-vectors (gbgrad::rotate_tensor_transpose)
+struct TensorFromLocal {
+    static constexpr int NC = 6;
+    __device__ static void apply(const Frame& f, double (&v)[NC]) { gbgrad::rotate_tensor_transpose(f, v); }
 };
 
 // Two points per thread with 16-byte accesses (n_points even, values and frame 16-byte aligned), ROT_EB epochs per
@@ -269,6 +270,35 @@ gb_gradient_coefficients_adjoint_kernel(const double* __restrict__ in, double* _
     }
 }
 
+// The transpose of gb_gravity_gradient_coefficients_kernel, summed over the pairs: in [E][6][L+2][L+2] -> anm [E][L][L]
+// packed.  One thread per output coefficient (n, m, s) of one set, for GC_EB sets: the composed terms of
+// gbgrad::apply_pair read degree n + 2 of each pair, added in the order xx, xy, xz, yy, yz, zz (a gather, no atomics).
+__global__ void __launch_bounds__(256)
+gb_gravity_gradient_coefficients_adjoint_kernel(const double* __restrict__ in, double* __restrict__ anm, int L, int E) {
+    const int Lo = L + 2;
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= L * L) return;
+    const int r = idx / L, c = idx - r * L;
+    const int s = r < c ? 1 : 0;                             // S_nm = anm[m - 1][n], C_nm = anm[n][m]
+    const int n = s ? c : r, m = s ? r + 1 : c;
+    const double q0 = grad_q(n), q1 = grad_q(n + 1);
+    const int e0 = blockIdx.y * GC_EB;
+    const int e1 = e0 + GC_EB < E ? e0 + GC_EB : E;
+    for (int e = e0; e < e1; ++e) {
+        double v = 0.0;
+#pragma unroll
+        for (int pair = 0; pair < 6; ++pair) {
+            const double* g = in + ((size_t)e * 6 + pair) * Lo * Lo;
+            // packed position of (n + 2, mp, sp): C at [n + 2][mp], S at [mp - 1][n + 2]
+            v = __dadd_rn(v, gbgrad::apply_pair(gbgrad::pair_a(pair), gbgrad::pair_b(pair), n, m, s, q0, q1,
+                                                [&](int mp, int sp) {
+                                                    return g[sp ? (mp - 1) * Lo + n + 2 : (n + 2) * Lo + mp];
+                                                }));
+        }
+        anm[(size_t)e * L * L + idx] = v;
+    }
+}
+
 }  // namespace
 
 extern "C" int gb_gradient_coefficients(const double* d_anm, int n_sets, int nmax, double* d_out, int device,
@@ -337,4 +367,27 @@ extern "C" int gb_gravity_gradient_coefficients(const double* d_anm, int n_sets,
 extern "C" int gb_rotate_tensor_to_local(double* d_v, const double* d_frame, int n_sets, int64_t n_points, int device,
                                          void* stream) {
     return rotate_sets<TensorToLocal>("gb_rotate_tensor_to_local", d_v, d_frame, n_sets, n_points, device, stream);
+}
+
+extern "C" int gb_gravity_gradient_coefficients_adjoint(const double* d_in, int n_sets, int nmax, double* d_anm,
+                                                        int device, void* stream) {
+    GB_REQUIRE(n_sets >= 0 && nmax >= 0, "gb_gravity_gradient_coefficients_adjoint: negative size (n_sets=%d, nmax=%d)",
+               n_sets, nmax);
+    if (n_sets == 0) return GB_OK;
+    GB_REQUIRE(d_in && d_anm, "gb_gravity_gradient_coefficients_adjoint: NULL device pointer");
+    GB_REQUIRE(nmax < 8192, "gb_gravity_gradient_coefficients_adjoint: nmax=%d too large (at most 8191)", nmax);
+    const int eb = (n_sets + GC_EB - 1) / GC_EB;
+    GB_REQUIRE(eb <= 65535, "gb_gravity_gradient_coefficients_adjoint: at most %d sets per call", 65535 * GC_EB);
+    GB_CUDA(cudaSetDevice(device));
+    const int L = nmax + 1;
+    dim3 grid((L * L + 255) / 256, eb);
+    gb_gravity_gradient_coefficients_adjoint_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_in, d_anm, L,
+                                                                                                         n_sets);
+    GB_LAUNCH_CHECK();
+    return GB_OK;
+}
+
+extern "C" int gb_rotate_tensor_from_local(double* d_v, const double* d_frame, int n_sets, int64_t n_points, int device,
+                                           void* stream) {
+    return rotate_sets<TensorFromLocal>("gb_rotate_tensor_from_local", d_v, d_frame, n_sets, n_points, device, stream);
 }

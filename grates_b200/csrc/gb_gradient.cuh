@@ -78,6 +78,19 @@ __device__ __forceinline__ double apply(const Terms& t, Read x) {
     return v;
 }
 
+// The components (a, b) of the six pairs xx, xy, xz, yy, yz, zz of the gravity gradient tensor
+__device__ __forceinline__ int pair_a(int pair) { return pair < 3 ? 0 : pair < 5 ? 1 : 2; }
+__device__ __forceinline__ int pair_b(int pair) { return pair < 3 ? pair : pair < 5 ? pair - 2 : 2; }
+
+// The composed terms of V_ab = T_a T_b for the input (n, m, s): the terms of T_b at degree n name at most two coefficients
+// (n + 1, mp, sp), each of them the terms of T_a at degree n + 1 of at most two values x(order, sine) at degree n + 2, so
+// at most four reads.  q0 = grad_q(n), q1 = grad_q(n + 1).  Every product of the degree-(n+2) values with the composed
+// transform -- the transposed transform, the Jacobian rows F''_p T_a T_b -- is this one expression.
+template <class Read>
+__device__ __forceinline__ double apply_pair(int a, int b, int n, int m, int s, double q0, double q1, Read x) {
+    return apply(grad_terms(b, n, m, s, q0), [&](int mp, int sp) { return apply(grad_terms(a, n + 1, mp, sp, q1), x); });
+}
+
 struct Frame { double ct, st, cl, sl; };
 
 // east  = -sl gx + cl gy
@@ -115,13 +128,43 @@ __device__ __forceinline__ void rotate_dir(const Frame& f, double& a, double& b,
     else rotate_back(f, a, b, c);
 }
 
-// Q M Q' of a 3 x 3 matrix in place: rotate on the three columns of M, then on the three rows of the result.  Even for a
-// symmetric M the result is symmetric only to rounding; callers keep one triangle or symmetrise.
+// Q M Q' (TO_LOCAL) or Q' M Q of a 3 x 3 matrix in place: rotate on the three columns of M, then on the three rows of the
+// result.  Even for a symmetric M the result is symmetric only to rounding; callers keep one triangle or symmetrise.
+template <bool TO_LOCAL = true>
 __device__ __forceinline__ void rotate_matrix(const Frame& f, double (&M)[3][3]) {
 #pragma unroll
-    for (int j = 0; j < 3; ++j) rotate(f, M[0][j], M[1][j], M[2][j]);
+    for (int j = 0; j < 3; ++j) rotate_dir<TO_LOCAL>(f, M[0][j], M[1][j], M[2][j]);
 #pragma unroll
-    for (int j = 0; j < 3; ++j) rotate(f, M[j][0], M[j][1], M[j][2]);
+    for (int j = 0; j < 3; ++j) rotate_dir<TO_LOCAL>(f, M[j][0], M[j][1], M[j][2]);
+}
+
+// A symmetric tensor stored as its upper triangle v = (xx, xy, xz, yy, yz, zz) -> the upper triangle (ee, en, eu, nn, nu,
+// uu) of Q V Q' (rotate_matrix), in place.
+__device__ __forceinline__ void rotate_tensor(const Frame& f, double (&v)[6]) {
+    double M[3][3] = {{v[0], v[1], v[2]}, {v[1], v[3], v[4]}, {v[2], v[4], v[5]}};
+    rotate_matrix(f, M);
+    v[0] = M[0][0];
+    v[1] = M[0][1];
+    v[2] = M[0][2];
+    v[3] = M[1][1];
+    v[4] = M[1][2];
+    v[5] = M[2][2];
+}
+
+// The transpose of rotate_tensor on 6-vectors.  rotate_tensor stores each off-diagonal entry once, so it is orthogonal
+// for the weights D = diag(1, 2, 2, 1, 2, 1) and not for the plain dot product: its transpose is D A^-1 D^-1, not the
+// inverse rotation.  The off-diagonal inputs are halved (exact), the symmetric matrix is rotated back as Q' V Q
+// (rotate_back on the columns, then on the rows), and the off-diagonal entries of its upper triangle are doubled (exact).
+__device__ __forceinline__ void rotate_tensor_transpose(const Frame& f, double (&v)[6]) {
+    const double h1 = __dmul_rn(0.5, v[1]), h2 = __dmul_rn(0.5, v[2]), h4 = __dmul_rn(0.5, v[4]);
+    double M[3][3] = {{v[0], h1, h2}, {h1, v[3], h4}, {h2, h4, v[5]}};
+    rotate_matrix<false>(f, M);
+    v[0] = M[0][0];
+    v[1] = __dmul_rn(2.0, M[0][1]);
+    v[2] = __dmul_rn(2.0, M[0][2]);
+    v[3] = M[1][1];
+    v[4] = __dmul_rn(2.0, M[1][2]);
+    v[5] = M[2][2];
 }
 
 }  // namespace gbgrad

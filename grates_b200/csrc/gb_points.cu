@@ -21,6 +21,10 @@
 //                          the normal equations sum_p J~_p' W_p J~_p of acceleration observations (J~_p = Q_p J_p): the
 //                          weighted, rotated Jacobian rows as both GEMM operands, contracted over observations on the
 //                          tiles of the upper triangle only, added into N and mirrored.
+//   gb_points_gravity_gradient_normals
+//                          the same for the six observations of the gravity gradient tensor per point, on a
+//                          gravity-gradient point set: one body templated on the order of the derivative, a row writer
+//                          per order.
 #include <vector>
 #include <cmath>
 #include "gb_common.cuh"
@@ -791,6 +795,49 @@ gb_points_gradient_normal_rows(double* __restrict__ At, double* __restrict__ Bt,
     }
 }
 
+// The rows sqrt(w_pc) J~_p[c] of gravity-gradient observations, observation o = 6 pp + c with the pairs c = xx, xy, xz, yy,
+// yz, zz, in the layouts of gb_points_gradient_normal_rows.  fr: the dense degree-(N+2) rows F'' of the block from degree
+// nmin + 2 on.  Entry (a, b) of the point is the composed F''_p T_a T_b of gbgrad::apply_pair (the expression of the
+// transposed transform), then gbgrad::rotate_tensor for the local frame (the upper triangle of Q V Q', as
+// gb_rotate_tensor_to_local), then the weights.
+__global__ void __launch_bounds__(256)
+gb_points_gravity_gradient_normal_rows(double* __restrict__ At, double* __restrict__ Bt, const double* __restrict__ fr,
+                                       long long kf, int nmin, long long Kc, int am, int bm, int rows, int count,
+                                       const double* __restrict__ weights, const double* __restrict__ frame,
+                                       long long npts, int p0) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x;
+    const int pp = blockIdx.y;
+    if (a >= am && a >= bm) return;
+    double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    if (a < Kc && pp < count) {
+        const long long ad = a + (long long)nmin * nmin;                          // degree-wise index from degree 0
+        int n = (int)sqrt((double)ad);
+        if ((long long)n * n > ad) --n;
+        if ((long long)(n + 1) * (n + 1) <= ad) ++n;
+        const int j = (int)(ad - (long long)n * n);                               // 0: C_n0, 2m-1: C_nm, 2m: S_nm
+        const int m = (j + 1) >> 1;
+        const int s = (j > 0 && (j & 1) == 0) ? 1 : 0;
+        const double* f = fr + (size_t)pp * kf + ((long long)(n + 2) * (n + 2) - (long long)(nmin + 2) * (nmin + 2));
+        auto at = [&](int mp, int sp) { return f[mp == 0 ? 0 : 2 * mp - 1 + sp]; };    // F'' of (n + 2, mp, sp)
+        const double q0 = gbgrad::grad_q(n), q1 = gbgrad::grad_q(n + 1);
+#pragma unroll
+        for (int c = 0; c < 6; ++c) v[c] = gbgrad::apply_pair(gbgrad::pair_a(c), gbgrad::pair_b(c), n, m, s, q0, q1, at);
+        const long long p = p0 + (long long)pp;
+        if (frame) gbgrad::rotate_tensor({frame[p], frame[npts + p], frame[2 * npts + p], frame[3 * npts + p]}, v);
+        if (weights) {
+#pragma unroll
+            for (int c = 0; c < 6; ++c) v[c] = __dmul_rn(__dsqrt_rn(weights[c * npts + p]), v[c]);
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < 6; ++c) {
+        const int o = 6 * pp + c;
+        if (o >= rows) break;
+        if (a < am) At[gb_ab_offset(a, o, rows)] = v[c];
+        if (a < bm) Bt[((size_t)(a / GB_S2_TN) * rows + o) * GB_S2_LDB + a % GB_S2_TN] = v[c];
+    }
+}
+
 // Epilogue of the normals: C[a][b] = sum_o J~[o][a] J~[o][b] over the block's observations, added to N[a][b] for b >= a
 // (upper triangle).  One thread per entry per launch and the launches in stream order: bit-reproducible.
 struct NormalsAddUpper {
@@ -822,31 +869,35 @@ gb_mirror_upper(double* __restrict__ N, long long K) {
     }
 }
 
-}  // namespace
-
-extern "C" int gb_points_gradient_normals(gb_points* p, int nmin, const double* d_weights, const double* d_frame,
-                                          double* d_normals, void* stream) {
-    GB_REQUIRE(p != nullptr, "gb_points_gradient_normals: point set is NULL");
-    GB_REQUIRE(p->nmax >= 1, "gb_points_gradient_normals: a gradient point set has degree nmax + 1 >= 1 (got %d)",
+// The normal equations of observations of the derivatives of order ORDER (1: the three components of grad V on a gradient
+// point set, 2: the six of the gravity gradient tensor on a gravity-gradient point set, degree nmax + ORDER): NC = 3 or 6
+// observation rows per point, written by the row writer of the order.
+template <int ORDER>
+int points_derivative_normals(const char* name, const char* kind, gb_points* p, int nmin, const double* d_weights,
+                              const double* d_frame, double* d_normals, void* stream) {
+    constexpr int NC = ORDER == 1 ? 3 : 6;
+    GB_REQUIRE(p != nullptr, "%s: point set is NULL", name);
+    GB_REQUIRE(p->nmax >= ORDER, "%s: a %s point set has degree nmax + %d >= %d (got %d)", name, kind, ORDER, ORDER,
                p->nmax);
-    const int nmax = p->nmax - 1;                                      // degree of the field
-    GB_REQUIRE(nmin >= 0 && nmin <= nmax, "gb_points_gradient_normals: min_degree=%d outside [0, %d]", nmin, nmax);
-    GB_REQUIRE(d_normals != nullptr, "gb_points_gradient_normals: NULL device pointer");
+    const int nmax = p->nmax - ORDER;                                  // degree of the field
+    GB_REQUIRE(nmin >= 0 && nmin <= nmax, "%s: min_degree=%d outside [0, %d]", name, nmin, nmax);
+    GB_REQUIRE(d_normals != nullptr, "%s: NULL device pointer", name);
     GB_CUDA(cudaSetDevice(p->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const long long Kc = (long long)(nmax + 1) * (nmax + 1) - (long long)nmin * nmin;   // coefficients of the field
-    const long long kf = (long long)p->L * p->L - (long long)(nmin + 1) * (nmin + 1);     // F' from degree nmin + 1
+    const long long f0 = (long long)(nmin + ORDER) * (nmin + ORDER);
+    const long long kf = (long long)p->L * p->L - f0;                  // the synthesis rows from degree nmin + ORDER
     const int n_mtiles = (int)((Kc + GB_TM - 1) / GB_TM);
     const int n_ntiles = (int)((Kc + GB_S2_TN - 1) / GB_S2_TN);
     const int am = n_mtiles * GB_TM, bm = n_ntiles * GB_S2_TN;
-    // points per block: an A operand of about 512 MB (the B operand is as large), a multiple of 4 points so that the 3 pb
-    // observation rows of a full block are whole k4 steps
-    long long pb = (512LL << 20) / ((long long)n_mtiles * GB_LDA * sizeof(double)) / 3;
+    // points per block: an A operand of about 512 MB (the B operand is as large), a multiple of 4 points so that the NC pb
+    // observation rows of a full block are whole k4 steps, and at most 49152 observation rows
+    long long pb = (512LL << 20) / ((long long)n_mtiles * GB_LDA * sizeof(double)) / NC;
     pb = pb / 4 * 4;
     if (pb < 4) pb = 4;
-    if (pb > 16384) pb = 16384;
+    if (pb > 49152 / NC) pb = 49152 / NC;
     if (pb > (p->npts + 3) / 4 * 4) pb = (p->npts + 3) / 4 * 4;
-    const int max_rows = (int)(3 * pb);
+    const int max_rows = (int)(NC * pb);
     double *d_at = nullptr, *d_bt = nullptr, *d_fr = nullptr;
     gb_retain_pool_memory(p->device);
     gb_scratch scratch(st);
@@ -865,14 +916,18 @@ extern "C" int gb_points_gradient_normals(gb_points* p, int nmin, const double* 
     const int threads = L >= 1024 ? 1024 : (L + 31) / 32 * 32;
     for (int p0 = 0; p0 < p->npts; p0 += (int)pb) {
         const int count = (p->npts - p0 < pb) ? (p->npts - p0) : (int)pb;
-        const int rows = (3 * count + 3) / 4 * 4;
-        gb_points_design_rows<<<count, threads, 0, st>>>(DenseRows{d_fr, kf, (long long)(nmin + 1) * (nmin + 1)},
-                                                         p->d_ct, p->d_kn, p->d_pmm, p->d_cml, p->d_sml, p->d_ra,
-                                                         p->d_rb, p->d_rc, L, nmin + 1, p0 + count, p0);
+        const int rows = (NC * count + 3) / 4 * 4;
+        gb_points_design_rows<<<count, threads, 0, st>>>(DenseRows{d_fr, kf, f0}, p->d_ct, p->d_kn, p->d_pmm, p->d_cml,
+                                                         p->d_sml, p->d_ra, p->d_rb, p->d_rc, L, nmin + ORDER,
+                                                         p0 + count, p0);
         GB_LAUNCH_CHECK();
-        dim3 grid((unsigned)(((am > bm ? am : bm) + 255) / 256), (unsigned)((rows + 2) / 3));
-        gb_points_gradient_normal_rows<<<grid, 256, 0, st>>>(d_at, d_bt, d_fr, kf, nmin, Kc, am, bm, rows, count,
-                                                             d_weights, d_frame, p->npts, p0);
+        dim3 grid((unsigned)(((am > bm ? am : bm) + 255) / 256), (unsigned)((rows + NC - 1) / NC));
+        if constexpr (ORDER == 1)
+            gb_points_gradient_normal_rows<<<grid, 256, 0, st>>>(d_at, d_bt, d_fr, kf, nmin, Kc, am, bm, rows, count,
+                                                                 d_weights, d_frame, p->npts, p0);
+        else
+            gb_points_gravity_gradient_normal_rows<<<grid, 256, 0, st>>>(d_at, d_bt, d_fr, kf, nmin, Kc, am, bm, rows,
+                                                                         count, d_weights, d_frame, p->npts, p0);
         GB_LAUNCH_CHECK();
         sh.a_rows = rows;
         sh.b_rows = rows;
@@ -884,4 +939,18 @@ extern "C" int gb_points_gradient_normals(gb_points* p, int nmin, const double* 
     gb_mirror_upper<<<dim3(nt32, nt32), dim3(32, 8), 0, st>>>(d_normals, Kc);
     GB_LAUNCH_CHECK();
     return GB_OK;
+}
+
+}  // namespace
+
+extern "C" int gb_points_gradient_normals(gb_points* p, int nmin, const double* d_weights, const double* d_frame,
+                                          double* d_normals, void* stream) {
+    return points_derivative_normals<1>("gb_points_gradient_normals", "gradient", p, nmin, d_weights, d_frame, d_normals,
+                                        stream);
+}
+
+extern "C" int gb_points_gravity_gradient_normals(gb_points* p, int nmin, const double* d_weights, const double* d_frame,
+                                                  double* d_normals, void* stream) {
+    return points_derivative_normals<2>("gb_points_gravity_gradient_normals", "gravity gradient", p, nmin, d_weights,
+                                        d_frame, d_normals, stream);
 }

@@ -673,26 +673,41 @@ def gradient_adjoint_at_positions(values, positions, max_degree, GM=GM_DEFAULT, 
     <gradient_at_positions(X), Y> = <X, gradient_adjoint_at_positions(Y)>: the operator J' of an iterative
     least-squares solver.  With a CUDA tensor input (or device_output=True) the result is a CUDA tensor, otherwise a
     numpy array.  Non-finite positions and the origin raise ValueError."""
+    return _derivative_adjoint_at_positions(values, positions, max_degree, GM, R, frame, device_output, 1)
+
+
+def gravity_gradient_adjoint_at_positions(values, positions, max_degree, GM=GM_DEFAULT, R=R_DEFAULT, frame='cartesian',
+                                          device_output=False):
+    """Transpose of ``gravity_gradient_at_positions``: values [E, 6, P] in s^-2 at Earth-fixed Cartesian positions [P, 3]
+    in metres, the six components (xx, xy, xz, yy, yz, zz) or (ee, en, eu, nn, nu, uu) of ``frame`` -> packed
+    coefficients [E, L, L], L = max_degree + 1, with
+    <gravity_gradient_at_positions(X), Y> = <X, gravity_gradient_adjoint_at_positions(Y)>.  The result's kind as for
+    ``gradient_adjoint_at_positions``.  Non-finite positions and the origin raise ValueError."""
+    return _derivative_adjoint_at_positions(values, positions, max_degree, GM, R, frame, device_output, 2)
+
+
+def _derivative_adjoint_at_positions(values, positions, max_degree, GM, R, frame, device_output, order):
+    ncomp = _DERIVATIVE_CALLS[order][0]
     if frame not in _FRAMES:
         raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
     if int(max_degree) < 0:
         raise ValueError("max_degree must be >= 0 (got {0})".format(max_degree))
     v = _host_or_cuda(values, "values")
     r, colat, lon = utilities.cartesian_to_spherical(positions)
-    if v.ndim != 3 or v.shape[1] != 3 or v.shape[2] != r.size:
-        raise ValueError("values must have shape [sets, 3, {0}] (got {1})".format(r.size, tuple(v.shape)))
-    p = _plan.get_gradient_points_plan(r, colat, lon, int(max_degree), GM, R)
+    if v.ndim != 3 or v.shape[1] != ncomp or v.shape[2] != r.size:
+        raise ValueError("values must have shape [sets, {0}, {1}] (got {2})".format(ncomp, r.size, tuple(v.shape)))
+    p = _plan._derivative_points_plan(r, colat, lon, int(max_degree), order, GM, R, None, True)
     on_device = isinstance(v, torch.Tensor)
     if on_device and v.device.index != p.device:
         raise ValueError("values must be a float64 CUDA tensor on device {0}".format(p.device))
     x = v if on_device else torch.as_tensor(np.ascontiguousarray(v)).to(torch.device("cuda", p.device))
-    out = p.gradient_adjoint(x, frame)
+    out = p._derivative_adjoint(x, frame, order)
     return out if (on_device or device_output) else out.cpu().numpy()
 
 
-def _positions_per_chunk(max_degree):
-    """Positions whose point-plan tables (four [P, N + 2] tables) take about 1 GB."""
-    return max(1, (1 << 30) // (8 * 4 * (int(max_degree) + 2)))
+def _positions_per_chunk(max_degree, order=1):
+    """Positions whose point-plan tables (four [P, N + order + 1] tables) take about 1 GB."""
+    return max(1, (1 << 30) // (8 * 4 * (int(max_degree) + order + 1)))
 
 
 def gradient_normal_equations_at_positions(observations, positions, min_degree, max_degree, GM=GM_DEFAULT, R=R_DEFAULT,
@@ -715,7 +730,50 @@ def gradient_normal_equations_at_positions(observations, positions, min_degree, 
     (gb_points_gradient_normals, ``gradient_adjoint_at_positions``); long position arrays are cut into chunks of
     positions_per_chunk (None: the positions whose tables take about 1 GB) with point plans of their own, closed after
     use.  Work: about 3 P K'^2 flops on the FP64 tensor cores (the upper triangle of N)."""
+    return _normal_equations_at_positions(observations, positions, min_degree, max_degree, GM, R, frame, weights,
+                                          block_size, positions_per_chunk, 1)
+
+
+def gravity_gradient_normal_equations_at_positions(observations, positions, min_degree, max_degree, GM=GM_DEFAULT,
+                                                   R=R_DEFAULT, frame='cartesian', weights=None, block_size=2048,
+                                                   positions_per_chunk=None):
+    """Least-squares normal equations of gravity-gradient observations (a gradiometer) at Earth-fixed Cartesian
+    positions, for the degree-wise coefficients from min_degree to max_degree, K' = (max_degree + 1)^2 - min_degree^2
+    unknowns.
+
+    observations: [E, 6, P] or [6, P] in s^-2 (numpy or CUDA float64, finite), E sets on the same positions sharing one
+    normal matrix; the components (xx, xy, xz, yy, yz, zz) Earth-fixed, or (ee, en, eu, nn, nu, uu) with frame='local',
+    as in ``gravity_gradient_at_positions``.  positions: [P, 3] in metres.  weights: [6, P] finite, non-negative weights
+    (inverse variances) per observation, or None for 1; a zero weight leaves the observation out (a component the
+    instrument measures badly).  With J~ the design matrix of the tensor in ``frame`` and W = diag(weights):
+
+      matrix                  N = J~' W J~ as a device ``lstsq.BlockMatrix`` with blocks of block_size
+      right_hand_side         n = J~' W l, CUDA tensor [K', E]
+      observation_square_sum  l' W l per set, numpy [E]
+      observation_count       the number of positive weights (6 P without weights)
+
+    returned as an ``lstsq.NormalEquations``.  Everything is formed on the device (gb_points_gravity_gradient_normals,
+    ``gravity_gradient_adjoint_at_positions``), in chunks of positions as ``gradient_normal_equations_at_positions``.
+    Work: about 6 P K'^2 flops on the FP64 tensor cores (the upper triangle of N)."""
+    return _normal_equations_at_positions(observations, positions, min_degree, max_degree, GM, R, frame, weights,
+                                          block_size, positions_per_chunk, 2)
+
+
+def _finite(x):
+    return bool((torch.isfinite(x) if isinstance(x, torch.Tensor) else np.isfinite(x)).all())
+
+
+# order of the derivative -> the uncached point plan of the chunks
+_CHUNK_PLANS = {1: _plan.gradient_points_plan, 2: _plan.gravity_gradient_points_plan}
+
+
+def _normal_equations_at_positions(observations, positions, min_degree, max_degree, GM, R, frame, weights, block_size,
+                                   positions_per_chunk, order):
+    """The normal equations of observations of the derivatives of order 1 (grad V, three components per position, with
+    positive weights) or 2 (the gravity gradient tensor, six components, with non-negative weights and finite
+    observations): every check before any device work, then the chunks of positions."""
     from .lstsq import BlockMatrix, NormalEquations
+    ncomp = _DERIVATIVE_CALLS[order][0]
     if frame not in _FRAMES:
         raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
     nmin, nmax = int(min_degree), int(max_degree)
@@ -732,16 +790,21 @@ def gradient_normal_equations_at_positions(observations, positions, min_degree, 
     single = obs.ndim == 2
     if single:
         obs = obs[None]
-    if obs.ndim != 3 or obs.shape[1] != 3 or obs.shape[2] != P or obs.shape[0] < 1:
-        raise ValueError("observations must have shape [sets, 3, {0}] or [3, {0}] (got {1})".format(
-            P, tuple(np.shape(observations))))
+    if obs.ndim != 3 or obs.shape[1] != ncomp or obs.shape[2] != P or obs.shape[0] < 1:
+        raise ValueError("observations must have shape [sets, {0}, {1}] or [{0}, {1}] (got {2})".format(
+            ncomp, P, tuple(np.shape(observations))))
+    if order == 2 and not _finite(obs):
+        raise ValueError("observations must be finite")
+    count = ncomp * P
     if w is not None:
-        if tuple(w.shape) != (3, P):
-            raise ValueError("weights must have shape [3, {0}] (got {1})".format(P, tuple(w.shape)))
-        ok = bool(torch.isfinite(w).all() and (w > 0).all()) if isinstance(w, torch.Tensor) else \
-            bool(np.all(np.isfinite(w)) and np.all(w > 0))
-        if not ok:
+        if tuple(w.shape) != (ncomp, P):
+            raise ValueError("weights must have shape [{0}, {1}] (got {2})".format(ncomp, P, tuple(w.shape)))
+        if order == 1 and not (_finite(w) and bool((w > 0).all())):
             raise ValueError("weights must be finite and positive")
+        if order == 2:
+            if not (_finite(w) and bool((w >= 0).all())):
+                raise ValueError("weights must be finite and non-negative")
+            count = int((w > 0).sum())
     dev = obs.device.index if isinstance(obs, torch.Tensor) else _plan._current_device(None)
     tdev = torch.device("cuda", dev)
 
@@ -756,17 +819,17 @@ def gradient_normal_equations_at_positions(observations, positions, min_degree, 
     normals = torch.zeros((kp, kp), dtype=torch.float64, device=tdev)
     anm = torch.zeros((E, nmax + 1, nmax + 1), dtype=torch.float64, device=tdev)
     lpl = torch.zeros(E, dtype=torch.float64, device=tdev)
-    chunk = _positions_per_chunk(nmax) if positions_per_chunk is None else int(positions_per_chunk)
+    chunk = _positions_per_chunk(nmax, order) if positions_per_chunk is None else int(positions_per_chunk)
     for p0 in range(0, P, chunk):
         p1 = min(P, p0 + chunk)
         l = on_device(obs, p0, p1)
         wc = None if w is None else on_device(w, p0, p1)
         wl = l if wc is None else l * wc
         lpl += (wl * l).sum(dim=(1, 2))
-        plan = _plan.gradient_points_plan(r[p0:p1], colat[p0:p1], lon[p0:p1], nmax, GM, R, dev)
+        plan = _CHUNK_PLANS[order](r[p0:p1], colat[p0:p1], lon[p0:p1], nmax, GM, R, dev)
         try:
-            plan.gradient_normals(normals, nmin, frame, wc)
-            anm += plan.gradient_adjoint(wl, frame)
+            plan._derivative_normals(normals, nmin, frame, wc, order)
+            anm += plan._derivative_adjoint(wl, frame, order)
         finally:
             plan.close()
     rhs = ravel_batch(anm, nmin).T.contiguous()
@@ -774,7 +837,7 @@ def gradient_normal_equations_at_positions(observations, positions, min_degree, 
     row_index, column_index = BlockMatrix.compute_block_index((kp, kp), int(block_size))
     matrix = BlockMatrix.from_array(normals, row_index, column_index)
     del normals
-    return NormalEquations(matrix, rhs, lpl.cpu().numpy(), 3 * P)
+    return NormalEquations(matrix, rhs, lpl.cpu().numpy(), count)
 
 
 def gridded_rms(temporal_gravityfield, epochs, kernel='ewh', base_grid=None):

@@ -627,13 +627,7 @@ class PointsPlan:
         its symmetric part (Sigma + Sigma') / 2.  frame 'cartesian' (x, y, z) or 'local' (east, north, up).  Returns a
         CUDA tensor [npts, 3, 3] of covariances in (m/s^2)^2 with full=True, else [3, npts] standard deviations in m/s^2
         (gb_points_gradient_covariance)."""
-        if frame not in ('cartesian', 'local'):
-            raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
-        if not hasattr(self, "frame"):
-            raise ValueError("gradient_covariance needs a gradient point plan (get_gradient_points_plan)")
-        nmax = self.max_degree - 1
-        if not 0 <= min_degree <= nmax:
-            raise ValueError("min_degree={0} outside [0, {1}]".format(min_degree, nmax))
+        nmax = self._derivative_field_degree(frame, min_degree, "gradient_covariance", 1)
         kp = (nmax + 1) ** 2 - min_degree ** 2
         if sigma.dim() != 2 or tuple(sigma.shape) != (kp, kp):
             raise ValueError("covariance matrix must have shape [{0}, {0}] (got {1})".format(kp, tuple(sigma.shape)))
@@ -648,23 +642,24 @@ class PointsPlan:
                                                            0 if full else 1, _stream_handle(self.device)))   # GB_COV_SQRT
         return out
 
-    def _gradient_field_degree(self, frame, min_degree, name):
+    def _derivative_field_degree(self, frame, min_degree, name, order):
+        """The degree N of the field of a plan of derivatives of order ``order`` (degree N + order), after the checks of
+        the frame, the plan's order and min_degree."""
         if frame not in ('cartesian', 'local'):
             raise ValueError("frame must be 'cartesian' or 'local' (got {0!r})".format(frame))
-        if not hasattr(self, "frame"):
-            raise ValueError("{0} needs a gradient point plan (get_gradient_points_plan)".format(name))
-        nmax = self.max_degree - 1
+        if getattr(self, "derivative_order", None) != order:
+            kind = _DERIVATIVES[order][0]
+            raise ValueError("{0} needs a {1} point plan (get_{2}_points_plan)".format(name, kind,
+                                                                                        kind.replace(" ", "_")))
+        nmax = self.max_degree - order
         if not 0 <= min_degree <= nmax:
             raise ValueError("min_degree={0} outside [0, {1}]".format(min_degree, nmax))
         return nmax
 
-    def gradient_normals(self, normals, min_degree, frame='cartesian', weights=None):
-        """Adds the normal equations sum_p J~_p' W_p J~_p of acceleration observations at the points of a gradient point
-        plan to ``normals``, a CUDA float64 tensor [K', K'] (K' = (N + 1)^2 - min_degree^2, degree-wise; zeroed by the
-        caller for a fresh matrix), and returns it with both triangles holding the sum.  J~_p: the Jacobian of grad V in
-        ``frame`` ('cartesian' or 'local'); weights: CUDA float64 tensor [3, npts] of positive weights (inverse variances)
-        or None for 1 (gb_points_gradient_normals)."""
-        nmax = self._gradient_field_degree(frame, min_degree, "gradient_normals")
+    def _derivative_normals(self, normals, min_degree, frame, weights, order):
+        ncomp, entry, _, _ = _POINT_CALLS[order]
+        nmax = self._derivative_field_degree(frame, min_degree, _DERIVATIVES[order][0].replace(" ", "_") + "_normals",
+                                             order)
         kp = (nmax + 1) ** 2 - min_degree ** 2
         if normals.dim() != 2 or tuple(normals.shape) != (kp, kp) or not normals.is_contiguous():
             raise ValueError("normal matrix must be a contiguous tensor of shape [{0}, {0}] (got {1})".format(
@@ -673,38 +668,73 @@ class PointsPlan:
             raise ValueError("normal matrix must be a float64 CUDA tensor on device {0}".format(self.device))
         w = None
         if weights is not None:
-            if tuple(weights.shape) != (3, self.npts):
-                raise ValueError("weights must have shape [3, {0}] (got {1})".format(self.npts, tuple(weights.shape)))
+            if tuple(weights.shape) != (ncomp, self.npts):
+                raise ValueError("weights must have shape [{0}, {1}] (got {2})".format(ncomp, self.npts,
+                                                                                      tuple(weights.shape)))
             if weights.dtype != torch.float64 or not weights.is_cuda or weights.device.index != self.device:
                 raise ValueError("weights must be a float64 CUDA tensor on device {0}".format(self.device))
             weights = weights.contiguous()
             w = ctypes.c_void_p(weights.data_ptr())
         fr = ctypes.c_void_p(self.frame.data_ptr()) if frame == 'local' else None
-        _lib.check(self._lib.gb_points_gradient_normals(self._handle, int(min_degree), w, fr,
-                                                        ctypes.c_void_p(normals.data_ptr()), _stream_handle(self.device)))
+        _lib.check(getattr(self._lib, entry)(self._handle, int(min_degree), w, fr, ctypes.c_void_p(normals.data_ptr()),
+                                             _stream_handle(self.device)))
         return normals
 
-    def gradient_adjoint(self, values, frame='cartesian'):
-        """Transpose of the acceleration at the points of a gradient point plan: values CUDA float64 [E, 3, npts] in
-        ``frame`` -> CUDA tensor [E, N + 1, N + 1] packed, sum_p J_p' Q_p' v_p: Q' for 'local' (gb_rotate_from_local), the
-        adjoint synthesis of the 3E component sets (``adjoint``) and T' (gb_gradient_coefficients_adjoint)."""
-        nmax = self._gradient_field_degree(frame, 0, "gradient_adjoint")
-        if values.dim() != 3 or values.shape[1] != 3 or values.shape[2] != self.npts:
-            raise ValueError("values must have shape [sets, 3, {0}] (got {1})".format(self.npts, tuple(values.shape)))
+    def _derivative_adjoint(self, values, frame, order):
+        ncomp, _, rotation, transform = _POINT_CALLS[order]
+        nmax = self._derivative_field_degree(frame, 0, _DERIVATIVES[order][0].replace(" ", "_") + "_adjoint", order)
+        if values.dim() != 3 or values.shape[1] != ncomp or values.shape[2] != self.npts:
+            raise ValueError("values must have shape [sets, {0}, {1}] (got {2})".format(ncomp, self.npts,
+                                                                                       tuple(values.shape)))
         if values.dtype != torch.float64 or not values.is_cuda or values.device.index != self.device:
             raise ValueError("values must be a float64 CUDA tensor on device {0}".format(self.device))
         E = values.shape[0]
         st = _stream_handle(self.device)
         if frame == 'local':
             values = values.clone(memory_format=torch.contiguous_format)
-            _lib.check(self._lib.gb_rotate_from_local(ctypes.c_void_p(values.data_ptr()),
-                                                      ctypes.c_void_p(self.frame.data_ptr()), E, self.npts, self.device,
-                                                      st))
-        g = self.adjoint(values.contiguous().view(3 * E, self.npts))
+            _lib.check(getattr(self._lib, rotation)(ctypes.c_void_p(values.data_ptr()),
+                                                    ctypes.c_void_p(self.frame.data_ptr()), E, self.npts, self.device,
+                                                    st))
+        g = self.adjoint(values.contiguous().view(ncomp * E, self.npts))
         out = torch.empty((E, nmax + 1, nmax + 1), dtype=torch.float64, device=values.device)
-        _lib.check(self._lib.gb_gradient_coefficients_adjoint(ctypes.c_void_p(g.data_ptr()), E, nmax,
-                                                              ctypes.c_void_p(out.data_ptr()), self.device, st))
+        _lib.check(getattr(self._lib, transform)(ctypes.c_void_p(g.data_ptr()), E, nmax, ctypes.c_void_p(out.data_ptr()),
+                                                 self.device, st))
         return out
+
+    def gradient_normals(self, normals, min_degree, frame='cartesian', weights=None):
+        """Adds the normal equations sum_p J~_p' W_p J~_p of acceleration observations at the points of a gradient point
+        plan to ``normals``, a CUDA float64 tensor [K', K'] (K' = (N + 1)^2 - min_degree^2, degree-wise; zeroed by the
+        caller for a fresh matrix), and returns it with both triangles holding the sum.  J~_p: the Jacobian of grad V in
+        ``frame`` ('cartesian' or 'local'); weights: CUDA float64 tensor [3, npts] of positive weights (inverse variances)
+        or None for 1 (gb_points_gradient_normals)."""
+        return self._derivative_normals(normals, min_degree, frame, weights, 1)
+
+    def gradient_adjoint(self, values, frame='cartesian'):
+        """Transpose of the acceleration at the points of a gradient point plan: values CUDA float64 [E, 3, npts] in
+        ``frame`` -> CUDA tensor [E, N + 1, N + 1] packed, sum_p J_p' Q_p' v_p: Q' for 'local' (gb_rotate_from_local), the
+        adjoint synthesis of the 3E component sets (``adjoint``) and T' (gb_gradient_coefficients_adjoint)."""
+        return self._derivative_adjoint(values, frame, 1)
+
+    def gravity_gradient_normals(self, normals, min_degree, frame='cartesian', weights=None):
+        """``gradient_normals`` for gravity-gradient observations at the points of a gravity-gradient point plan
+        (get_gravity_gradient_points_plan: degree N + 2 for a degree-N field): six observations per point, (xx, xy, xz,
+        yy, yz, zz) or with frame='local' (ee, en, eu, nn, nu, uu) as in ``gravity_gradient_at_positions``; weights: CUDA
+        float64 tensor [6, npts] of non-negative weights (0 leaves an observation out) or None for 1
+        (gb_points_gravity_gradient_normals)."""
+        return self._derivative_normals(normals, min_degree, frame, weights, 2)
+
+    def gravity_gradient_adjoint(self, values, frame='cartesian'):
+        """Transpose of the gravity gradient at the points of a gravity-gradient point plan: values CUDA float64
+        [E, 6, npts] in ``frame`` -> CUDA tensor [E, N + 1, N + 1] packed: the transposed rotation for 'local'
+        (gb_rotate_tensor_from_local), the adjoint synthesis of the 6E component sets (``adjoint``) and the transposed
+        transform (gb_gravity_gradient_coefficients_adjoint)."""
+        return self._derivative_adjoint(values, frame, 2)
+
+
+# order of the derivative -> (observations per point, normal equations, transposed rotation, transposed transform)
+_POINT_CALLS = {1: (3, "gb_points_gradient_normals", "gb_rotate_from_local", "gb_gradient_coefficients_adjoint"),
+                2: (6, "gb_points_gravity_gradient_normals", "gb_rotate_tensor_from_local",
+                    "gb_gravity_gradient_coefficients_adjoint")}
 
 
 def get_points_plan(grid, max_degree, kernel='ewh', GM=3.9860044150e+14, R=6.3781363000e+06, device=None):
@@ -793,6 +823,7 @@ def _derivative_plan(grid, max_degree, order, GM, R, device):
         plan = SHPlan(meridians, parallels, a, f, int(max_degree) + order, name, GM, R, dev, degree_factors=kn)
         nlat, nlon = plan.nlat, plan.nlon
         plan.frame = _frame_table(np.repeat(plan.colat, nlon), np.tile(meridians, nlat), dev)
+        plan.derivative_order = order
         return plan
     return _cached(key, make)
 
@@ -823,6 +854,7 @@ def _derivative_points_plan(radius, colat, lon, max_degree, order, GM, R, device
         plan = PointsPlan(lon, 0.5 * np.pi - colat, utilities.A_GRS80, utilities.F_GRS80, int(max_degree) + order, name,
                           GM, R, dev, degree_factors=kn, colatitude=colat)
         plan.frame = _frame_table(colat, lon, dev)
+        plan.derivative_order = order
         return plan
     if not cached:
         return make()
@@ -847,6 +879,13 @@ def get_gravity_gradient_points_plan(radius, colat, lon, max_degree, GM=3.986004
     """Cached PointsPlan at degree max_degree + 2 for the gravity gradient tensor at points, as get_gradient_points_plan
     with the degree factors of gravity_gradient_degree_factors and its own cache variant."""
     return _derivative_points_plan(radius, colat, lon, max_degree, 2, GM, R, device, True)
+
+
+def gravity_gradient_points_plan(radius, colat, lon, max_degree, GM=3.9860044150e+14, R=6.3781363000e+06,
+                                 device=None):
+    """The PointsPlan of get_gravity_gradient_points_plan, not cached: the caller closes it (long position arrays in
+    chunks)."""
+    return _derivative_points_plan(radius, colat, lon, max_degree, 2, GM, R, device, False)
 
 
 def clear_plan_cache():

@@ -53,7 +53,7 @@ typedef struct gb_plan gb_plan;
 
 /* Library version (major*10000 + minor*100 + patch); bumped with every change of this header.  The Python binding
  * refuses a library whose version differs from the one it was written for (grates_b200/_lib.py). */
-#define GB_VERSION 206
+#define GB_VERSION 207
 int gb_version(void);
 
 /* Thread-local description of the last error returned on this thread. */
@@ -299,6 +299,16 @@ int gb_points_gradient_covariance(gb_points* points, const double* d_sigma, int 
  * Bit-reproducible from run to run. */
 int gb_points_gradient_normals(gb_points* points, int nmin, const double* d_weights, const double* d_frame,
                                double* d_normals, void* stream);
+/* Normal equations of gravity-gradient observations at the points of a GRAVITY-GRADIENT point set (degree nmax + 2 for a
+ * degree-nmax field, factors GM/R^3 (R/r)^(n''+1)): ADDS N = sum_p J~_p' W_p J~_p to d_normals [K'][K'], K' =
+ * (nmax + 1)^2 - nmin^2, with the contract of gb_points_gradient_normals.  J~_p holds the six observations of the point,
+ * (xx, xy, xz, yy, yz, zz) Earth-fixed, or with d_frame (ee, en, eu, nn, nu, uu): the upper triangle of Q V Q' as
+ * gb_rotate_tensor_to_local.  Observation (a, b) is V_ab = F''_p T_a T_b x, the definition of
+ * gb_gravity_gradient_coefficients.
+ *   d_weights [6][npts] non-negative weights (inverse variances; 0 leaves an observation out), or NULL for 1
+ * About 6 npts K'^2 flops on the upper-triangle tiles.  Bit-reproducible from run to run. */
+int gb_points_gravity_gradient_normals(gb_points* points, int nmin, const double* d_weights, const double* d_frame,
+                                       double* d_normals, void* stream);
 
 /*
  * Consumers of gridded epoch batches that keep the grids on the device.
@@ -373,6 +383,17 @@ int gb_gravity_gradient_coefficients(const double* d_anm, int n_sets, int nmax, 
                                      void* stream);
 int gb_rotate_tensor_to_local(double* d_v, const double* d_frame, int n_sets, int64_t n_points, int device,
                               void* stream);
+/* The transposes, for the adjoint of the gravity gradient at points:
+ *   gb_gravity_gradient_coefficients_adjoint   d_in [n_sets][6][L+2][L+2] packed (xx .. zz) -> d_anm [n_sets][L][L]
+ *                                              packed, anm = sum over the pairs of (T_a T_b)' in_ab in the order xx .. zz;
+ *                                              degrees 0 and 1 of d_in are not read.  A gather, no atomics.
+ *   gb_rotate_tensor_from_local                the transpose of gb_rotate_tensor_to_local on the 6-vectors, in place.  It
+ *                                              is not the inverse rotation: the off-diagonal inputs are halved, rotated
+ *                                              back as Q' V Q, and the off-diagonal outputs doubled. */
+int gb_gravity_gradient_coefficients_adjoint(const double* d_in, int n_sets, int nmax, double* d_anm, int device,
+                                             void* stream);
+int gb_rotate_tensor_from_local(double* d_v, const double* d_frame, int n_sets, int64_t n_points, int device,
+                                void* stream);
 
 /* Pinned host memory for the *_host entry points. */
 int gb_host_alloc(void** ptr, uint64_t bytes);
